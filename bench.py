@@ -1,10 +1,12 @@
 #!/usr/bin/env python
 """bench.py -- SHA-256 witness-generation throughput (blocks/s, bit-exact cells) on N B200s, next to the CPU path.
 
-    python bench.py --gpus N --steps K --warmup W [--workload cfg2] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--workload cfg2] [--impl reference] [--dump-outputs DIR]
 
-A "step" is one pass of the hot path over one batch of synthetic messages: every advice / lookup / spread cell of
-every instance is generated into HBM (column-major Fr, Montgomery form) plus digests and cell checksums.
+A pass of the hot path over one batch of synthetic messages generates every advice / lookup / spread cell of every
+instance into HBM (column-major Fr, Montgomery form) plus digests and cell checksums.  A timed step is L such passes back
+to back (--launches-per-step; by default as many as make one step take >= 30 ms), and exactly K steps are timed.
+--dump-outputs DIR writes what the last timed step computed to DIR (see dump_outputs).
 At N=1 the workload is BASELINE.json configs[1] (1024 random 55-byte messages, one block each); with N>1 every
 rank generates its own shard of the same size (weak scaling, no data-path collective; digests and checksums are
 gathered over NCCL after the timed region).
@@ -32,6 +34,29 @@ if ROOT not in sys.path:
 
 METRIC = "SHA-256 blocks/sec witness-gen (bit-exact cells)"
 UNIT = "blocks/s"
+DUMP_BYTES_PER_ARRAY = 12 << 20   # --dump-outputs: five arrays, at most 60 MiB in all
+DUMP_SEED = 0
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each output tensor as out_dir/<name>.npy without losing a bit: uint8 arrays as float32, 64-bit words as two
+    float64 values each (low 32 bits first), one row per digest / per instance's checksums / per 32-byte cell.  An output
+    larger than DUMP_BYTES_PER_ARRAY is a sample of its rows, drawn with a fixed seed and sorted; the row numbers (of the
+    tensor flattened to rows) go to out_dir/<name>_rows.npy.  Equal arguments to bench.py give equal inputs, so the files of
+    two builds compare entry for entry."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        rows = t.reshape(-1, t.shape[-1])
+        row_bytes = rows.shape[1] * (4 if t.dtype == torch.uint8 else 16)
+        if rows.shape[0] * row_bytes > DUMP_BYTES_PER_ARRAY:
+            m = DUMP_BYTES_PER_ARRAY // (row_bytes + 8)
+            idx = np.sort(np.random.default_rng(DUMP_SEED).choice(rows.shape[0], m, replace=False))
+            rows = rows[torch.from_numpy(idx).to(rows.device)]
+            np.save(os.path.join(out_dir, f"{name}_rows.npy"), idx.astype(np.float64))
+        h = rows.cpu().numpy()
+        h = h.astype(np.float32) if h.dtype == np.uint8 else h.view(np.uint32).astype(np.float64)
+        np.save(os.path.join(out_dir, f"{name}.npy"), h)
 
 
 def measured_peak_gbs():
@@ -155,12 +180,12 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
-def measure_full(ctx, w, min_seconds=0.5, max_steps=64, mem_frac=0.6, split=True, verify=8, limit_instances=0):
+def measure_full(ctx, w, min_seconds=0.5, max_steps=64, mem_frac=0.6, split=True, verify=8, limit_instances=0, steps=0):
     """A WHOLE configuration (or, with limit_instances, its first instances) sharded by instance over the ranks and streamed through
     each GPU's HBM in chunks: a step = every instance of the shard generated once (the witness of a chunk is overwritten by the next
     chunk, as a prover that consumes chunk by chunk would allow; digests and per-instance checksums of all instances are kept).
-    Times >= min_seconds of steps with CUDA events on the launching stream (max over ranks), samples clocks during them, then checks
-    digests against hashlib, the last chunk's witness under the device-side MockProver pass and `verify` instances against the oracle."""
+    Times `steps` steps (0: >= min_seconds of them, at most max_steps) with CUDA events on the launching stream (max over ranks),
+    samples clocks during them, then checks digests against hashlib, the last chunk's witness under the device-side MockProver pass and `verify` instances against the oracle."""
     import hashlib
 
     import torch
@@ -201,7 +226,7 @@ def measure_full(ctx, w, min_seconds=0.5, max_steps=64, mem_frac=0.6, split=True
     step(); stream.synchronize()
     w0.record(stream); step(); w1.record(stream); w1.synchronize()
     est_ms = max(w0.elapsed_time(w1), 1e-3)
-    steps = int(min(max_steps, max(1, np.ceil(min_seconds * 1e3 / est_ms))))
+    steps = steps or int(min(max_steps, max(1, np.ceil(min_seconds * 1e3 / est_ms))))
     if world > 1:
         t = torch.tensor([steps], dtype=torch.int64, device=dev); dist.all_reduce(t, op=dist.ReduceOp.MAX); steps = int(t.item())
     barrier()
@@ -337,7 +362,7 @@ def run_full_workload(args):
     """--full-workload: the WHOLE BASELINE configuration (all its instances, e.g. 2^16 x 5 blocks or 2^18 x 33 blocks), see measure_full."""
     ctx = _gpu_context(args)
     w = ctx["S"].WORKLOADS[args.workload]
-    r = measure_full(ctx, w, min_seconds=0.5, max_steps=max(1, args.steps))
+    r = measure_full(ctx, w, steps=args.steps)
     if ctx["rank"] == 0:
         print(json.dumps({
             "metric": METRIC, "value": r["value"], "unit": UNIT, "n_gpus": ctx["world"], "steps": r["steps"], "warmup": 1, "ms_per_step": r["ms_per_step"],
@@ -370,13 +395,20 @@ def main():
                     help="generate the WHOLE configuration (all instances, sharded over the ranks, streamed through HBM in chunks) "
                          "instead of one HBM-sized batch per step; e.g. --workload cfg5 = 2^18 messages x 33 blocks = 22.5 TB of witness")
     ap.add_argument("--launches-per-step", type=int, default=0,
-                    help="passes over the batch per timed step (0 = as many as make the K timed steps cover >= 0.6 s)")
+                    help="passes over the batch per timed step (0 = as many as make one step take >= 30 ms)")
     ap.add_argument("--no-north-star", action="store_true", help="skip the north-star block (config 4 split over the ranks), the other configurations and the config-1 latency")
     ap.add_argument("--cpu-sample", type=int, default=1024, help="instances in the CPU-baseline sample")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-witness-d2h", action="store_true", help="skip the extra end-to-end leg that copies the whole witness to the host")
     ap.add_argument("--verify", type=int, default=8, help="instances per rank checked cell-for-cell against the oracle after timing")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed on rank 0 (digests, checksums, gate / lookup / spread "
+                         "cells; a seeded sample of the larger ones) as DIR/<name>.npy in float32 / float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.full_workload):
+        ap.error("--dump-outputs applies to the default GPU mode")
 
     if args.impl == "reference":
         run_reference(args)
@@ -444,15 +476,15 @@ def main():
     for _ in range(max(args.warmup, 3)):
         launch_resident()
     stream.synchronize()
-    # A step = L back-to-back passes of the hot path over the batch, L chosen so that the K timed steps cover >= ~0.6 s: long enough
-    # for the 100 ms clock sampler to see the load the steps are timed under (round 1 timed 10 ms in total)
+    # A step = L back-to-back passes of the hot path over the batch, L chosen so that one step takes >= ~30 ms (0.6 s for the default
+    # 20 steps): a pass over the default batch takes under a millisecond on a B200, too short a window to time on its own
     p0, p1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     p0.record(stream)
     for _ in range(8):
         launch_resident()
     p1.record(stream); p1.synchronize()
     est_launch_ms = max(p0.elapsed_time(p1) / 8, 1e-3)
-    L = args.launches_per_step or int(min(4096, max(1, np.ceil(600.0 / (max(1, args.steps) * est_launch_ms)))))
+    L = args.launches_per_step or int(min(4096, max(1, np.ceil(30.0 / est_launch_ms))))
     if world > 1:
         t = torch.tensor([L], dtype=torch.int64, device=dev); dist.all_reduce(t, op=dist.ReduceOp.MAX); L = int(t.item())
     blocks_per_step = L * blocks_per_launch
@@ -472,6 +504,8 @@ def main():
     ev1.record(stream)
     barrier()
     total_ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"digests": d_digests, "checksums": d_cks, "gate": gate, "lookup": lookup, "spread": spread})
     # per-kernel durations, measured live with CUDA events on the launching stream over the same launches (>= 0.5 s of them)
     t_loop = time.perf_counter()
     while len(kernel_ms) < args.steps or time.perf_counter() - t_loop < 0.5:
@@ -937,4 +971,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True   # the bench writes nothing into the tree it runs from (which may be read-only)
     main()

@@ -1,5 +1,5 @@
 import sys, os, time
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 import __graft_entry__ as ge
 from oracle import oracle as O
