@@ -29,7 +29,7 @@ H2SHA_OK, H2SHA_EINVAL, H2SHA_EPANIC, H2SHA_ECUDA, H2SHA_ENOMEM = 0, -1, -2, -3,
 # symbols include/h2sha_b200.h declares (checked by tests/test_abi.py)
 EXPORTED_SYMBOLS = [
     "h2sha_create", "h2sha_destroy", "h2sha_last_error", "h2sha_build_id", "h2sha_get_layout", "h2sha_get_breaks", "h2sha_get_handles", "h2sha_get_digest_ranges", "h2sha_get_shape", "h2sha_get_lookup_tables",
-    "h2sha_digest_batch", "h2sha_export_instance", "h2sha_export_batch", "h2sha_get_compact_info", "h2sha_get_compact_map", "h2sha_expand_compact", "h2sha_get_lookup_info", "h2sha_lookup_multiplicities", "h2sha_permute_lookup", "h2sha_permute_lookup_from_raw", "h2sha_check_batch", "h2sha_gather", "h2sha_zero_outputs", "h2sha_debug_mont_from_u64", "h2sha_debug_mont_from_u32", "h2sha_debug_store_probe", "h2sha_debug_int_probe", "h2sha_last_launch_count", "h2sha_last_kernel_ms", "H2SHA_CK_M",
+    "h2sha_digest_batch", "h2sha_export_instance", "h2sha_export_batch", "h2sha_get_compact_info", "h2sha_get_compact_map", "h2sha_expand_compact", "h2sha_get_lookup_info", "h2sha_lookup_multiplicities", "h2sha_permute_lookup", "h2sha_permute_lookup_from_raw", "h2sha_lookup_product", "h2sha_check_batch", "h2sha_gather", "h2sha_zero_outputs", "h2sha_debug_mont_from_u64", "h2sha_debug_mont_from_u32", "h2sha_debug_store_probe", "h2sha_debug_int_probe", "h2sha_last_launch_count", "h2sha_last_kernel_ms", "H2SHA_CK_M",
 ]
 
 
@@ -120,6 +120,8 @@ def load_library():
     sig("h2sha_lookup_multiplicities", [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p])
     sig("h2sha_permute_lookup", [C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
     sig("h2sha_permute_lookup_from_raw", [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
+    sig("h2sha_lookup_product", [C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p,
+                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
     sig("h2sha_check_batch", [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
     sig("h2sha_gather", [C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
     sig("h2sha_zero_outputs", [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p])
@@ -491,6 +493,28 @@ class Sha256DynamicConfig:
         if int(err.item()):
             raise EngineError(H2SHA_EINVAL, f"{int(err.item())} instance(s) whose multiplicities do not cover usable_rows")
         return a, s
+
+    def lookup_product(self, res: "BatchResult", lookup_idx: int, a_p, s_p, usable_rows: int, beta_mont: np.ndarray, gamma_mont: np.ndarray,
+                       theta_mont: Optional[np.ndarray] = None):
+        """(z [n_inst, usable_rows + 1, 4] int64 device tensor, instances whose z[usable_rows] != 1) of lookup `lookup_idx`, halo2's
+        `commit_product` from the batch's witness `res` and the permuted pair (A', S') [n_inst, usable_rows, 4] of the same instances."""
+        import torch
+        n = a_p.shape[0]
+        if tuple(a_p.shape) != (n, usable_rows, 4) or tuple(s_p.shape) != (n, usable_rows, 4):
+            raise EngineError(H2SHA_EINVAL, "A' and S' must be [n_instances, usable_rows, 4]")
+        for buf in (res.lookup, res.spread):
+            if buf is not None and buf.shape[0] < n:
+                raise EngineError(H2SHA_EINVAL, "the witness holds fewer instances than A' and S'")
+        dev = torch.device("cuda", self.device)
+        z = torch.empty((n, usable_rows + 1, 4), dtype=torch.int64, device=dev)
+        err = torch.zeros(1, dtype=torch.int32, device=dev)
+        ch = [None if x is None else np.ascontiguousarray(x, dtype=np.uint64) for x in (theta_mont, beta_mont, gamma_mont)]
+        assert all(x is None or x.shape == (4,) for x in ch)
+        ptr = lambda t: t.data_ptr() if t is not None else None
+        _check(load_library().h2sha_lookup_product(self._h, n, lookup_idx, ptr(res.lookup), ptr(res.spread), a_p.data_ptr(), s_p.data_ptr(), usable_rows,
+                                                   *[x.ctypes.data if x is not None else None for x in ch], z.data_ptr(), err.data_ptr(),
+                                                   torch.cuda.current_stream(self.device).cuda_stream))
+        return z, int(err.item())
 
     def launches_last_batch(self) -> int:
         return int(load_library().h2sha_last_launch_count(self._h))

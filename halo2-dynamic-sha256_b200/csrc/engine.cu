@@ -1473,6 +1473,8 @@ struct h2sha_engine {
   uint64_t lk_ws_bytes = 0;
   uint32_t* d_lk_tab = nullptr;   // compressed spread table in sorted order
   uint32_t* d_range_tab = nullptr;   // Montgomery form of the range table's values
+  uint64_t* d_lp_ws = nullptr;   // lookup product (lookup_product.cuh): spread table, tile products and tile constants
+  uint64_t lp_ws_bytes = 0;
   // device-side batch check (batch_check.cuh)
   uint32_t *d_chk_gate_on = nullptr, *d_chk_pairs = nullptr, *d_chk_out_bytes = nullptr;
   uint64_t *d_chk_fixed = nullptr, *d_chk_bytes = nullptr;
@@ -1777,7 +1779,7 @@ void h2sha_destroy(h2sha_engine_t* e) {
     if (H.copied) cudaEventDestroy(H.copied);
   if (e->pinned_arena) cudaFreeHost(e->pinned_arena);
   for (int i = 0; i < 4; i++) if (e->ev[i]) cudaEventDestroy(e->ev[i]);
-  cudaFree(e->d_lk_ws); cudaFree(e->d_lk_tab); cudaFree(e->d_range_tab); cudaFree(e->d_lookup_raw); cudaFree(e->d_dense_raw);
+  cudaFree(e->d_lk_ws); cudaFree(e->d_lk_tab); cudaFree(e->d_range_tab); cudaFree(e->d_lp_ws); cudaFree(e->d_lookup_raw); cudaFree(e->d_dense_raw);
   cudaFree(e->d_chk_gate_on); cudaFree(e->d_chk_pairs); cudaFree(e->d_chk_out_bytes); cudaFree(e->d_chk_fixed); cudaFree(e->d_chk_bytes); cudaFree(e->d_chk_viol);
   delete e;
 }
@@ -2136,6 +2138,7 @@ int h2sha_last_kernel_ms(h2sha_engine_t* e, float* trace_ms, float* expand_ms) {
 
 #include "lookup_prework.cuh"
 #include "batch_check.cuh"
+#include "lookup_product.cuh"
 #include "export.cuh"
 
 void h2sha_free_compact_state(h2sha_compact_state* s) { delete s; }

@@ -87,6 +87,13 @@ class Sha256DynamicConfig {
     check(h2sha_permute_lookup(engine_, n_instances, lookup_idx, mult_dev, usable_rows, theta_mont, permuted_input_dev, permuted_table_dev,
                                errors_dev, stream));
   }
+  // grand-product column z [n_instances][usable_rows + 1] of one lookup (halo2 `commit_product`); beta / gamma / theta on the host
+  void lookup_product(uint64_t n_instances, uint32_t lookup_idx, const void* lookup, const void* spread, const void* permuted_input_dev,
+                      const void* permuted_table_dev, uint32_t usable_rows, const uint64_t* theta_mont, const uint64_t* beta_mont,
+                      const uint64_t* gamma_mont, void* z_dev, uint32_t* errors_dev, void* stream) {
+    check(h2sha_lookup_product(engine_, n_instances, lookup_idx, lookup, spread, permuted_input_dev, permuted_table_dev, usable_rows, theta_mont,
+                               beta_mont, gamma_mont, z_dev, errors_dev, stream));
+  }
   // MockProver-style check of every instance of a batch on the device (lib.rs:525-526): violations[5] = gates, copies,
   // range lookups, spread lookups, digest bytes
   void check_batch(uint64_t n_instances, const void* gate, const void* lookup, const void* spread, const uint8_t* digests_dev,

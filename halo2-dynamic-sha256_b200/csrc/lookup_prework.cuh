@@ -422,6 +422,30 @@ bool u256_less(const U256& a, const U256& b) {
   return false;
 }
 
+// the range table's values in Montgomery form (e->d_range_tab), built on first use
+int ensure_range_tab(h2sha_engine* e, cudaStream_t st) {
+  if (e->d_range_tab) return H2SHA_OK;
+  const uint32_t n_vals = 1u << e->plan.cfg.lookup_bits;
+  CUDA_TRY(cudaMalloc(&e->d_range_tab, (size_t)n_vals * 32));
+  k_range_table<<<(n_vals + 255) / 256, 256, 0, st>>>(e->d_range_tab, n_vals);
+  CUDA_TRY(cudaGetLastError());
+  CUDA_TRY(cudaStreamSynchronize(st));   // one-time: later calls may come on another stream
+  return H2SHA_OK;
+}
+
+// compressed table expression dense * theta + spread of every spread-table row (halo2 `compress_expressions`), Montgomery form,
+// in table-row order: 2^num_bits_lookup field multiplications, done on the host with the plan-time helpers
+std::vector<U256> compressed_spread_table(const U256& theta_mont, uint32_t limb_bits) {
+  static const U256 r2 = fr::to_mont(fr::mont_r());   // R^2 mod p: mont_mul(v, r2) = Montgomery form of v
+  std::vector<U256> rows(1u << limb_bits);
+  for (uint32_t i = 0; i < rows.size(); i++) {
+    uint64_t sp = 0;
+    for (uint32_t b = 0; b < limb_bits; b++) sp |= (uint64_t)((i >> b) & 1u) << (2 * b);   // spread.rs:171-180
+    rows[i] = fr::add(fr::mont_mul(theta_mont, fr::mont_mul(fr::from_u64(i), r2)), fr::mont_mul(fr::from_u64(sp), r2));
+  }
+  return rows;
+}
+
 }  // namespace
 
 extern "C" {
@@ -529,25 +553,18 @@ int permute_lookup_impl(h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup
   A.errors = errors_dev;
   A.out_input = (uint64_t*)permuted_input_dev; A.out_table = (uint64_t*)permuted_table_dev;
   if (is_range) {
-    if (!e->d_range_tab) {
-      CUDA_TRY(cudaMalloc(&e->d_range_tab, (size_t)n_vals * 32));
-      k_range_table<<<(n_vals + 255) / 256, 256, 0, st>>>(e->d_range_tab, n_vals);
-      CUDA_TRY(cudaGetLastError());
-      CUDA_TRY(cudaStreamSynchronize(st));   // one-time: later calls may come on another stream
-    }
+    int rc = ensure_range_tab(e, st);
+    if (rc) return rc;
     A.vals = tune_value("lktab", 1) ? e->d_range_tab : nullptr;   // lktab=0: convert each value on the fly (mont_from_u32) instead of the 32-byte gather
   } else {
-    // compressed table expression dense * theta + spread (halo2 `compress_expressions`), sorted by canonical value
-    // (`impl Ord for Fr`): 2^num_bits_lookup field multiplications, done on the host with the plan-time helpers
+    // the compressed table rows sorted by canonical value (`impl Ord for Fr`)
     U256 th_m; memcpy(th_m.l, theta_mont, 32);
     if (fr::geq_p(th_m.l)) return set_err(H2SHA_EINVAL, "theta is not a reduced field element");
-    static const U256 r2 = fr::to_mont(fr::mont_r());   // R^2 mod p: mont_mul(v, r2) = Montgomery form of v
+    const std::vector<U256> cm = compressed_spread_table(th_m, G.limb_bits);
     struct Row { U256 c, cm; uint32_t row; };
     std::vector<Row> rows(n_vals);
     for (uint32_t i = 0; i < n_vals; i++) {
-      uint64_t sp = 0;
-      for (uint32_t b = 0; b < G.limb_bits; b++) sp |= (uint64_t)((i >> b) & 1u) << (2 * b);   // spread.rs:171-180
-      rows[i].cm = fr::add(fr::mont_mul(th_m, fr::mont_mul(fr::from_u64(i), r2)), fr::mont_mul(fr::from_u64(sp), r2));
+      rows[i].cm = cm[i];
       rows[i].c = fr::mont_mul(rows[i].cm, fr::from_u64(1));   // canonical value: what `Ord` compares
       rows[i].row = i;
     }
@@ -559,7 +576,7 @@ int permute_lookup_impl(h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup
       host[8 * n_vals + i] = rows[i].row;
       memcpy(&host[8 * i], rows[i].cm.l, 32);
     }
-    if (!e->d_lk_tab) CUDA_TRY(cudaMalloc(&e->d_lk_tab, (size_t)(1u << 8) * 9 * 4));
+    if (!e->d_lk_tab) CUDA_TRY(cudaMalloc(&e->d_lk_tab, host.size() * 4));   // n_vals = 2^num_bits_lookup: fixed per engine
     CUDA_TRY(cudaMemcpyAsync(e->d_lk_tab, host.data(), host.size() * 4, cudaMemcpyHostToDevice, st));   // pageable: staged before return
     A.vals = e->d_lk_tab; A.order = e->d_lk_tab + 8 * n_vals;
   }

@@ -234,6 +234,25 @@ int h2sha_permute_lookup(h2sha_engine_t* e, uint64_t n_instances, uint32_t looku
 int h2sha_permute_lookup_from_raw(h2sha_engine_t* e, uint64_t first_instance, uint64_t n_instances, uint32_t lookup_idx, uint32_t usable_rows,
                                   const uint64_t* theta_mont, void* permuted_input_dev, void* permuted_table_dev, uint32_t* errors_dev, void* stream);
 
+/* The grand-product column z of lookup `lookup_idx` for every instance, once beta and gamma are drawn (halo2_proofs
+ * plonk/lookup/prover.rs `Permuted::commit_product`), with A / S the (theta-compressed) input and table expressions and
+ * A' / S' the permuted pair:
+ *   u_i = (A[i] + beta)(S[i] + gamma),  v_i = (A'[i] + beta)(S'[i] + gamma),  z[0] = 1,  z[j+1] = z[j] * u_j / v_j,  j < usable_rows.
+ * A row with v_i = 0 has the fraction 0 (ff's batch_invert leaves a zero as zero), so every later z is 0.
+ *   lookup / spread        the batch buffers of h2sha_digest_batch; only the one this lookup reads is needed (the other may be NULL)
+ *   permuted_input_dev / permuted_table_dev   [n_instances][usable_rows] Fr (device): A', S', e.g. from h2sha_permute_lookup
+ *   theta_mont / beta_mont / gamma_mont       host, 4 x u64 Montgomery, reduced (< p) or H2SHA_EINVAL; theta only for spread lookups
+ *   z_dev                  [n_instances][usable_rows + 1] Fr (device): z[0 .. usable_rows]; the blinding rows after them are the prover's
+ *   errors_dev             device u32, may be NULL: incremented for every instance whose z[usable_rows] != 1 (A', S' are then no
+ *                          permutation of the input and table expressions, or a denominator was 0)
+ * Instance i of the four device buffers belongs together: a slice of a batch is passed by offsetting all of them.  Fr buffers
+ * must be 32-byte aligned.  Every num_bits_lookup works (the table's compressed values are computed per call).  Asynchronous on
+ * `stream`. */
+int h2sha_lookup_product(h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup_idx, const void* lookup, const void* spread,
+                         const void* permuted_input_dev, const void* permuted_table_dev, uint32_t usable_rows,
+                         const uint64_t* theta_mont, const uint64_t* beta_mont, const uint64_t* gamma_mont,
+                         void* z_dev, uint32_t* errors_dev, void* stream);
+
 /* MockProver-style check of a whole batch where it lies, in HBM -- what the reference's tests accept a witness by
  * (`MockProver::run(..).verify() == Ok(())`, lib.rs:525-526), for every instance instead of one:
  *   violations[0] gates           q * (a + b*c - d) = 0 on every enabled gate row (halo2-base FlexGate, Vertical)
