@@ -29,7 +29,7 @@ H2SHA_OK, H2SHA_EINVAL, H2SHA_EPANIC, H2SHA_ECUDA, H2SHA_ENOMEM = 0, -1, -2, -3,
 # symbols include/h2sha_b200.h declares (checked by tests/test_abi.py)
 EXPORTED_SYMBOLS = [
     "h2sha_create", "h2sha_destroy", "h2sha_last_error", "h2sha_build_id", "h2sha_get_layout", "h2sha_get_breaks", "h2sha_get_handles", "h2sha_get_digest_ranges", "h2sha_get_shape", "h2sha_get_lookup_tables",
-    "h2sha_digest_batch", "h2sha_export_instance", "h2sha_export_batch", "h2sha_get_compact_info", "h2sha_get_compact_map", "h2sha_expand_compact", "h2sha_get_lookup_info", "h2sha_lookup_multiplicities", "h2sha_permute_lookup", "h2sha_permute_lookup_from_raw", "h2sha_lookup_product", "h2sha_check_batch", "h2sha_gather", "h2sha_zero_outputs", "h2sha_debug_mont_from_u64", "h2sha_debug_mont_from_u32", "h2sha_debug_store_probe", "h2sha_debug_int_probe", "h2sha_last_launch_count", "h2sha_last_kernel_ms", "H2SHA_CK_M",
+    "h2sha_digest_batch", "h2sha_export_instance", "h2sha_export_batch", "h2sha_get_compact_info", "h2sha_get_compact_map", "h2sha_expand_compact", "h2sha_get_lookup_info", "h2sha_lookup_multiplicities", "h2sha_permute_lookup", "h2sha_permute_lookup_from_raw", "h2sha_lookup_product", "h2sha_get_permutation", "h2sha_permutation_product", "h2sha_check_batch", "h2sha_gather", "h2sha_zero_outputs", "h2sha_debug_mont_from_u64", "h2sha_debug_mont_from_u32", "h2sha_debug_store_probe", "h2sha_debug_int_probe", "h2sha_last_launch_count", "h2sha_last_kernel_ms", "H2SHA_CK_M",
 ]
 
 
@@ -66,6 +66,15 @@ class _Batch(C.Structure):
                 ("checksums_host", C.c_void_p), ("stream", C.c_void_p), ("reuse_inputs", C.c_int32), ("time_kernels", C.c_int32),
                 ("only_digest", C.c_uint32), ("lookup_mult_dev", C.c_void_p), ("mult_usable_rows", C.c_uint32), ("mult_not_in_table_dev", C.c_void_p),
                 ("compact_dict", C.c_void_p), ("keep_lookup_raw", C.c_uint32)]
+
+
+# column kinds of a permutation column list (h2sha_perm_desc_t; numbered like chip::ColumnKind, instance is new)
+COL_GATE, COL_LOOKUP, COL_DENSE, COL_SPREAD, COL_FIXED, COL_INSTANCE = 0, 1, 2, 3, 4, 6
+
+
+class _PermDesc(C.Structure):
+    _fields_ = [("n_columns", C.c_uint32), ("columns", C.c_void_p), ("num_fixed", C.c_uint32), ("columns_per_chunk", C.c_uint32),
+                ("bind_output_bytes", C.c_uint32), ("k", C.c_uint32)]
 
 
 class _CompactInfo(C.Structure):
@@ -122,6 +131,9 @@ def load_library():
     sig("h2sha_permute_lookup_from_raw", [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
     sig("h2sha_lookup_product", [C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p,
                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
+    sig("h2sha_get_permutation", [C.c_void_p, C.POINTER(_PermDesc), C.c_uint32, C.c_void_p])
+    sig("h2sha_permutation_product", [C.c_void_p, C.c_uint64, C.POINTER(_PermDesc), C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                      C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
     sig("h2sha_check_batch", [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
     sig("h2sha_gather", [C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
     sig("h2sha_zero_outputs", [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p])
@@ -514,6 +526,51 @@ class Sha256DynamicConfig:
         _check(load_library().h2sha_lookup_product(self._h, n, lookup_idx, ptr(res.lookup), ptr(res.spread), a_p.data_ptr(), s_p.data_ptr(), usable_rows,
                                                    *[x.ctypes.data if x is not None else None for x in ch], z.data_ptr(), err.data_ptr(),
                                                    torch.cuda.current_stream(self.device).cuda_stream))
+        return z, int(err.item())
+
+    # ---- permutation argument (halo2 plonk/permutation: keygen Assembly, prover `Argument::commit`) ----
+    @staticmethod
+    def _perm_desc(columns, num_fixed: int, columns_per_chunk: int, bind_output_bytes: bool, k: int):
+        cols = np.ascontiguousarray(np.asarray(columns, dtype=np.uint32).reshape(-1, 2))
+        return _PermDesc(len(cols), cols.ctypes.data, num_fixed, columns_per_chunk, 1 if bind_output_bytes else 0, k), cols
+
+    def permutation_mapping(self, columns, usable_rows: int, *, columns_per_chunk: int, num_fixed: int = 1, bind_output_bytes: bool = False,
+                            k: int = 0) -> np.ndarray:
+        """halo2 keygen `Assembly` mapping of the chip's copy constraints: [len(columns), usable_rows, 2] u32 (column position, row).
+        `columns`: (kind, index) pairs (COL_*) in the order of `cs.permutation.columns`.  Works on a plan-only configuration
+        (device=-1, build_shape=True)."""
+        d, cols = self._perm_desc(columns, num_fixed, columns_per_chunk, bind_output_bytes, k)
+        m = np.zeros((len(cols), usable_rows, 2), dtype=np.uint32)
+        _check(load_library().h2sha_get_permutation(self._h, C.byref(d), usable_rows, m.ctypes.data_as(C.c_void_p)))
+        return m
+
+    def permutation_product(self, res: "BatchResult", columns, usable_rows: int, beta_mont: np.ndarray, gamma_mont: np.ndarray, *,
+                            columns_per_chunk: int, num_fixed: int = 1, bind_output_bytes: bool = False, digests=None, k: int = 0):
+        """(z [n_inst, n_chunks, usable_rows + 1, 4] int64 device tensor, instances whose last z[usable_rows] != 1): the permutation
+        argument's product columns (halo2 `permutation::prover` commit) of a batch's witness `res`.  `digests` ([n_msgs, 32] u8, host
+        array or device tensor) fills the instance column; needed only with bind_output_bytes."""
+        import torch
+        n = res.gate.shape[0]
+        for buf in (res.lookup, res.spread):
+            if buf is not None and buf.shape[0] < n:
+                raise EngineError(H2SHA_EINVAL, "the witness buffers hold different numbers of instances")
+        d, cols = self._perm_desc(columns, num_fixed, columns_per_chunk, bind_output_bytes, k)
+        dev = torch.device("cuda", self.device)
+        n_chunks = -(-len(cols) // columns_per_chunk) if columns_per_chunk else 0
+        z = torch.empty((n, n_chunks, usable_rows + 1, 4), dtype=torch.int64, device=dev)
+        err = torch.zeros(1, dtype=torch.int32, device=dev)
+        dg = None
+        if digests is not None:
+            dg = digests if isinstance(digests, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(digests, dtype=np.uint8))
+            dg = dg.to(dev).contiguous()
+            if dg.numel() < n * 32 * len(self.max_variable_byte_sizes):
+                raise EngineError(H2SHA_EINVAL, "digests holds fewer messages than the batch")
+        bg = [np.ascontiguousarray(x, dtype=np.uint64) for x in (beta_mont, gamma_mont)]
+        assert all(x.shape == (4,) for x in bg)
+        ptr = lambda t: t.data_ptr() if t is not None else None
+        _check(load_library().h2sha_permutation_product(self._h, n, C.byref(d), usable_rows, ptr(res.gate), ptr(res.lookup), ptr(res.spread), ptr(dg),
+                                                        bg[0].ctypes.data, bg[1].ctypes.data, z.data_ptr(), err.data_ptr(),
+                                                        torch.cuda.current_stream(self.device).cuda_stream))
         return z, int(err.item())
 
     def launches_last_batch(self) -> int:

@@ -30,6 +30,7 @@
 
 #include "../../include/h2sha_b200.h"
 #include "h2sha_defs.h"
+#include "permutation.h"
 #include "planner.h"
 
 using namespace h2sha;
@@ -1435,6 +1436,7 @@ struct HostSlot {
 enum { H2SHA_N_SETS = 2, H2SHA_N_SLOTS = 8 };
 
 struct h2sha_compact_state;   // export.cuh
+struct h2sha_perm_state;      // permutation_product.cuh
 
 struct h2sha_engine {
   Plan plan;
@@ -1482,6 +1484,8 @@ struct h2sha_engine {
   uint32_t n_chk_gate_on = 0, n_chk_pairs = 0;
   // compact hand-off (export.cuh): the cell -> dictionary-entry map, planned on first use
   h2sha_compact_state* compact = nullptr;
+  // permutation product (permutation_product.cuh): the moved cells of the last column list, planned on first use
+  h2sha_perm_state* perm = nullptr;
 };
 
 namespace {
@@ -1760,6 +1764,7 @@ int h2sha_create(const h2sha_config_t* cfg, h2sha_engine_t** out) {
 }
 
 void h2sha_free_compact_state(h2sha_compact_state* s);   // defined after export.cuh (complete type)
+void h2sha_free_perm_state(h2sha_perm_state* s);         // permutation_product.cuh
 
 void h2sha_destroy(h2sha_engine_t* e) {
   if (!e) return;
@@ -1780,6 +1785,7 @@ void h2sha_destroy(h2sha_engine_t* e) {
   if (e->pinned_arena) cudaFreeHost(e->pinned_arena);
   for (int i = 0; i < 4; i++) if (e->ev[i]) cudaEventDestroy(e->ev[i]);
   cudaFree(e->d_lk_ws); cudaFree(e->d_lk_tab); cudaFree(e->d_range_tab); cudaFree(e->d_lp_ws); cudaFree(e->d_lookup_raw); cudaFree(e->d_dense_raw);
+  h2sha_free_perm_state(e->perm); e->perm = nullptr;
   cudaFree(e->d_chk_gate_on); cudaFree(e->d_chk_pairs); cudaFree(e->d_chk_out_bytes); cudaFree(e->d_chk_fixed); cudaFree(e->d_chk_bytes); cudaFree(e->d_chk_viol);
   delete e;
 }
@@ -2139,6 +2145,7 @@ int h2sha_last_kernel_ms(h2sha_engine_t* e, float* trace_ms, float* expand_ms) {
 #include "lookup_prework.cuh"
 #include "batch_check.cuh"
 #include "lookup_product.cuh"
+#include "permutation_product.cuh"
 #include "export.cuh"
 
 void h2sha_free_compact_state(h2sha_compact_state* s) { delete s; }

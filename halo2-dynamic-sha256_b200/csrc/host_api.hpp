@@ -94,6 +94,20 @@ class Sha256DynamicConfig {
     check(h2sha_lookup_product(engine_, n_instances, lookup_idx, lookup, spread, permuted_input_dev, permuted_table_dev, usable_rows, theta_mont,
                                beta_mont, gamma_mont, z_dev, errors_dev, stream));
   }
+  // ---- permutation argument (copy constraints; halo2 plonk/permutation) ----
+  // keygen Assembly mapping [desc.n_columns][usable_rows][2] (column position, row); works on a plan-only engine with build_shape
+  std::vector<uint32_t> permutation_mapping(const h2sha_perm_desc_t& desc, uint32_t usable_rows) const {
+    std::vector<uint32_t> m((size_t)desc.n_columns * usable_rows * 2);
+    check(h2sha_get_permutation(engine_, &desc, usable_rows, m.data()));
+    return m;
+  }
+  // product columns z [n_instances][n_chunks][usable_rows + 1] (halo2 `permutation::prover` commit); beta / gamma on the host
+  void permutation_product(uint64_t n_instances, const h2sha_perm_desc_t& desc, uint32_t usable_rows, const void* gate, const void* lookup,
+                           const void* spread, const uint8_t* digests_dev, const uint64_t* beta_mont, const uint64_t* gamma_mont, void* z_dev,
+                           uint32_t* errors_dev, void* stream) {
+    check(h2sha_permutation_product(engine_, n_instances, &desc, usable_rows, gate, lookup, spread, digests_dev, beta_mont, gamma_mont, z_dev,
+                                    errors_dev, stream));
+  }
   // MockProver-style check of every instance of a batch on the device (lib.rs:525-526): violations[5] = gates, copies,
   // range lookups, spread lookups, digest bytes
   void check_batch(uint64_t n_instances, const void* gate, const void* lookup, const void* spread, const uint8_t* digests_dev,

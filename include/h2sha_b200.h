@@ -253,6 +253,56 @@ int h2sha_lookup_product(h2sha_engine_t* e, uint64_t n_instances, uint32_t looku
                          const uint64_t* theta_mont, const uint64_t* beta_mont, const uint64_t* gamma_mont,
                          void* z_dev, uint32_t* errors_dev, void* stream);
 
+/* ---- Permutation argument (copy constraints): halo2_proofs plonk/permutation ------------------------------------------
+ * The columns with equality enabled, in the order of `cs.permutation.columns` (the order of the enable_equality calls), as
+ * (kind, index) pairs.  Kinds are numbered like chip::ColumnKind (csrc/chip_api.hpp); the instance column is new. */
+#define H2SHA_COL_GATE 0u      /* gate advice column `index` (< n_gate_cols)                                       */
+#define H2SHA_COL_LOOKUP 1u    /* lookup advice column `index` (< n_lookup_cols)                                   */
+#define H2SHA_COL_DENSE 2u     /* SpreadConfig denses[index] (< num_advice_columns)                                */
+#define H2SHA_COL_SPREAD 3u    /* SpreadConfig spreads[index]                                                      */
+#define H2SHA_COL_FIXED 4u     /* fixed (constants) column `index` (< num_fixed)                                   */
+#define H2SHA_COL_INSTANCE 6u  /* the instance column (index 0) the output bytes are bound to                      */
+typedef struct {
+  uint32_t n_columns;
+  const uint32_t* columns;      /* [n_columns][2] (kind, index): every column the chip copies from or to, each once        */
+  uint32_t num_fixed;           /* fixed columns Context::assign_fixed fills round-robin (constant k -> column k % num_fixed,
+                                   row k / num_fixed); 0 -> 1                                                            */
+  uint32_t columns_per_chunk;   /* cs.degree() - 2: columns per product column z                                          */
+  uint32_t bind_output_bytes;   /* 1: constrain_instance(output_bytes[i], instance, i) for the 32 * n_digests output bytes
+                                   in order (the reference's TestCircuit, lib.rs:480-482); the list then has the instance
+                                   column, and only then                                                                 */
+  uint32_t k;                   /* domain size 2^k; 0 -> the smallest 2^k > usable_rows + 1                              */
+} h2sha_perm_desc_t;
+
+/* Keygen half: the permutation mapping halo2's `permutation::keygen::Assembly` builds from the chip's copy constraints, replayed
+ * in the order the chip API issues them (chip_api.hpp `assign_digest`: per digest() call its shape copies, then per spread limb
+ * the dense and the spread copy; then range.finalize's lookup copies; then the instance binding).  Region rows = circuit rows
+ * (the region starts at row 0).  mapping: [n_columns][usable_rows][2] u32 (column position in desc->columns, row), or NULL to
+ * validate only.  sigma_c(w^r) = delta^c' w^r' with (c', r') = mapping[c][r].  Works on a plan-only engine (device = -1); needs
+ * build_shape.  H2SHA_EINVAL when a column the chip copies is missing, a column is listed twice or out of range, an assigned
+ * cell lies at or above usable_rows, or columns_per_chunk == 0. */
+int h2sha_get_permutation(h2sha_engine_t* e, const h2sha_perm_desc_t* desc, uint32_t usable_rows, uint32_t* mapping);
+
+/* The permutation argument's product columns for every instance, once beta and gamma are drawn (halo2_proofs
+ * plonk/permutation/prover.rs `Argument::commit` without the blinding rows): chunk h covers columns [h*m, min(C, (h+1)*m)),
+ * m = columns_per_chunk, and with one deltaomega running over all columns,
+ *   z_h[0] = z_{h-1}[U] (1 for h = 0),  z_h[i+1] = z_h[i] * prod_j (p_j(w^i) + beta delta^j w^i + gamma) / prod_j (p_j(w^i) + beta sigma_j(w^i) + gamma)
+ * for i < U = usable_rows.  A zero denominator gives the fraction 0 (ff's batch_invert leaves a zero as zero), so the rest of
+ * that chunk and every later chunk is 0.  The fixed column holds the shape's constants at their round-robin rows and 0 elsewhere;
+ * the instance column holds byte i of the instance's digests at row i and 0 above.
+ *   gate / lookup / spread    the batch buffers of h2sha_digest_batch (each may be NULL when no listed column reads it)
+ *   digests_dev               device [n_instances * n_digests][32]; needed only with bind_output_bytes
+ *   beta_mont / gamma_mont    host, 4 x u64 Montgomery, reduced (< p) or H2SHA_EINVAL
+ *   z_dev                     [n_instances][n_chunks][usable_rows + 1] Fr (device, 32-byte aligned), n_chunks = ceil(C / m)
+ *   errors_dev                device u32, may be NULL: incremented for every instance whose last chunk ends with z[U] != 1
+ * Only cells whose sigma is not the identity enter the products; a cell with sigma = id contributes exactly 1.  The one departure
+ * from halo2: a zero term p + beta delta^j w^i + gamma at such a cell (probability ~2^-230 over beta, gamma) is taken as 1 where
+ * halo2 would zero the fraction.  The moved cells are planned once per (desc, usable_rows) and kept on the device.  Asynchronous
+ * on `stream` after the first call for a desc. */
+int h2sha_permutation_product(h2sha_engine_t* e, uint64_t n_instances, const h2sha_perm_desc_t* desc, uint32_t usable_rows,
+                              const void* gate, const void* lookup, const void* spread, const uint8_t* digests_dev,
+                              const uint64_t* beta_mont, const uint64_t* gamma_mont, void* z_dev, uint32_t* errors_dev, void* stream);
+
 /* MockProver-style check of a whole batch where it lies, in HBM -- what the reference's tests accept a witness by
  * (`MockProver::run(..).verify() == Ok(())`, lib.rs:525-526), for every instance instead of one:
  *   violations[0] gates           q * (a + b*c - d) = 0 on every enabled gate row (halo2-base FlexGate, Vertical)

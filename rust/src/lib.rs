@@ -26,7 +26,7 @@ use halo2_base::gates::range::RangeConfig;
 use halo2_base::halo2_proofs::{
     circuit::{Cell, Layouter, Region, Value},
     halo2curves::bn256::Fr,
-    plonk::{Advice, Column, ConstraintSystem, Error, TableColumn},
+    plonk::{Advice, Any, Column, ConstraintSystem, Error, Instance, TableColumn},
     poly::Rotation,
 };
 use halo2_base::{AssignedValue, Context, ContextParams};
@@ -329,6 +329,39 @@ impl Sha256DynamicConfig {
     }
 }
 
+impl Sha256DynamicConfig {
+    /// The permutation argument's column list for `h2sha_perm_desc_t`: `meta`'s equality-enabled columns in the order of
+    /// `cs.permutation.columns`, each as (H2SHA_COL_* kind, index) of the chip's columns; `instance` is the column the output bytes
+    /// are bound to (`constrain_instance`), if any.  Panics on an equality column the chip does not own.
+    pub fn permutation_columns(&self, meta: &ConstraintSystem<Fr>, instance: Option<Column<Instance>>) -> Vec<[u32; 2]> {
+        let gates: Vec<Column<Any>> = self.range.gate.basic_gates[0].iter().map(|g| g.value.into()).collect(); // CHECK: BasicGateConfig.value
+        let lookups: Vec<Column<Any>> = self.range.lookup_advice[0].iter().map(|c| (*c).into()).collect(); // CHECK: RangeConfig.lookup_advice
+        let fixed: Vec<Column<Any>> = self.range.gate.constants.iter().map(|c| (*c).into()).collect(); // CHECK: FlexGateConfig.constants
+        let denses: Vec<Column<Any>> = self.spread.denses.iter().map(|c| (*c).into()).collect();
+        let spreads: Vec<Column<Any>> = self.spread.spreads.iter().map(|c| (*c).into()).collect();
+        let inst: Option<Column<Any>> = instance.map(|c| c.into());
+        meta.permutation().get_columns().into_iter() // CHECK: ConstraintSystem::permutation() / permutation::Argument::get_columns()
+            .map(|col| {
+                let pos = |v: &[Column<Any>]| v.iter().position(|c| *c == col).map(|i| i as u32);
+                if let Some(i) = pos(&gates) { [H2SHA_COL_GATE, i] }
+                else if let Some(i) = pos(&lookups) { [H2SHA_COL_LOOKUP, i] }
+                else if let Some(i) = pos(&denses) { [H2SHA_COL_DENSE, i] }
+                else if let Some(i) = pos(&spreads) { [H2SHA_COL_SPREAD, i] }
+                else if let Some(i) = pos(&fixed) { [H2SHA_COL_FIXED, i] }
+                else if inst == Some(col) { [H2SHA_COL_INSTANCE, 0] }
+                else { panic!("equality-enabled column {col:?} is none of the chip's") }
+            })
+            .collect()
+    }
+
+    /// keygen `Assembly` mapping of the chip's copy constraints: per listed column and usable row, (column position, row).
+    pub fn permutation_mapping(&self, desc: &h2sha_perm_desc_t, usable_rows: u32) -> Result<Vec<[u32; 2]>, Error> {
+        let mut m = vec![[0u32; 2]; desc.n_columns as usize * usable_rows as usize];
+        check(unsafe { h2sha_get_permutation(self.engine, desc, usable_rows, m.as_mut_ptr() as *mut u32) })?;
+        Ok(m)
+    }
+}
+
 impl Drop for Sha256DynamicConfig {
     fn drop(&mut self) { unsafe { h2sha_destroy(self.engine) } }
 }
@@ -340,6 +373,14 @@ pub mod batch {
     pub fn gather(comm: *mut std::ffi::c_void, n_per_rank: usize, n_digests: u32, digests: u64, checksums: u64, all_digests: u64, all_checksums: u64,
                   stream: *mut std::ffi::c_void) -> Result<(), Error> {
         check(unsafe { h2sha_gather(comm, n_per_rank as u64, n_digests, digests as *const u8, checksums as *const u64, all_digests as *mut u8, all_checksums as *mut u64, stream) })
+    }
+    /// halo2 `permutation::prover` commit without the blinding rows, for every instance of a batch: z [n][n_chunks][usable_rows + 1]
+    /// Fr at `z_dev`; beta / gamma as Montgomery limbs (the memory layout of halo2curves bn256::Fr).
+    pub fn permutation_product(engine: *mut h2sha_engine_t, n: usize, desc: &h2sha_perm_desc_t, usable_rows: u32, gate: u64, lookup: u64, spread: u64,
+                               digests_dev: u64, beta_mont: &[u64; 4], gamma_mont: &[u64; 4], z_dev: u64, errors_dev: u64,
+                               stream: *mut std::ffi::c_void) -> Result<(), Error> {
+        check(unsafe { h2sha_permutation_product(engine, n as u64, desc, usable_rows, gate as *const _, lookup as *const _, spread as *const _,
+                                                 digests_dev as *const u8, beta_mont.as_ptr(), gamma_mont.as_ptr(), z_dev as *mut _, errors_dev as *mut u32, stream) })
     }
     /// `MockProver::run(..).verify()` (lib.rs:525-526) for every instance of a batch, on the device.
     pub fn check_batch(engine: *mut h2sha_engine_t, n: usize, gate: u64, lookup: u64, spread: u64, digests_dev: u64, stream: *mut std::ffi::c_void) -> Result<[u64; 5], Error> {
