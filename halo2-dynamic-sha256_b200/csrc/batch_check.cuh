@@ -15,60 +15,6 @@
 
 namespace {
 
-// Montgomery product a * b * 2^-256 mod p (CIOS), inputs < p
-__device__ __forceinline__ void mont_mul_dev(const uint64_t a[4], const uint64_t b[4], uint64_t r[4]) {
-  typedef unsigned __int128 u128;
-  const uint64_t P0 = c_fr.p[0], P1 = c_fr.p[1], P2 = c_fr.p[2], P3 = c_fr.p[3];
-  uint64_t t0 = 0, t1 = 0, t2 = 0, t3 = 0, t4 = 0;
-#pragma unroll
-  for (int i = 0; i < 4; i++) {
-    u128 c = (u128)a[0] * b[i] + t0; t0 = (uint64_t)c;
-    c = (u128)a[1] * b[i] + t1 + (uint64_t)(c >> 64); t1 = (uint64_t)c;
-    c = (u128)a[2] * b[i] + t2 + (uint64_t)(c >> 64); t2 = (uint64_t)c;
-    c = (u128)a[3] * b[i] + t3 + (uint64_t)(c >> 64); t3 = (uint64_t)c;
-    c = (u128)t4 + (uint64_t)(c >> 64);
-    t4 = (uint64_t)c;
-    const uint64_t t5 = (uint64_t)(c >> 64);
-    const uint64_t m = t0 * c_fr_ninv;
-    c = (u128)m * P0 + t0;
-    c = (u128)m * P1 + t1 + (uint64_t)(c >> 64); t0 = (uint64_t)c;
-    c = (u128)m * P2 + t2 + (uint64_t)(c >> 64); t1 = (uint64_t)c;
-    c = (u128)m * P3 + t3 + (uint64_t)(c >> 64); t2 = (uint64_t)c;
-    c = (u128)t4 + (uint64_t)(c >> 64);
-    t3 = (uint64_t)c;
-    t4 = t5 + (uint64_t)(c >> 64);
-  }
-  uint64_t s0, s1, s2, s3, borrow;
-  asm("sub.cc.u64 %0, %5, %9;\n\t"
-      "subc.cc.u64 %1, %6, %10;\n\t"
-      "subc.cc.u64 %2, %7, %11;\n\t"
-      "subc.cc.u64 %3, %8, %12;\n\t"
-      "subc.u64 %4, %13, 0;"
-      : "=l"(s0), "=l"(s1), "=l"(s2), "=l"(s3), "=l"(borrow)
-      : "l"(t0), "l"(t1), "l"(t2), "l"(t3), "l"(P0), "l"(P1), "l"(P2), "l"(P3), "l"(t4));
-  if ((borrow >> 63) == 0) { t0 = s0; t1 = s1; t2 = s2; t3 = s3; }   // t >= p (t4 carries the 257th bit)
-  r[0] = t0; r[1] = t1; r[2] = t2; r[3] = t3;
-}
-
-// (x + y) mod p and (x - y) mod p for x, y < p
-__device__ __forceinline__ void fr_add_dev(const uint64_t x[4], const uint64_t y[4], uint64_t r[4]) {
-  typedef unsigned __int128 u128;
-  u128 c = (u128)x[0] + y[0]; uint64_t t0 = (uint64_t)c;
-  c = (u128)x[1] + y[1] + (uint64_t)(c >> 64); uint64_t t1 = (uint64_t)c;
-  c = (u128)x[2] + y[2] + (uint64_t)(c >> 64); uint64_t t2 = (uint64_t)c;
-  c = (u128)x[3] + y[3] + (uint64_t)(c >> 64); uint64_t t3 = (uint64_t)c;   // p < 2^254: no carry out
-  uint64_t s0, s1, s2, s3, borrow;
-  asm("sub.cc.u64 %0, %5, %9;\n\t"
-      "subc.cc.u64 %1, %6, %10;\n\t"
-      "subc.cc.u64 %2, %7, %11;\n\t"
-      "subc.cc.u64 %3, %8, %12;\n\t"
-      "subc.u64 %4, 0, 0;"
-      : "=l"(s0), "=l"(s1), "=l"(s2), "=l"(s3), "=l"(borrow)
-      : "l"(t0), "l"(t1), "l"(t2), "l"(t3), "l"(c_fr.p[0]), "l"(c_fr.p[1]), "l"(c_fr.p[2]), "l"(c_fr.p[3]));
-  if (borrow == 0) { t0 = s0; t1 = s1; t2 = s2; t3 = s3; }
-  r[0] = t0; r[1] = t1; r[2] = t2; r[3] = t3;
-}
-
 struct CheckArgs {
   uint64_t gate_inst_cells, lookup_inst_cells, spread_inst_cells;
   const uint64_t* gate;
@@ -215,9 +161,8 @@ int h2sha_check_batch(h2sha_engine_t* e, uint64_t n_instances, const void* gate,
   memset(violations_host, 0, 5 * 8);
   if (n_instances == 0) return H2SHA_OK;
   CUDA_TRY(cudaSetDevice(e->device));
-  int rc = ensure_lookup_consts(e);
+  int rc = ensure_check_tables(e);
   if (rc) return rc;
-  if ((rc = ensure_check_tables(e))) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   const Plan& P = e->plan;
   CheckArgs A{};

@@ -17,40 +17,6 @@
 
 namespace {
 
-__constant__ uint64_t c_fr_ninv;   // -p^-1 mod 2^64 (derived from p at first use)
-
-// Montgomery reduction: x * 2^-256 mod p, canonical (Montgomery form -> the integer the cell stands for)
-__device__ __forceinline__ void mont_reduce(const uint64_t x[4], uint64_t r[4]) {
-  typedef unsigned __int128 u128;
-  uint64_t t0 = x[0], t1 = x[1], t2 = x[2], t3 = x[3];
-  const uint64_t P0 = c_fr.p[0], P1 = c_fr.p[1], P2 = c_fr.p[2], P3 = c_fr.p[3];
-#pragma unroll
-  for (int i = 0; i < 4; i++) {
-    const uint64_t m = t0 * c_fr_ninv;
-    u128 c = (u128)m * P0 + t0;            // low limb becomes 0
-    c = (u128)m * P1 + t1 + (uint64_t)(c >> 64); t0 = (uint64_t)c;
-    c = (u128)m * P2 + t2 + (uint64_t)(c >> 64); t1 = (uint64_t)c;
-    c = (u128)m * P3 + t3 + (uint64_t)(c >> 64); t2 = (uint64_t)c;
-    t3 = (uint64_t)(c >> 64);
-  }
-  // t < 2p: one conditional subtraction
-  uint64_t s0, s1, s2, s3, borrow;
-  asm("sub.cc.u64 %0, %5, %9;\n\t"
-      "subc.cc.u64 %1, %6, %10;\n\t"
-      "subc.cc.u64 %2, %7, %11;\n\t"
-      "subc.cc.u64 %3, %8, %12;\n\t"
-      "subc.u64 %4, 0, 0;"
-      : "=l"(s0), "=l"(s1), "=l"(s2), "=l"(s3), "=l"(borrow)
-      : "l"(t0), "l"(t1), "l"(t2), "l"(t3), "l"(P0), "l"(P1), "l"(P2), "l"(P3));
-  if (borrow == 0) { t0 = s0; t1 = s1; t2 = s2; t3 = s3; }
-  r[0] = t0; r[1] = t1; r[2] = t2; r[3] = t3;
-}
-
-__device__ __forceinline__ void load_cell(const uint64_t* p, uint64_t x[4]) {
-  const ulonglong2 a = reinterpret_cast<const ulonglong2*>(p)[0], b = reinterpret_cast<const ulonglong2*>(p)[1];
-  x[0] = a.x; x[1] = a.y; x[2] = b.x; x[3] = b.y;
-}
-
 struct LookupGeom {
   uint64_t n_inst;
   uint64_t lookup_inst_cells, spread_inst_cells;   // Fr per instance in the lookup / spread buffers
@@ -386,16 +352,6 @@ __global__ void k_range_table(uint32_t* tab, uint32_t n) {
   store_cell2(tab + (uint64_t)i * 8, make_uint4(x[0], x[1], x[2], x[3]), make_uint4(x[4], x[5], x[6], x[7]));
 }
 
-int ensure_lookup_consts(h2sha_engine* e) {
-  if (e->lookup_consts_ready) return H2SHA_OK;
-  uint64_t inv = 1;   // Newton: inv = p^-1 mod 2^64
-  for (int i = 0; i < 6; i++) inv *= 2 - fr::P[0] * inv;
-  const uint64_t ninv = 0 - inv;
-  CUDA_TRY(cudaMemcpyToSymbol(c_fr_ninv, &ninv, 8));
-  e->lookup_consts_ready = true;
-  return H2SHA_OK;
-}
-
 LookupGeom lookup_geom(const h2sha_engine* e, uint64_t n_inst, uint32_t usable_rows) {
   const Plan& P = e->plan;
   LookupGeom G{};
@@ -470,8 +426,6 @@ int h2sha_lookup_multiplicities(h2sha_engine_t* e, uint64_t n_instances, const v
   if (usable_rows < lookup_rows_needed(e->plan)) return set_err(H2SHA_EINVAL, "usable_rows is smaller than an assigned column or a lookup table");
   if (n_instances == 0) return H2SHA_OK;
   CUDA_TRY(cudaSetDevice(e->device));
-  int rc = ensure_lookup_consts(e);
-  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   const LookupGeom G = lookup_geom(e, n_instances, usable_rows);
   const uint64_t range_words = (uint64_t)G.n_lookup_cols << G.lookup_bits;

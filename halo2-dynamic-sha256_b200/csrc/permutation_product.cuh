@@ -1,7 +1,6 @@
 // permutation_product.cuh -- the permutation argument's product columns on the device (PSE halo2_proofs
 // plonk/permutation/prover.rs `Argument::commit`, without the blinding rows) for the chip's copy constraints, for every instance
-// of a batch.  Included at the end of engine.cu after lookup_product.cuh, whose Montgomery and tile helpers it reuses
-// (mont_mul_dev, fr_add_dev, fr_one, store_fr, the shuffles, k_product_fold).
+// of a batch.  Included at the end of engine.cu after grand_product.cuh.
 //
 // Chunk h of the C listed columns covers [h*m, min(C, (h+1)*m)); chunks chain (z_h[0] = z_{h-1}[U]), so the columns of all chunks
 // form ONE sequence of fractions over (chunk, row).  A cell whose sigma is the identity contributes exactly 1 to its row's
@@ -11,13 +10,9 @@
 //                               (buffer and Fr offset in an instance, fixed constant, digest byte), identity delta^j w^r and sigma;
 //                               per chunk a row index ptr[h][0 .. U+1] into that list
 //   k_perm_prep                 per call: a = beta id + gamma, b = beta sigma + gamma per moved cell (shared by all instances)
-//   k_perm_tiles                grid (tiles of all chunks, instances): tile products of u_i = prod (p + a), v_i = prod (p + b)
-//                               over the rows with moved cells
-//   k_product_fold              (lookup_product.cuh) one warp per instance walks the tiles of all chunks in chain order: one
-//                               inversion per instance, per tile C_t = U_<t / V_<=t, the last chunk's z[U] checked against 1
-//   k_perm_fill                 grid (tiles, instances): z[j] = C_t * prod_{t0 <= i < j} u_i * prod_{j <= i < t1} v_i; a warp
-//                               whose 256 rows hold no moved cell only stores its constant
-// Rows run 0 .. U in every chunk (row U has no moved cell), so the fill writes z[0 .. U] of every chunk.
+//   grand_product.cuh           with the row source PermRows: u_i = prod (p + a), v_i = prod (p + b) over the moved cells of a row;
+//                               rows run 0 .. U in every chunk (row U has no moved cell), so the fill writes z[0 .. U] of every
+//                               chunk, and the closing value the fold checks against 1 is the last chunk's z[U]
 // Bound: the integer arithmetic of the rows that hold moved cells, not HBM (z leaves at 0.02-0.04 of the store probe; DESIGN.md §4e).
 // Zero terms: a zero denominator at a moved cell gives the row the fraction 0 (u, v) := (0, 1), like ff's batch_invert.  The
 // one departure from halo2: a zero term p + beta delta^j w^i + gamma at an UNMOVED cell (probability ~2^-230 over beta, gamma) is
@@ -26,11 +21,11 @@
 
 namespace {
 
-enum { PP_THREADS = 256, PP_ROWS = 8, PP_TILE = PP_THREADS * PP_ROWS };
 enum : uint64_t { PS_GATE = 0, PS_LOOKUP = 1, PS_SPREAD = 2, PS_FIXED = 3, PS_BYTE = 4, PS_ZERO = 5 };   // source kind (bits 60..63)
 constexpr uint64_t PS_OFF_MASK = (1ull << 60) - 1;
 
-struct PermArgs {
+// the moved cells of a batch as a row source of grand_product.cuh
+struct PermRows {
   const uint64_t* gate;         // batch buffers at instance 0 of the launch
   const uint64_t* lookup;
   const uint64_t* spread;
@@ -42,10 +37,10 @@ struct PermArgs {
   const uint64_t* src;          // [n_moved] (kind << 60) | offset
   const uint64_t* ab;           // [n_moved][2][4]: beta id + gamma, beta sigma + gamma
   const uint32_t* ptr;          // [n_chunks][U + 2]: first moved cell of each row
-  uint32_t usable_rows, n_chunks, tiles_per_chunk;
-  uint64_t* tiles;              // [n][n_chunks * tiles_per_chunk][2][4]
-  const uint64_t* consts;       // [n][n_chunks * tiles_per_chunk][4]
-  uint64_t* z;                  // [n][n_chunks][U + 1]
+  uint32_t usable_rows;
+
+  __device__ __forceinline__ bool any(uint32_t h, uint32_t i0, uint32_t i1) const;
+  __device__ bool terms(uint64_t inst, uint32_t h, uint32_t i, uint64_t u[4], uint64_t v[4]) const;
 };
 
 struct PermChallenges {
@@ -64,7 +59,7 @@ __global__ void k_perm_prep(const uint64_t* __restrict__ idsig, uint64_t* __rest
   }
 }
 
-__device__ __forceinline__ void perm_value(const PermArgs& A, uint64_t inst, uint64_t s, uint64_t p[4]) {
+__device__ __forceinline__ void perm_value(const PermRows& A, uint64_t inst, uint64_t s, uint64_t p[4]) {
   const uint64_t off = s & PS_OFF_MASK;
   switch (s >> 60) {
     case PS_GATE: load_cell(A.gate + (inst * A.gate_inst + off) * 4, p); break;
@@ -76,148 +71,31 @@ __device__ __forceinline__ void perm_value(const PermArgs& A, uint64_t inst, uin
   }
 }
 
-// u, v of one row from its moved cells [k0, k1) (k0 < k1), zero rule applied
-__device__ void perm_row_terms(const PermArgs& A, uint64_t inst, uint32_t k0, uint32_t k1, uint64_t u[4], uint64_t v[4]) {
+// a moved cell in rows [i0, i1) of chunk h (ptr ends at index U + 1)
+__device__ __forceinline__ bool PermRows::any(uint32_t h, uint32_t i0, uint32_t i1) const {
+  const uint32_t* pr = ptr + (uint64_t)h * (usable_rows + 2);
+  return pr[min(i0, usable_rows + 1)] != pr[min(i1, usable_rows + 1)];
+}
+
+// u, v of a row from its moved cells [k0, k1); false for a row without any
+__device__ bool PermRows::terms(uint64_t inst, uint32_t h, uint32_t i, uint64_t u[4], uint64_t v[4]) const {
+  const uint32_t* pr = ptr + (uint64_t)h * (usable_rows + 2);
+  const uint32_t k0 = pr[i], k1 = pr[i + 1];
+  if (k0 == k1) return false;
   uint64_t p[4], t[4];
   for (uint32_t k = k0; k < k1; k++) {
-    perm_value(A, inst, A.src[k], p);
+    perm_value(*this, inst, src[k], p);
     if (k == k0) {
-      fr_add_dev(p, A.ab + (uint64_t)k * 8, u);
-      fr_add_dev(p, A.ab + (uint64_t)k * 8 + 4, v);
+      fr_add_dev(p, ab + (uint64_t)k * 8, u);
+      fr_add_dev(p, ab + (uint64_t)k * 8 + 4, v);
     } else {
-      fr_add_dev(p, A.ab + (uint64_t)k * 8, t);
+      fr_add_dev(p, ab + (uint64_t)k * 8, t);
       fr_mul_into(u, t);
-      fr_add_dev(p, A.ab + (uint64_t)k * 8 + 4, t);
+      fr_add_dev(p, ab + (uint64_t)k * 8 + 4, t);
       fr_mul_into(v, t);
     }
   }
-  if (fr_is_zero(v)) {   // batch_invert leaves the zero denominator as 0: fraction 0
-    u[0] = u[1] = u[2] = u[3] = 0;
-    fr_one(v);
-  }
-}
-
-__global__ void __launch_bounds__(PP_THREADS) k_perm_tiles(const PermArgs A) {
-  __shared__ uint64_t s_w[PP_THREADS / 32][2][4];
-  __shared__ uint32_t s_any[PP_THREADS / 32];
-  const uint64_t inst = blockIdx.y;
-  const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const uint32_t h = blockIdx.x / A.tiles_per_chunk, t0 = (blockIdx.x % A.tiles_per_chunk) * (uint32_t)PP_TILE;
-  const uint32_t* pr = A.ptr + (uint64_t)h * (A.usable_rows + 2);
-  uint64_t pu[4], pv[4], u[4], v[4];
-  fr_one(pu); fr_one(pv);
-  bool mine = false;
-#pragma unroll 1
-  for (uint32_t r = 0; r < PP_ROWS; r++) {
-    const uint32_t i = t0 + r * PP_THREADS + threadIdx.x;
-    if (i > A.usable_rows) break;
-    const uint32_t k0 = pr[i], k1 = pr[i + 1];
-    if (k0 == k1) continue;
-    perm_row_terms(A, inst, k0, k1, u, v);
-    if (mine) { fr_mul_into(pu, u); fr_mul_into(pv, v); }
-    else { fr_copy(u, pu); fr_copy(v, pv); mine = true; }
-  }
-  const uint32_t any = __ballot_sync(0xffffffffu, mine);
-  if (any) {
-#pragma unroll
-    for (uint32_t o = 16; o > 0; o >>= 1) {
-      fr_shfl_down(pu, o, u);
-      fr_shfl_down(pv, o, v);
-      fr_mul_into(pu, u);   // lanes >= 32 - o fold garbage, but only lane 0's result is used
-      fr_mul_into(pv, v);
-    }
-  }
-  if (lane == 0) { fr_copy(pu, s_w[warp][0]); fr_copy(pv, s_w[warp][1]); s_any[warp] = any; }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    for (int w = 1; w < PP_THREADS / 32; w++)
-      if (s_any[w]) { fr_mul_into(pu, s_w[w][0]); fr_mul_into(pv, s_w[w][1]); }
-    uint64_t* out = A.tiles + (inst * A.n_chunks * A.tiles_per_chunk + blockIdx.x) * 8;
-    fr_copy(pu, out); fr_copy(pv, out + 4);
-  }
-}
-
-__global__ void __launch_bounds__(PP_THREADS) k_perm_fill(const PermArgs A) {
-  __shared__ uint64_t s_w[PP_THREADS / 32][2][4];   // per warp: inclusive product of u, of v; then the warp's constant
-  const uint64_t inst = blockIdx.y;
-  const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const uint32_t h = blockIdx.x / A.tiles_per_chunk;
-  const uint32_t s = (blockIdx.x % A.tiles_per_chunk) * (uint32_t)PP_TILE + threadIdx.x * PP_ROWS;
-  const uint32_t* pr = A.ptr + (uint64_t)h * (A.usable_rows + 2);
-  const uint32_t last = A.usable_rows + 1;   // ptr index bound
-  const bool mine = pr[min(s, last)] != pr[min(s + PP_ROWS, last)];
-  const bool warp_any = __ballot_sync(0xffffffffu, mine) != 0;
-  uint64_t u[PP_ROWS][4], sv[PP_ROWS][4];   // u of each row; v, then the suffix products of v inside the segment
-  uint64_t pu[4], pv[4], x[4], y[4];
-  if (warp_any) {
-    if (mine) {
-#pragma unroll
-      for (int r = 0; r < PP_ROWS; r++) {
-        const uint32_t i = s + r;
-        if (i <= A.usable_rows && pr[i] != pr[i + 1]) perm_row_terms(A, inst, pr[i], pr[i + 1], u[r], sv[r]);
-        else { fr_one(u[r]); fr_one(sv[r]); }
-      }
-#pragma unroll
-      for (int r = PP_ROWS - 2; r >= 0; r--) fr_mul_into(sv[r], sv[r + 1]);
-      fr_copy(u[0], pu);
-#pragma unroll
-      for (int r = 1; r < PP_ROWS; r++) fr_mul_into(pu, u[r]);
-      fr_copy(sv[0], pv);
-    } else {
-      fr_one(pu); fr_one(pv);
-    }
-    // inclusive prefix of pu, inclusive suffix of pv over the warp
-#pragma unroll
-    for (uint32_t o = 1; o < 32; o <<= 1) {
-      fr_shfl_up(pu, o, x);
-      fr_shfl_down(pv, o, y);
-      if (lane >= o) fr_mul_into(pu, x);
-      if (lane + o < 32) fr_mul_into(pv, y);
-    }
-    if (lane == 31) fr_copy(pu, s_w[warp][0]);
-    if (lane == 0) fr_copy(pv, s_w[warp][1]);
-    fr_shfl_up(pu, 1, x);     // exclusive
-    fr_shfl_down(pv, 1, y);
-    if (lane == 0) fr_one(x);
-    if (lane == 31) fr_one(y);
-  } else if (lane == 0) {
-    fr_one(s_w[warp][0]); fr_one(s_w[warp][1]);
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    // K_w = C_t * (prod u of the warps before w) * (prod v of the warps after w)
-    uint64_t c[4], acc[4], k[PP_THREADS / 32][4];
-    load_cell(A.consts + (inst * A.n_chunks * A.tiles_per_chunk + blockIdx.x) * 4, c);
-    fr_copy(c, acc);
-    for (int w = 0; w < PP_THREADS / 32; w++) { fr_copy(acc, k[w]); fr_mul_into(acc, s_w[w][0]); }
-    fr_one(acc);
-    for (int w = PP_THREADS / 32 - 1; w >= 0; w--) { fr_mul_into(k[w], acc); fr_mul_into(acc, s_w[w][1]); }
-    for (int w = 0; w < PP_THREADS / 32; w++) fr_copy(k[w], s_w[w][0]);
-  }
-  __syncthreads();
-  uint64_t w[4];
-  if (warp_any) {
-    mont_mul_dev(s_w[warp][0], x, pu);
-    mont_mul_dev(pu, y, w);   // z[s] / sv[0]: the product of u before the segment over the product of v from its end on
-  } else {
-    fr_copy(s_w[warp][0], w);
-  }
-  uint64_t* zr = A.z + ((inst * A.n_chunks + h) * (A.usable_rows + 1ull) + s) * 4;
-  if (mine) {
-#pragma unroll
-    for (int r = 0; r < PP_ROWS; r++) {
-      if (s + r > A.usable_rows) break;
-      mont_mul_dev(w, sv[r], x);
-      store_fr(zr + r * 4, x);
-      if (r + 1 < PP_ROWS) fr_mul_into(w, u[r]);
-    }
-  } else {
-#pragma unroll
-    for (int r = 0; r < PP_ROWS; r++) {
-      if (s + r > A.usable_rows) break;
-      store_fr(zr + r * 4, w);
-    }
-  }
+  return true;
 }
 
 }  // namespace
@@ -363,18 +241,19 @@ int h2sha_permutation_product(h2sha_engine_t* e, uint64_t n_instances, const h2s
     if ((uintptr_t)b & 31u) return set_err(H2SHA_EINVAL, "Fr buffers must be 32-byte aligned");
   if (n_instances == 0) return H2SHA_OK;
   CUDA_TRY(cudaSetDevice(e->device));
-  int rc = ensure_lookup_consts(e);
+  int rc = ensure_perm_state(e, *desc, C);
   if (rc) return rc;
-  if ((rc = ensure_perm_state(e, *desc, C))) return rc;
   h2sha_perm_state* S = e->perm;
   cudaStream_t st = (cudaStream_t)stream;
-  PermArgs A{};
-  A.usable_rows = usable_rows; A.n_chunks = C.n_chunks;
-  A.tiles_per_chunk = (uint32_t)((usable_rows + 1ull + PP_TILE - 1) / PP_TILE);
-  const uint32_t n_tiles = A.n_chunks * A.tiles_per_chunk;
+  PermRows A{};
+  A.usable_rows = usable_rows;
   A.gate_inst = e->dplan.gate_inst_cells; A.lookup_inst = e->dplan.lookup_inst_cells; A.spread_inst = e->dplan.spread_inst_cells;
   A.digest_bytes = 32u * (uint32_t)P.digests.size();
   A.fixed = S->d_fixed; A.bytes = S->d_bytes; A.src = S->d_src; A.ab = S->d_ab; A.ptr = S->d_ptr;
+  GrandProduct Z{};
+  Z.rows = usable_rows + 1; Z.n_chunks = C.n_chunks; Z.z_stride = usable_rows + 1;
+  Z.tiles_per_chunk = (uint32_t)((usable_rows + 1ull + GP_TILE - 1) / GP_TILE);
+  const uint32_t n_tiles = Z.n_chunks * Z.tiles_per_chunk;
   // per call: a, b of every moved cell
   PermChallenges ch;
   memcpy(ch.beta, beta_mont, 32); memcpy(ch.gamma, gamma_mont, 32);
@@ -390,29 +269,17 @@ int h2sha_permutation_product(h2sha_engine_t* e, uint64_t n_instances, const h2s
     CUDA_TRY(cudaMalloc(&S->d_ws, need));
     S->ws_bytes = need;
   }
-  A.tiles = S->d_ws;
-  A.consts = S->d_ws + chunk * n_tiles * 8;
-  // the fold of lookup_product.cuh over the tiles of all chunks in chain order; z seen as [n][n_chunks * (U + 1)], so its
-  // "z[U]" is the last chunk's z[U]
-  ProductArgs F{};
-  F.tiles = A.tiles; F.consts = const_cast<uint64_t*>(A.consts); F.n_tiles = n_tiles;
-  F.usable_rows = (uint32_t)((uint64_t)A.n_chunks * (usable_rows + 1ull) - 1);
-  F.errors = errors_dev;
-  const uint64_t z_inst = (uint64_t)A.n_chunks * (usable_rows + 1ull) * 4;
+  Z.tiles = S->d_ws;
+  Z.consts = S->d_ws + chunk * n_tiles * 8;
+  Z.errors = errors_dev;
   for (uint64_t i0 = 0; i0 < n_instances; i0 += chunk) {
     const unsigned ni = (unsigned)std::min<uint64_t>(chunk, n_instances - i0);
     A.gate = gate ? (const uint64_t*)gate + i0 * A.gate_inst * 4 : nullptr;
     A.lookup = lookup ? (const uint64_t*)lookup + i0 * A.lookup_inst * 4 : nullptr;
     A.spread = spread ? (const uint64_t*)spread + i0 * A.spread_inst * 4 : nullptr;
     A.digests = digests_dev ? digests_dev + i0 * A.digest_bytes : nullptr;
-    A.z = (uint64_t*)z_dev + i0 * z_inst;
-    F.z = A.z;
-    k_perm_tiles<<<dim3(n_tiles, ni), PP_THREADS, 0, st>>>(A);
-    CUDA_TRY(cudaGetLastError());
-    k_product_fold<<<(ni + LP_FOLD_WARPS - 1) / LP_FOLD_WARPS, 32 * LP_FOLD_WARPS, 0, st>>>(F, ni);
-    CUDA_TRY(cudaGetLastError());
-    k_perm_fill<<<dim3(n_tiles, ni), PP_THREADS, 0, st>>>(A);
-    CUDA_TRY(cudaGetLastError());
+    Z.z = (uint64_t*)z_dev + i0 * Z.n_chunks * (usable_rows + 1ull) * 4;
+    if ((rc = launch_product(Z, A, ni, st))) return rc;
   }
   return H2SHA_OK;
 }

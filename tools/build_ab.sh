@@ -1,7 +1,7 @@
 #!/bin/bash
 # Builds the engine of another revision next to the in-tree one, for A/B timing on one GPU box:
 #     tools/build_ab.sh <git-rev> [name] [extra nvcc flags, e.g. -DH2SHA_TILE_MODE]   ->  tools/ab/libh2sha_<name>.so   (default name: base)
-# <git-rev> may be WORK for the working tree as it is.
+# <git-rev> may be WORK for the working tree as it is.  engine.cu is linked with every *.cc source that revision has.
 # then e.g.  TUNE_SUSTAIN=1 TUNE_LIB=tools/ab/libh2sha_base.so python tools/tune.py cfg2 parts=3   (tools/ab.sh interleaves A and B).
 # tools/ab/ is scratch: delete it before committing a round (the .so files are git-ignored but would ship to the GPU box).
 set -euo pipefail
@@ -17,6 +17,6 @@ else
   done
 fi
 /usr/local/cuda/bin/nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -shared -Xcompiler -fPIC -cudart shared -ldl $extra \
-  -o "$root/tools/ab/libh2sha_$name.so" "$tmp/halo2-dynamic-sha256_b200/csrc/engine.cu" "$tmp/halo2-dynamic-sha256_b200/csrc/planner.cc"
+  -o "$root/tools/ab/libh2sha_$name.so" "$tmp/halo2-dynamic-sha256_b200/csrc/engine.cu" "$tmp"/halo2-dynamic-sha256_b200/csrc/*.cc
 rm -rf "$tmp"
 echo "$root/tools/ab/libh2sha_$name.so"

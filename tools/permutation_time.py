@@ -20,8 +20,11 @@ import __graft_entry__ as ge  # noqa: E402
 
 n_cfg2 = int(sys.argv[1]) if len(sys.argv) > 1 else 256
 n_tc = int(sys.argv[2]) if len(sys.argv) > 2 else 64
-ge.build()
 pkg = ge.load_package()
+if os.environ.get("TUNE_LIB"):   # A/B: time another build of the engine (tools/build_ab.sh) with the same harness
+    pkg.LIB_PATH = os.path.abspath(os.environ["TUNE_LIB"])
+else:
+    ge.build()
 dev = torch.device("cuda", 0)
 st = torch.cuda.current_stream(dev)
 usable, m = (1 << 17) - 6, 2

@@ -51,10 +51,10 @@ def timed(fn, reps=5):
 t_m = timed(lambda: L.h2sha_lookup_multiplicities(cfg._h, n, res.lookup.data_ptr(), res.spread.data_ptr(), usable, mult.data_ptr(), bad.data_ptr(), st.cuda_stream))
 print(f"multiplicities: {n} instances {t_m:.3f} ms, reads {n * (lay.n_lookup_cells + 2 * lay.n_spread_limbs) * 32 / t_m / 1e6:.0f} GB/s, bad={int(bad.item())}")
 
-# Thread-level instructions per row of k_product_tiles + k_product_fill, counted once from `cuobjdump -sass` of the sm_100a build:
-# a Montgomery product (mont_mul_dev) with its loads and additions is ~516 SASS instructions (k_product_fill: 35 104 for its 8 rows a
-# thread, 68 products); a row costs 4 + 10/8 products in k_product_tiles and 7 + 1/8 in k_product_fill, one more in each pass for the
-# theta compression of a spread lookup.
+# Thread-level instructions per row of k_product_tiles<LookupRows> + k_product_fill<LookupRows>, counted once from `cuobjdump -sass` of
+# the sm_100a build: a Montgomery product (mont_mul_dev) with its loads and additions is ~516 SASS instructions (k_product_fill: 35 296
+# for its 8 rows a thread, 68 products); a row costs 4 + 10/8 products in k_product_tiles and 7 + 1/8 in k_product_fill, one more in
+# each pass for the theta compression of a spread lookup.
 INST_PER_ROW = {"range": 6400, "spread": 7400}
 
 smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader", "-i", "0"], capture_output=True, text=True).stdout.strip()
