@@ -14,8 +14,7 @@
 //   lookup_prework.cuh  k_range_mult / k_spread_mult / k_permute_scan / k_permute_fill: lookup-argument pre-work
 //   batch_check.cuh     k_check_gates / k_check_pairs / k_check_digest_bytes: MockProver-style pass over a whole batch; h2sha_gather
 // Build-time switches (never set for the product): H2SHA_DEBUG_TIMING (1 | 2: %globaltimer prints of the producer / consumer
-// hand-over); H2SHA_TILE_MODE (also instantiates k_expand<.., TILE = true>, the value-major phase 2 of the round-2 experiment:
-// bit-exact but slower, selected at run time with H2SHA_TUNE tile=N; DESIGN.md section 10).  The wrong-cell experiment builds of round 1 (profiles/r1_power_probe.txt) are gone from this file.
+// hand-over).
 // There is no CPU path: every entry point fails with H2SHA_ECUDA when no device is usable.
 #include <cuda_runtime.h>
 #include <dlfcn.h>
@@ -63,13 +62,11 @@ struct DevPlan {
   uint32_t blob_bytes;
   // byte offsets inside the blob (all 16-byte aligned)
   uint32_t off_fill, off_cells, off_chunks, off_items, off_table_lo, off_table_hi, off_resident, off_prog, off_groups, off_tasks, off_types, off_classes,
-      off_raw, off_breaks, off_digests, off_item_dict, off_vdst;
-  uint32_t tile_cells;   // > 0: value-major phase 2 (k_expand<.., TILE = true>): per consumer warp a tile of this many cells instead of the scratch table
+      off_raw, off_breaks, off_digests, off_item_dict;
   uint32_t n_breaks, n_digests, n_block_parts, n_classes;
   // dynamic shared memory layout after the blob
   uint32_t off_trace, off_scratch, off_misc, smem_bytes;
   uint32_t stage_bytes, stage_off_slots, stage_off_desc;   // per producer warp: trace | slots | StageDesc
-  uint32_t cons_sleep, prod_sleep, wait_hint;                         // back-off (ns) between polls of the full / empty barrier; cons_sleep 0 = tight spin
   uint32_t max_fill, scratch_bytes, n_resident;            // per consumer warp: lo[max_fill] | hi[max_fill]
   // layout
   int32_t spread_cols_shift;   // log2(spread_cols) when it is a power of two, else -1
@@ -403,26 +400,10 @@ __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
-// wait with a suspend-time hint: the hardware parks the warp until the phase completes or `hint_ns` have passed, so a
-// waiting warp issues one instruction per `hint_ns` instead of polling (mode 1), or -- mode 0 -- polls with __nanosleep
-// back-off between tries (the round-1 behaviour)
-__device__ __forceinline__ void mbar_wait_relaxed(uint64_t* bar, uint32_t parity, uint32_t ns, uint32_t use_hint) {
+// the producers' wait: polls with a 256 ns __nanosleep back-off between tries (longer sleeps, suspend-time hints and a
+// back-off for the consumers' wait measured no better in time or power: DESIGN.md section 10)
+__device__ __forceinline__ void mbar_wait_relaxed(uint64_t* bar, uint32_t parity) {
   uint32_t done = 0;
-  if (use_hint) {
-    for (;;) {
-      asm volatile(
-          "{\n"
-          ".reg .pred P1;\n"
-          "mbarrier.try_wait.parity.shared::cta.b64 P1, [%1], %2, %3;\n"
-          "selp.u32 %0, 1, 0, P1;\n"
-          "}"
-          : "=r"(done)
-          : "r"(smem_u32(bar)), "r"(parity), "r"(ns)
-          : "memory");
-      if (done) break;
-    }
-    return;
-  }
   for (;;) {
     asm volatile(
         "{\n"
@@ -434,7 +415,7 @@ __device__ __forceinline__ void mbar_wait_relaxed(uint64_t* bar, uint32_t parity
         : "r"(smem_u32(bar)), "r"(parity)
         : "memory");
     if (done) break;
-    __nanosleep(ns);
+    __nanosleep(256);
   }
 }
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
@@ -579,31 +560,10 @@ __device__ __forceinline__ void flush_checksums(unsigned long long* cks, uint64_
   }
 }
 
-// ---- tile mode (value-major phase 2) ----
-// One Fr cell into the warp's tile (which has the layout of the output column).  `x` = byte offset of the cell in the tile
-// (destination * 32, as the planner stores it), `tile_par` = tile + 16 * (lane & 1): odd lanes write the high half first.  A 128-bit
-// shared store is served a quarter-warp at a time over eight 16-byte bank groups and the low halves of 32-byte cells only ever
-// touch the even ones, so alternating halves by lane parity is what lets eight lanes with suitable destinations (the planner
-// arranges: distinct destination mod 4 among the lanes of one parity) go out in one wavefront.
-__device__ __forceinline__ void tile_store(uint8_t* tile_par, uint32_t x, const uint4& first, const uint4& second) {
-  const uint32_t a = smem_u32(tile_par) + x;
-  asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(a), "r"(first.x), "r"(first.y), "r"(first.z), "r"(first.w) : "memory");
-  asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(a ^ 16u), "r"(second.x), "r"(second.y), "r"(second.z), "r"(second.w) : "memory");
-}
-// tile -> global: one bulk copy (UBLKCP) issued by one lane; the global store never touches the LSU pipe
-__device__ __forceinline__ void bulk_store(uint32_t* gdst, uint32_t tile_smem_addr, uint32_t bytes) {
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(tile_smem_addr), "r"(bytes) : "memory");
-}
-
 // MODE 0: cells (+ checksums); 1: also write the raw values of the looked-up cells (A.lookup_raw / A.dense_raw: the input of the
 // multiplicity kernel); 2: also write the dictionary of distinct values
 // (A.dict).  Separate instantiations: the extra code costs registers the plain path (80 per thread at 768 threads) does not have.
-// TILE: value-major phase 2 (DevPlan::tile_cells > 0).  A chunk's distinct values never leave the registers of the lane that made
-// them: the lane scatters its value into the warp's shared-memory tile at every gate cell that carries it (destination tables made
-// by the planner), stores it straight to its lookup / spread-column cells, and the finished tile -- a contiguous run of one output
-// column -- leaves with one bulk copy.  Against the scratch path this drops the per-value scratch store, the per-cell scratch read
-// and every global store instruction of the gate stream from the LSU pipe.
-template <int NCONS, int NPROD, int MODE, bool TILE>
+template <int NCONS, int NPROD, int MODE>
 __global__ void __launch_bounds__((NCONS + NPROD) * 32, 1) k_expand(const DevPlan P, const JobArgs A) {
   constexpr bool MULT = MODE == 1, DICT = MODE == 2;
   extern __shared__ __align__(128) uint8_t smem[];
@@ -631,7 +591,6 @@ __global__ void __launch_bounds__((NCONS + NPROD) * 32, 1) k_expand(const DevPla
   const uint32_t* s_breaks = reinterpret_cast<const uint32_t*>(smem + P.off_breaks);
   const DevDigest* s_digests = reinterpret_cast<const DevDigest*>(smem + P.off_digests);
   [[maybe_unused]] const uint32_t* s_item_dict = reinterpret_cast<const uint32_t*>(smem + P.off_item_dict);
-  [[maybe_unused]] const uint16_t* s_vdst = reinterpret_cast<const uint16_t*>(smem + P.off_vdst);
   uint64_t* s_full = reinterpret_cast<uint64_t*>(smem + P.off_misc);   // [NPROD]
   uint64_t* s_empty = s_full + NPROD;                                  // [NPROD]
   if (tid == 0) {
@@ -665,7 +624,7 @@ __global__ void __launch_bounds__((NCONS + NPROD) * 32, 1) k_expand(const DevPla
     StageDesc* desc = reinterpret_cast<StageDesc*>(stage + P.stage_off_desc);
     for (int i = lane; i < 64; i += 32) s_trace[TR_K + i] = c_K[i];
     for (uint32_t k = 0;; k++) {
-      mbar_wait_relaxed(&s_empty[st], (k & 1u) ^ 1u, P.prod_sleep, P.wait_hint);   // consumers are done with this stage's previous job
+      mbar_wait_relaxed(&s_empty[st], (k & 1u) ^ 1u);   // consumers are done with this stage's previous job
 #ifdef H2SHA_DEBUG_TIMING
       unsigned long long dbg_p0; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(dbg_p0));
 #endif
@@ -771,8 +730,7 @@ __global__ void __launch_bounds__((NCONS + NPROD) * 32, 1) k_expand(const DevPla
 
   // =========================== consumer warp ===========================
   WarpScratch ws;
-  [[maybe_unused]] uint8_t* const tile = smem + P.off_scratch + (size_t)warp * P.scratch_bytes;   // TILE: scratch_bytes = tile_cells * 32
-  if constexpr (!TILE) {
+  {
     uint8_t* base = smem + P.off_scratch + (size_t)warp * P.scratch_bytes;
     ws.lo = reinterpret_cast<uint4*>(base);
     ws.hi = ws.lo + P.max_fill;
@@ -791,7 +749,7 @@ __global__ void __launch_bounds__((NCONS + NPROD) * 32, 1) k_expand(const DevPla
 #ifdef H2SHA_DEBUG_TIMING
     unsigned long long dbg_w0; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(dbg_w0));
 #endif
-    if (P.cons_sleep) mbar_wait_relaxed(&s_full[st], round & 1u, P.cons_sleep, P.wait_hint); else mbar_wait(&s_full[st], round & 1u);
+    mbar_wait(&s_full[st], round & 1u);
 #ifdef H2SHA_DEBUG_TIMING
     {
       unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
@@ -838,131 +796,6 @@ __global__ void __launch_bounds__((NCONS + NPROD) * 32, 1) k_expand(const DevPla
       // ---- compact hand-off: the chunk's distinct values also go to the instance's dictionary, fill entry i -> entry dict_chunk + i ----
       [[maybe_unused]] uint32_t* dict_chunk = nullptr;
       if constexpr (DICT) dict_chunk = A.dict + (inst * A.dict_inst_cells + desc->dict0 + s_item_dict[jc.item_off + it]) * 8;
-      if constexpr (TILE) {
-        const bool want_gate = gate_out != nullptr && ch.gate_len != 0;
-        const bool per_cell_ck = straddle && A.cks;          // then w0 = w1 = 0 and every gate cell adds its own weight
-        const uint32_t gbase = g_lo + ch.gate_dst_min;        // instance-relative gate-stream index of tile cell 0
-        const uint32_t l_lo = lk0 + item.lk_rel, m_lo = limb0 + item.limb_rel;
-        uint32_t loff0 = 0, loff1 = 0, wrap = 0xffffffffu;    // lookup column wrap at max_rows (range.finalize), as in the scratch path
-        if (P.n_lookup_cols > 1) {
-          const uint32_t col0 = l_lo / P.max_rows;
-          wrap = (col0 + 1) * P.max_rows;
-          loff0 = col0 * (P.lookup_col_rows - P.max_rows);
-          loff1 = (col0 + 1) * (P.lookup_col_rows - P.max_rows);
-        }
-        // the bulk copy of this warp's previous chunk must have finished READING the tile before it is overwritten
-        if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-        __syncwarp();
-        // ---- resident constants: cell-major, straight from the static table (entry = table index | byte offset in the tile) ----
-        const bool odd = lane & 1;
-        uint8_t* const tile_par = tile + (odd ? 16 : 0);
-        if (want_gate || per_cell_ck) {
-          const CellEntry* rc = s_cells + ch.lk_off;
-          for (uint32_t i = lane; i < ch.n_fill32; i += 32) {
-            const uint32_t v = rc[i].v, x = v >> 16;
-            const uint4 lo = s_table_lo[v & 0xffffu], hi = s_table_hi[v & 0xffffu];
-            if (want_gate) tile_store(tile_par, x, odd ? hi : lo, odd ? lo : hi);
-            if (per_cell_ck) {
-              const uint32_t gidx = gbase + (x >> 5), pos = gidx + ((gidx >= next_brk) ? off1 : off0);
-              ck_g += (unsigned long long)hash8(lo, hi) * (unsigned long long)(2u * pos + 1u);
-            }
-          }
-        }
-        // ---- the chunk's distinct values, 32 at a time: lane = value; scatter rounds = the largest use count in the batch ----
-        uint32_t voff = ch.gate_off;
-        auto emit = [&](const FillEntry& e, bool active, const uint4& lo, const uint4& hi, uint32_t h, uint32_t raw32) {
-          const uint32_t gc = active ? H2SHA_FE_GATE_CNT(e) : 0u, lc = active ? H2SHA_FE_LK_CNT(e) : 0u, mc = active ? H2SHA_FE_LIMB_CNT(e) : 0u;
-          const uint32_t Rg = __reduce_max_sync(0xffffffffu, gc), Rl = __reduce_max_sync(0xffffffffu, lc), Rm = __reduce_max_sync(0xffffffffu, mc);
-          const uint16_t* dp = s_vdst + voff + lane;
-          if (want_gate && !per_cell_ck) {
-            const uint4 first = odd ? hi : lo, second = odd ? lo : hi;
-            for (uint32_t r = 0; r < Rg; r++)
-              if (r < gc) tile_store(tile_par, dp[r * 32], first, second);
-          } else if (per_cell_ck) {   // a column break inside the chunk (rare): every gate cell adds its own checksum weight
-            for (uint32_t r = 0; r < Rg; r++) {
-              if (r < gc) {
-                const uint32_t x = dp[r * 32];
-                if (want_gate) tile_store(tile_par, x, odd ? hi : lo, odd ? lo : hi);
-                const uint32_t gidx = gbase + (x >> 5), pos = gidx + ((gidx >= next_brk) ? off1 : off0);
-                ck_g += (unsigned long long)h * (unsigned long long)(2u * pos + 1u);
-              }
-            }
-          }
-          dp += Rg * 32;
-          // lookup-column cells (range.finalize copies cells_to_lookup in push order, wrapping at max_rows)
-          for (uint32_t r = 0; r < Rl; r++) {
-            if (r < lc) {
-              const uint32_t li = l_lo + dp[r * 32];
-              const uint32_t pos = li + ((li >= wrap) ? loff1 : loff0);
-              if (lk_out) store_cell2(lk_out + (uint64_t)pos * 8, lo, hi);
-              if constexpr (MULT) A.lookup_raw[inst * A.n_lookup_total + li] = raw32;
-              ck_l += (unsigned long long)h * (unsigned long long)(2u * pos + 1u);
-            }
-          }
-          dp += Rl * 32;
-          // spread-table columns: limb n -> column n % cols, row n / cols (spread.rs:202,228-231); dense then spread
-          for (uint32_t r = 0; r < Rm; r++) {
-            if (r < mc) {
-              const uint32_t x = dp[r * 32], n = m_lo + (x >> 1), which = x & 1u;
-              uint32_t row, col;
-              if (P.spread_cols_shift >= 0) { row = n >> P.spread_cols_shift; col = n & (P.spread_cols - 1u); }
-              else { row = n / P.spread_cols; col = n - row * P.spread_cols; }
-              if (MULT && which == 0) A.dense_raw[inst * A.n_limb_total + n] = (uint8_t)raw32;
-              const uint32_t pos = (which * P.spread_cols + col) * P.spread_rows + row;
-              if (sp_out) store_cell2(sp_out + (uint64_t)pos * 8, lo, hi);
-              ck_s += (unsigned long long)h * (unsigned long long)(2u * pos + 1u);
-            }
-          }
-          voff += (Rg + Rl + Rm) * 32;
-        };
-        const FillEntry* fl = s_fill + ch.fill_off;
-        const uint32_t n_tab = ch.n_fill_table, n_all = ch.n_fill;
-        for (uint32_t i0 = 0; i0 < n_tab; i0 += 32) {
-          const uint32_t i = i0 + lane;
-          const bool active = i < n_tab;
-          const FillEntry e = fl[active ? i : 0u];
-          uint32_t raw;
-          uint4 lo, hi;
-          value_table(e, slots, s_table_lo, s_table_hi, &raw, &lo, &hi);
-          const uint32_t h = hash8(lo, hi);
-          if (active) {
-            ck_g += (unsigned long long)h * (H2SHA_FE_GATE_CNT(e) * w0 + e.sumdst * w1);
-            if constexpr (DICT) store_cell2(dict_chunk + (uint64_t)i * 8, lo, hi);
-          }
-          emit(e, active, lo, hi, h, raw);
-        }
-        for (uint32_t i0 = n_tab; i0 < n_all; i0 += 32) {
-          const uint32_t i = i0 + lane;
-          const bool active = i < n_all;
-          const FillEntry e = fl[active ? i : n_tab];
-          uint64_t raw;
-          uint4 lo, hi;
-          value_generic(e, slots, active, &raw, &lo, &hi);
-          const uint32_t h = hash8(lo, hi);
-          if (active) {
-            ck_g += (unsigned long long)h * (H2SHA_FE_GATE_CNT(e) * w0 + e.sumdst * w1);
-            if constexpr (DICT) store_cell2(dict_chunk + (uint64_t)i * 8, lo, hi);
-          }
-          emit(e, active, lo, hi, h, (raw >> 32) ? 0xffffffffu : (uint32_t)raw);
-        }
-        if (lane == 0 && !straddle) ck_g += ch.res_a + ch.res_b * w0;
-        // ---- the finished tile is a contiguous run of the output column (two runs when a column break falls inside) ----
-        if (want_gate) {
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy tile writes -> visible to the bulk-copy engine
-          __syncwarp();
-          if (lane == 0) {
-            const uint32_t ta = smem_u32(tile);
-            if (!straddle) {
-              bulk_store(gate_out + (uint64_t)(gbase + off0) * 8, ta, (uint32_t)ch.gate_len * 32u);
-            } else {
-              const uint32_t n1 = next_brk - gbase;
-              bulk_store(gate_out + (uint64_t)(gbase + off0) * 8, ta, n1 * 32u);
-              bulk_store(gate_out + (uint64_t)(next_brk + off1) * 8, ta + n1 * 32u, ((uint32_t)ch.gate_len - n1) * 32u);
-            }
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-          }
-        }
-      } else {
       // ---- fill: table copies, then Barrett conversions ----
       {
         const FillEntry* fl = s_fill + ch.fill_off;
@@ -1066,7 +899,6 @@ __global__ void __launch_bounds__((NCONS + NPROD) * 32, 1) k_expand(const DevPla
           ck_s += (unsigned long long)hash8(lo, hi) * (unsigned long long)(2u * pos + 1u);
         }
       }
-      }   // !TILE
       if (A.cks && jc.batch > 1) {   // batched digest jobs: the items of a warp belong to different instances
         flush_checksums(A.cks, inst, ck_g, ck_l, ck_s, lane);
         ck_g = 0; ck_l = 0; ck_s = 0;
@@ -1077,9 +909,6 @@ __global__ void __launch_bounds__((NCONS + NPROD) * 32, 1) k_expand(const DevPla
     if (lane == 0) mbar_arrive(&s_empty[st]);   // this warp no longer reads the stage
     // ---- checksums: warp reduce, one global atomic per kind and warp (block jobs: one instance per job) ----
     if (A.cks && jc.batch == 1) flush_checksums(A.cks, inst0, ck_g, ck_l, ck_s, lane);
-  }
-  if constexpr (TILE) {   // the tile must outlive the bulk copies that read it
-    if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
   }
 #ifdef H2SHA_DEBUG_TIMING
   if (lane == 0 && (H2SHA_DEBUG_TIMING == 2 ? (warp == 0 || warp == NCONS - 1) : ((blockIdx.x % 37) == 0 && (warp % 7) == 0))) {
@@ -1221,16 +1050,10 @@ __global__ void k_zero_ranges(uint4* buf, uint64_t inst_cells, uint64_t n_inst, 
 struct ExpandVariant {
   int ncons, nprod;
   const void* fn[3];        // by MODE: plain | + lookup multiplicities | + dictionary of distinct values
-  const void* fn_tile[3];   // the same for the value-major phase 2 (tile mode)
 };
 template <int NC, int NP>
 ExpandVariant make_variant() {
-  return ExpandVariant{NC, NP, {(const void*)k_expand<NC, NP, 0, false>, (const void*)k_expand<NC, NP, 1, false>, (const void*)k_expand<NC, NP, 2, false>},
-#ifdef H2SHA_TILE_MODE   // experiment build (tools/build_ab.sh -DH2SHA_TILE_MODE): the value-major phase 2 measured slower, see DESIGN.md section 10
-                       {(const void*)k_expand<NC, NP, 0, true>, (const void*)k_expand<NC, NP, 1, true>, (const void*)k_expand<NC, NP, 2, true>}};
-#else
-                       {nullptr, nullptr, nullptr}};
-#endif
+  return ExpandVariant{NC, NP, {(const void*)k_expand<NC, NP, 0>, (const void*)k_expand<NC, NP, 1>, (const void*)k_expand<NC, NP, 2>}};
 }
 const ExpandVariant* expand_variants(int* n) {
   // the tuned default and the fallback chain for plans that need more shared memory (fewer consumer warps = less scratch)
@@ -1430,7 +1253,6 @@ int h2sha_create(const h2sha_config_t* cfg, h2sha_engine_t** out) {
   pc.max_fill = (uint32_t)tune_value("fill", (int)pc.max_fill);
   pc.resident_consts = (uint32_t)tune_value("res", (int)pc.resident_consts);
   pc.digest_batch = (uint32_t)tune_value("dbatch", (int)pc.digest_batch);
-  pc.tile_cells = (uint32_t)tune_value("tile", (int)pc.tile_cells);
   h2sha_engine* e = new h2sha_engine();
   e->device = cfg->device;
   EngineGuard guard{e};   // every early return below destroys the half-built engine (h2sha_destroy frees what exists)
@@ -1509,16 +1331,11 @@ int h2sha_create(const h2sha_config_t* cfg, h2sha_engine_t** out) {
   D.off_breaks = put(P.breaks.data(), P.breaks.size() * 4);
   D.off_digests = put(dds.data(), dds.size() * sizeof(DevDigest));
   D.off_item_dict = put(P.item_dict.data(), P.item_dict.size() * 4);
-  D.off_vdst = put(P.vdst.data(), P.vdst.size() * 2);
-  D.tile_cells = pc.tile_cells;
   D.blob_bytes = (uint32_t)blob.size();
   D.n_breaks = (uint32_t)P.breaks.size();
   D.n_digests = (uint32_t)P.digests.size();
   D.n_block_parts = P.n_block_parts;
   D.n_classes = (uint32_t)P.classes.size();
-  D.cons_sleep = (uint32_t)tune_value("csleep", 0);
-  D.prod_sleep = (uint32_t)tune_value("psleep", 256);
-  D.wait_hint = (uint32_t)tune_value("hint", 0);
   D.off_trace = D.blob_bytes;
   D.stage_off_slots = align_up(4 * std::max<uint32_t>(P.max_trace_words, TR_BLOCK_WORDS_WITH_K), 16);
   D.stage_off_desc = align_up(D.stage_off_slots + 8 * (P.max_slots + 1), 16);
@@ -1536,8 +1353,8 @@ int h2sha_create(const h2sha_config_t* cfg, h2sha_engine_t** out) {
         if (vs[i].ncons != pref[pi][0] || vs[i].nprod != pref[pi][1]) continue;
         e->variant = vs[i];
         D.max_fill = pc.max_fill;
-        D.scratch_bytes = pc.tile_cells ? pc.tile_cells * 32 : pc.max_fill * 32;   // per consumer warp: the tile, or the scratch table
-        D.off_scratch = align_up(D.off_trace + e->variant.nprod * D.stage_bytes, 128);   // tiles: tile_store relies on 32-byte alignment
+        D.scratch_bytes = pc.max_fill * 32;   // per consumer warp: the scratch table
+        D.off_scratch = align_up(D.off_trace + e->variant.nprod * D.stage_bytes, 128);
         D.off_misc = align_up(D.off_scratch + e->variant.ncons * D.scratch_bytes, 16);
         D.smem_bytes = D.off_misc + 2 * e->variant.nprod * 8;
         ok = D.smem_bytes <= 227 * 1024;
@@ -1546,7 +1363,7 @@ int h2sha_create(const h2sha_config_t* cfg, h2sha_engine_t** out) {
     if (!ok) return set_err(H2SHA_EINVAL, "configuration needs more than 227 KB of shared memory (or H2SHA_TUNE names no launch variant)");
   }
   D.max_rows = pc.max_rows; D.spread_cols = pc.spread_cols;
-  const uint32_t mult_scratch = pc.tile_cells ? D.scratch_bytes : pc.max_fill * 36, mult_misc = align_up(D.off_scratch + e->variant.ncons * mult_scratch, 16);
+  const uint32_t mult_scratch = pc.max_fill * 36, mult_misc = align_up(D.off_scratch + e->variant.ncons * mult_scratch, 16);
   e->mult_fits = mult_misc + 2 * e->variant.nprod * 8 <= 227 * 1024;
   D.spread_cols_shift = -1;
   for (int sh = 0; sh < 16; sh++) if ((1u << sh) == pc.spread_cols) D.spread_cols_shift = sh;
@@ -1573,10 +1390,6 @@ int h2sha_create(const h2sha_config_t* cfg, h2sha_engine_t** out) {
   const int expand_threads = (e->variant.ncons + e->variant.nprod) * 32;
   // the attribute belongs to the kernel function, not to this engine: always raise it to the 227 KB cap, so that engines of
   // different configurations that share a launch variant never lower each other's limit
-  if (pc.tile_cells) {
-    if (!e->variant.fn_tile[0]) return set_err(H2SHA_EINVAL, "H2SHA_TUNE tile=N needs a library built with -DH2SHA_TILE_MODE (experiment build)");
-    memcpy(e->variant.fn, e->variant.fn_tile, sizeof e->variant.fn);   // this engine's copy of the variant: tile-mode kernels
-  }
   for (const void* fn : e->variant.fn) CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
   int occ = 0;
   for (const void* fn : e->variant.fn) {
@@ -1586,9 +1399,8 @@ int h2sha_create(const h2sha_config_t* cfg, h2sha_engine_t** out) {
   }
   if (occ < 1) return set_err(H2SHA_ECUDA, "expand kernel does not fit on an SM");
   if (getenv("H2SHA_VERBOSE"))
-    fprintf(stderr, "[h2sha] k_expand<%d,%d>%s: blob %u B, stage %u B x %d, %s %u B x %d, shared memory %u B, %d CTAs\n", e->variant.ncons, e->variant.nprod,
-            pc.tile_cells ? " tile mode" : "", D.blob_bytes, D.stage_bytes, e->variant.nprod, pc.tile_cells ? "tile" : "scratch", D.scratch_bytes, e->variant.ncons,
-            D.smem_bytes, occ * e->n_sms);
+    fprintf(stderr, "[h2sha] k_expand<%d,%d>: blob %u B, stage %u B x %d, scratch %u B x %d, shared memory %u B, %d CTAs\n", e->variant.ncons, e->variant.nprod,
+            D.blob_bytes, D.stage_bytes, e->variant.nprod, D.scratch_bytes, e->variant.ncons, D.smem_bytes, occ * e->n_sms);
   e->expand_ctas = occ * e->n_sms;
   e->dplan_mult = e->dplan;
   if (e->mult_fits) { e->dplan_mult.scratch_bytes = mult_scratch; e->dplan_mult.off_misc = mult_misc; e->dplan_mult.smem_bytes = mult_misc + 2 * e->variant.nprod * 8; }

@@ -97,22 +97,10 @@ struct alignas(16) FillEntry {
 };
 #define H2SHA_FE_GATE_CNT(e) ((e).cnt & 0xffffu)
 #define H2SHA_FE_LK_CNT(e) ((e).cnt >> 16)
-// Tile mode (Config::tile_cells > 0, the value-major phase 2): there is no scratch table, so the `dst` field of the entry holds
-// the number of spread-column cells that carry the value instead (H2SHA_FE_LIMB_CNT), and the value's destinations follow in the
-// chunk's destination table (Plan::vdst).
-#define H2SHA_FE_LIMB_CNT(e) ((e).lo & 0xffffu)
 
 // multipliers of the cell checksum hash (include/h2sha_b200.h: H2SHA_CK_M)
 static const uint32_t kCkM[8] = {0x9E3779B1u, 0x85EBCA77u, 0xC2B2AE3Du, 0x27D4EB2Fu, 0x165667B1u, 0xD3A2646Du, 0xFD7046C5u, 0xB55A4F09u};
 
-// Tile mode reuses the same 48-byte descriptor with these meanings (the scratch path's in parentheses):
-//   gate_off  = index of the chunk's destination table in Plan::vdst (u16 entries; per batch of 32 fill entries: Rg rounds of 32
-//               gate destinations as byte offsets into the tile (32 x tile-relative cell index), Rl rounds of unit-relative lookup
-//               indices, Rm rounds of (limb << 1 | dense/spread), lane-minor, R* = the largest count in the batch; unused places
-//               hold 0xffff)
-//   lk_off    = CellEntry index of the chunk's resident-constant cells: static-table index (16) | byte offset into the tile (16)
-//   n_fill32  = number of those cells
-//   limb_off  = unused
 struct alignas(16) Chunk {
   uint64_t res_a, res_b;   // gate-checksum contribution of the resident constants of the chunk: res_a + res_b * (2*pos0 + 1)
   uint32_t fill_off;   // FillEntry index

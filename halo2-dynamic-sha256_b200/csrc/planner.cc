@@ -104,7 +104,6 @@ class Builder {
     if (cfg_.lookup_bits < 8 || cfg_.lookup_bits > 32) fail("lookup_bits must be in [8, 32]");
     if (cfg_.max_rows < 64) fail("max_rows too small");
     if (cfg_.max_fill < 64 || cfg_.max_fill > H2SHA_MAX_FILL_LIMIT || cfg_.max_fill % 8) fail("max_fill must be a multiple of 8 in [64, 256]");
-    if (cfg_.tile_cells && (cfg_.tile_cells < 32 || cfg_.tile_cells > 2048 || cfg_.tile_cells % 32)) fail("tile_cells must be a multiple of 32 in [32, 2048]");
     uint32_t max_r = 0;
     for (uint32_t m : cfg_.max_variable_byte_sizes) {
       if (m == 0 || m % 64 != 0) fail("max_variable_byte_size must be a positive multiple of 64 (lib.rs:57-59)");
@@ -954,156 +953,15 @@ class Builder {
     }
   }
 
-  // Tile mode: emits one chunk for the value-major phase 2.  `for_each(visit)` calls visit(kind, value index, dst, sym) for every cell
-  // of the chunk in emission order; `order` holds the chunk's distinct values.  Fill entries: table copies first, then the Barrett
-  // entries (<= 32 bit, then 64 bit / signed), each group sorted by the number of gate cells that carry the value (descending), so
-  // that the 32 lanes of a batch run about the same number of scatter rounds.  See Chunk (h2sha_defs.h) for the layout.
-  template <class ForEach>
-  void flush_tile_chunk(const std::vector<Sym>& order, ForEach for_each) {
-    Plan& P = *P_;
-    const uint32_t nd = (uint32_t)order.size();
-    std::vector<std::vector<uint16_t>> gd(nd), ld(nd), md(nd);
-    std::vector<uint32_t> sumdst(nd, 0), res_cnt(nd, 0), res_sum(nd, 0);
-    uint32_t dmin = 0xffffffffu, dmax = 0;
-    for_each([&](uint8_t kind, uint32_t, uint32_t dst, const Sym&) { if (kind == EV_GATE) { dmin = std::min(dmin, dst); dmax = std::max(dmax, dst); } });
-    if (dmin == 0xffffffffu) dmin = dmax = 0;
-    if (dmax - dmin >= cfg_.tile_cells || (dmax - dmin) * 32u >= 0xffffu) fail("tile mode: a chunk has more gate cells than the tile");
-    Chunk c{};
-    c.gate_dst_min = (uint16_t)dmin; c.gate_dst_max = (uint16_t)dmax;
-    c.lk_off = (uint32_t)P.cells.size();
-    uint32_t n_res_cells = 0, n_gate = 0, n_lk = 0, n_limb = 0;
-    std::vector<std::pair<uint32_t, uint32_t>> res_cells;   // (static-table index, tile-relative destination)
-    for_each([&](uint8_t kind, uint32_t vi, uint32_t dst, const Sym& ps) {
-      const Sym& sy = order[vi];
-      const bool res = is_resident(sy);
-      if (kind == EV_GATE) {
-        n_gate++;
-        if (res) { res_cells.push_back({table_index(sy), dst - dmin}); n_res_cells++; res_cnt[vi]++; res_sum[vi] += dst; }
-        else { gd[vi].push_back((uint16_t)(dst - dmin)); sumdst[vi] += dst; }
-      } else if (kind == EV_LK) {
-        const bool ok = (sy.kind == KIND_TABLE && sy.table == T_BYTE) || (sy.kind == KIND_GENERIC && !sy.neg);
-        if (!ok || res || dst >= 0xffff) fail("a looked-up cell holds a constant, a negated or a signed value");
-        ld[vi].push_back((uint16_t)dst); n_lk++;
-      } else {
-        if (res || dst >= 0xffff || !limb_cell_ok(ps, dst)) fail("spread-column cell does not fit its descriptor");
-        md[vi].push_back((uint16_t)dst); n_limb++;
-      }
-    });
-    // Order of the resident-constant cells (lane i % 32 of trip i / 32 handles cell i).  Shared-memory accesses of 16 bytes per lane
-    // are served a quarter-warp at a time over eight 16-byte bank groups; the kernel's lanes store the low half first when even, the
-    // high half first when odd (tile_store), so a quarter's tile stores are conflict-free when its lanes of one parity have distinct
-    // (destination mod 4), and its table loads when different constants sit in different bank groups (index mod 8).
-    {
-      std::vector<uint8_t> taken(res_cells.size(), 0);
-      uint32_t sts[4][2][4] = {}, lds[4][8] = {};
-      std::vector<uint32_t> quarter_consts[4];
-      for (size_t i = 0; i < res_cells.size(); i++) {
-        const uint32_t lane = (uint32_t)(i % 32), q = lane / 8, par = lane & 1u;
-        if (lane == 0) { memset(sts, 0, sizeof sts); memset(lds, 0, sizeof lds); for (auto& v : quarter_consts) v.clear(); }
-        size_t best = res_cells.size(); uint32_t best_cost = 0xffffffffu;
-        for (size_t k = 0; k < res_cells.size(); k++) {
-          if (taken[k]) continue;
-          const uint32_t tbl = res_cells[k].first, d = res_cells[k].second;
-          const bool seen = std::find(quarter_consts[q].begin(), quarter_consts[q].end(), tbl) != quarter_consts[q].end();
-          const uint32_t cost = 2u * sts[q][par][d & 3u] + (seen ? 0u : 2u * lds[q][tbl & 7u]);
-          if (cost < best_cost) { best_cost = cost; best = k; if (!cost) break; }
-        }
-        taken[best] = 1;
-        const uint32_t tbl = res_cells[best].first, d = res_cells[best].second;
-        sts[q][par][d & 3u]++;
-        if (std::find(quarter_consts[q].begin(), quarter_consts[q].end(), tbl) == quarter_consts[q].end()) { quarter_consts[q].push_back(tbl); lds[q][tbl & 7u]++; }
-        if (d * 32u > 0xffffu) fail("tile too large for a 16-bit byte offset");
-        P.cells.push_back(CellEntry{tbl | ((d * 32u) << 16)});
-      }
-    }
-    for (uint32_t i2 = 0; i2 < nd; i2++)
-      if (res_cnt[i2]) {
-        const uint32_t* x = reinterpret_cast<const uint32_t*>(P.mont_table[table_index(order[i2])].l);
-        uint32_t h = 0;
-        for (int k = 0; k < 8; k++) h += x[k] * kCkM[k];
-        c.res_a += (uint64_t)h * (2ull * res_sum[i2]);
-        c.res_b += (uint64_t)h * (uint64_t)res_cnt[i2];
-      }
-    c.fill_off = (uint32_t)P.fill.size();
-    c.gate_off = (uint32_t)P.vdst.size();
-    std::vector<uint32_t> tab_ids, gen_ids;
-    for (int cls = 0; cls < 3; cls++) {
-      std::vector<uint32_t> ids;
-      for (uint32_t i2 = 0; i2 < nd; i2++) if (fill_class(order[i2]) == cls && !is_resident(order[i2])) ids.push_back(i2);
-      std::stable_sort(ids.begin(), ids.end(), [&](uint32_t a, uint32_t b) { return gd[a].size() > gd[b].size(); });
-      auto& dst_ids = cls == 0 ? tab_ids : gen_ids;
-      dst_ids.insert(dst_ids.end(), ids.begin(), ids.end());
-      if (cls == 1) c.n_fill32 = 0;   // (the scratch path's count of <= 32-bit entries is not used in tile mode: the field counts resident cells)
-    }
-    // Lane order inside every batch of 32 and the round in which a value goes to each of its cells: greedy, value by value, so that
-    // in every scatter round the lanes of one quarter-warp and one parity have distinct (destination mod 4) -- see above.
-    for (auto* ids : {&tab_ids, &gen_ids}) {
-      for (size_t b0 = 0; b0 < ids->size(); b0 += 32) {
-        const size_t n_in = std::min<size_t>(32, ids->size() - b0);
-        std::vector<uint32_t> pool(ids->begin() + b0, ids->begin() + b0 + n_in), lanes;
-        std::vector<std::array<std::array<std::array<uint32_t, 4>, 2>, 4>> occ;   // [round][quarter][parity][destination mod 4]
-        while (!pool.empty()) {
-          const uint32_t lane = (uint32_t)lanes.size(), q = lane / 8, par = lane & 1u;
-          const size_t cnt0 = gd[pool[0]].size();   // candidates: the values with as many cells as the next one (keeps the descending order)
-          if (occ.size() < cnt0) occ.resize(cnt0);
-          size_t best_k = 0; uint32_t best_cost = 0xffffffffu; std::vector<uint16_t> best_perm = gd[pool[0]];
-          for (size_t k = 0; k < pool.size() && k < 16 && gd[pool[k]].size() == cnt0 && best_cost; k++) {
-            std::vector<uint16_t> perm = gd[pool[k]];
-            std::sort(perm.begin(), perm.end());
-            int tries = 0;
-            do {
-              uint32_t cost = 0;
-              for (size_t r = 0; r < cnt0; r++) cost += occ[r][q][par][perm[r] & 3u];
-              if (cost < best_cost) { best_cost = cost; best_k = k; best_perm = perm; }
-            } while (best_cost && ++tries < 24 && std::next_permutation(perm.begin(), perm.end()));
-          }
-          const uint32_t v = pool[best_k];
-          gd[v] = best_perm;
-          for (size_t r = 0; r < cnt0; r++) occ[r][q][par][best_perm[r] & 3u]++;
-          lanes.push_back(v);
-          pool.erase(pool.begin() + best_k);
-        }
-        std::copy(lanes.begin(), lanes.end(), ids->begin() + b0);
-      }
-    }
-    for (const auto* ids : {&tab_ids, &gen_ids}) {
-      for (uint32_t i2 : *ids) {
-        const Sym& sy = order[i2];
-        if (gd[i2].size() > 0xffff || ld[i2].size() > 0xffff || md[i2].size() > 0xffff) fail("chunk too large for the fill-entry counters");
-        TmplEntry te = tmpl_pack((uint32_t)md[i2].size(), sy.kind == KIND_TABLE ? table_index(sy) : 0, sy.slot, sy.sh, sy.w, sy.shl, sy.kind, sy.neg);
-        P.fill.push_back(FillEntry{te.lo, te.hi, (uint32_t)gd[i2].size() | ((uint32_t)ld[i2].size() << 16), sumdst[i2]});
-      }
-      for (size_t b0 = 0; b0 < ids->size(); b0 += 32) {
-        const size_t n_in = std::min<size_t>(32, ids->size() - b0);
-        for (const auto* lists : {&gd, &ld, &md}) {
-          size_t R = 0;
-          for (size_t l = 0; l < n_in; l++) R = std::max(R, (*lists)[(*ids)[b0 + l]].size());
-          for (size_t r = 0; r < R; r++)
-            for (size_t l = 0; l < 32; l++) {
-              uint16_t v = 0xffff;
-              if (l < n_in) { const auto& li = (*lists)[(*ids)[b0 + l]]; if (r < li.size()) v = (lists == &gd) ? (uint16_t)(li[r] * 32u) : li[r]; }
-              P.vdst.push_back(v);
-            }
-        }
-      }
-    }
-    c.n_fill_table = (uint16_t)tab_ids.size();
-    c.n_fill = (uint16_t)(tab_ids.size() + gen_ids.size());
-    c.gate_len = (uint16_t)n_gate; c.lk_len = (uint16_t)n_lk; c.limb_len = (uint16_t)n_limb;
-    c.n_fill32 = (uint16_t)n_res_cells;
-    P.chunks.push_back(c);
-  }
-
   void build_chunks(const UnitRec& u, UnitType* ut) {
     // pass 1: greedy, to learn how many chunks the distinct-value limit forces; pass 2: the same number of chunks with
     // balanced cell counts (multiples of 32 gate cells)
     Plan& P = *P_;
     const size_t f0 = P.fill.size(), c0 = P.cells.size(), k0 = P.chunks.size();
-    const size_t v0 = P.vdst.size();
-    build_chunks_pass(u, ut, cfg_.tile_cells ? cfg_.tile_cells : 0xffffffffu);
+    build_chunks_pass(u, ut, 0xffffffffu);
     const uint32_t n = ut->n_chunks;
     if (n > 1) {
-      P.fill.resize(f0); P.cells.resize(c0); P.chunks.resize(k0); P.vdst.resize(v0);
+      P.fill.resize(f0); P.cells.resize(c0); P.chunks.resize(k0);
       uint32_t cap = ((ut->gate_len + n - 1) / n + 31) / 32 * 32;
       build_chunks_pass(u, ut, cap);
     }
@@ -1140,11 +998,6 @@ class Builder {
           index[k] = (uint32_t)order.size();
           order.push_back(pc.s);
         }
-      if (cfg_.tile_cells) {   // value-major phase 2: no scratch slots, destination tables instead of cell lists
-        flush_tile_chunk(order, [&](auto&& visit) { for (auto& pc : cur) visit(pc.kind, index.at(sym_key(pc.s)), pc.dst, pc.s); });
-        cur.clear(); distinct.clear(); gate_in_chunk = 0;
-        return;
-      }
       // ---- scratch slot of every distinct value, chosen to avoid shared-memory bank conflicts in the copy loops ----
       // A 128-bit shared load is served one quarter-warp (8 lanes x 16 B) at a time: two lanes of a quarter conflict
       // when they read different slots with the same (slot mod 8).  Greedy colouring of the co-occurrence graph;
@@ -1407,7 +1260,6 @@ class Builder {
         trial[sym_key(sy)] = sy;
       }
       auto scratch_need = [&](const std::map<uint64_t, Sym>& m) {
-        if (cfg_.tile_cells) return (size_t)0;   // tile mode: no scratch table, only the tile's cell capacity limits a chunk
         size_t n = P.resident.size();
         for (auto& kv : m) if (!is_resident(kv.second)) n++;
         return n;
@@ -1519,37 +1371,6 @@ class Builder {
       std::vector<uint32_t> ent(std::max<uint32_t>(cfg_.max_fill, 1));
       for (uint32_t c = 0; c < ut.n_chunks; c++) {
         const Chunk& ch = P.chunks[ut.chunk_off + c];
-        if (cfg_.tile_cells) {   // tile mode: walk the destination tables the way the kernel does
-          for (uint32_t i = 0; i < ch.n_fill32; i++) {
-            const CellEntry ce = P.cells[ch.lk_off + i];
-            P.map_gate[gate0 + ch.gate_dst_min + (ce.v >> 21)] = 0x80000000u | (ce.v & 0xffffu);
-          }
-          uint32_t voff = ch.gate_off;
-          const uint32_t bounds[3] = {0, ch.n_fill_table, ch.n_fill};
-          for (int grp = 0; grp < 2; grp++)
-            for (uint32_t b0 = bounds[grp]; b0 < bounds[grp + 1]; b0 += 32) {
-              const uint32_t n_in = std::min(32u, bounds[grp + 1] - b0);
-              for (int kind = 0; kind < 3; kind++) {
-                auto count = [&](uint32_t i) {
-                  const FillEntry& e = P.fill[ch.fill_off + i];
-                  return kind == 0 ? H2SHA_FE_GATE_CNT(e) : kind == 1 ? H2SHA_FE_LK_CNT(e) : H2SHA_FE_LIMB_CNT(e);
-                };
-                uint32_t R = 0;
-                for (uint32_t l = 0; l < n_in; l++) R = std::max(R, count(b0 + l));
-                for (uint32_t r = 0; r < R; r++)
-                  for (uint32_t l = 0; l < n_in; l++) {
-                    if (r >= count(b0 + l)) continue;
-                    const uint32_t x = P.vdst[voff + r * 32 + l], entry = doff + b0 + l;
-                    if (kind == 0) P.map_gate[gate0 + ch.gate_dst_min + (x >> 5)] = entry;
-                    else if (kind == 1) P.map_lookup[lk0 + x] = entry;
-                    else ((x & 1u) ? P.map_spread : P.map_dense)[limb0 + (x >> 1)] = entry;
-                  }
-                voff += R * 32;
-              }
-            }
-          doff += ch.n_fill;
-          continue;
-        }
         std::fill(ent.begin(), ent.end(), kUnset);
         for (uint32_t sl = 0; sl < P.resident.size(); sl++) ent[sl] = 0x80000000u | P.resident[sl];
         for (uint32_t i = 0; i < ch.n_fill; i++) ent[H2SHA_TE_DST(P.fill[ch.fill_off + i])] = doff + i;

@@ -28,8 +28,6 @@ struct Config {
   uint32_t max_fill = 144;                        // engine tuning: distinct values per chunk (size of a warp's scratch table)
   uint32_t digest_batch = 0;                      // engine tuning: instances per digest job (0 = as many as fit, <= 32)
   uint32_t resident_consts = 16;                  // engine tuning: most-used constants kept permanently in every warp's scratch
-  uint32_t tile_cells = 0;                        // engine tuning: > 0 = value-major phase 2: chunks of at most this many gate cells are
-                                                  // assembled in a shared-memory tile and leave with one bulk copy (0 = scratch + copy loops)
 };
 
 enum : uint32_t { CP_GATE = 0, CP_FIXED = 1 };
@@ -56,7 +54,6 @@ struct Plan {
   std::vector<FillEntry> fill;          // fill lists of all chunks
   std::vector<uint32_t> resident;       // static-table indices of the constants every warp keeps in scratch slots [0, n)
   std::vector<CellEntry> cells;         // cell lists of all chunks
-  std::vector<uint16_t> vdst;           // tile mode: destination tables of all chunks (see Chunk)
   std::vector<Chunk> chunks;
   std::vector<ItemDesc> items;          // phase-2 work items of all classes
   std::vector<uint32_t> item_dict;      // per item: dictionary index of its chunk's first distinct value, relative to the job's dictionary base

@@ -1,6 +1,6 @@
 #!/bin/bash
 # Builds the engine of another revision next to the in-tree one, for A/B timing on one GPU box:
-#     tools/build_ab.sh <git-rev> [name] [extra nvcc flags, e.g. -DH2SHA_TILE_MODE]   ->  tools/ab/libh2sha_<name>.so   (default name: base)
+#     tools/build_ab.sh <git-rev> [name] [extra nvcc flags, e.g. -DH2SHA_DEBUG_TIMING=2]   ->  tools/ab/libh2sha_<name>.so   (default name: base)
 # <git-rev> may be WORK for the working tree as it is.  engine.cu is linked with every *.cc source that revision has.
 # then e.g.  TUNE_SUSTAIN=1 TUNE_LIB=tools/ab/libh2sha_base.so python tools/tune.py cfg2 parts=3   (tools/ab.sh interleaves A and B).
 # tools/ab/ is scratch: delete it before committing a round (the .so files are git-ignored but would ship to the GPU box).
