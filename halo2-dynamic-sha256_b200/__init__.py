@@ -29,7 +29,7 @@ H2SHA_OK, H2SHA_EINVAL, H2SHA_EPANIC, H2SHA_ECUDA, H2SHA_ENOMEM = 0, -1, -2, -3,
 # symbols include/h2sha_b200.h declares (checked by tests/test_abi.py)
 EXPORTED_SYMBOLS = [
     "h2sha_create", "h2sha_destroy", "h2sha_last_error", "h2sha_build_id", "h2sha_get_layout", "h2sha_get_breaks", "h2sha_get_handles", "h2sha_get_digest_ranges", "h2sha_get_shape", "h2sha_get_lookup_tables",
-    "h2sha_digest_batch", "h2sha_export_instance", "h2sha_export_batch", "h2sha_get_compact_info", "h2sha_get_compact_map", "h2sha_expand_compact", "h2sha_get_lookup_info", "h2sha_lookup_multiplicities", "h2sha_permute_lookup", "h2sha_permute_lookup_from_raw", "h2sha_lookup_product", "h2sha_get_permutation", "h2sha_permutation_product", "h2sha_check_batch", "h2sha_gather", "h2sha_zero_outputs", "h2sha_debug_mont_from_u64", "h2sha_debug_mont_from_u32", "h2sha_debug_store_probe", "h2sha_debug_int_probe", "h2sha_last_launch_count", "h2sha_last_kernel_ms", "H2SHA_CK_M",
+    "h2sha_digest_batch", "h2sha_export_instance", "h2sha_export_batch", "h2sha_get_compact_info", "h2sha_get_compact_map", "h2sha_expand_compact", "h2sha_get_lookup_info", "h2sha_lookup_multiplicities", "h2sha_permute_lookup", "h2sha_permute_lookup_from_raw", "h2sha_lookup_product", "h2sha_get_permutation", "h2sha_permutation_product", "h2sha_permute_lookup_per_instance", "h2sha_permute_lookup_from_raw_per_instance", "h2sha_lookup_product_per_instance", "h2sha_permutation_product_per_instance", "h2sha_check_batch", "h2sha_gather", "h2sha_zero_outputs", "h2sha_debug_mont_from_u64", "h2sha_debug_mont_from_u32", "h2sha_debug_store_probe", "h2sha_debug_int_probe", "h2sha_last_launch_count", "h2sha_last_kernel_ms", "H2SHA_CK_M",
 ]
 
 
@@ -134,6 +134,14 @@ def load_library():
     sig("h2sha_get_permutation", [C.c_void_p, C.POINTER(_PermDesc), C.c_uint32, C.c_void_p])
     sig("h2sha_permutation_product", [C.c_void_p, C.c_uint64, C.POINTER(_PermDesc), C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
+    sig("h2sha_permute_lookup_per_instance", [C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                              C.c_void_p])
+    sig("h2sha_permute_lookup_from_raw_per_instance", [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                       C.c_void_p, C.c_void_p])
+    sig("h2sha_lookup_product_per_instance", [C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p,
+                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
+    sig("h2sha_permutation_product_per_instance", [C.c_void_p, C.c_uint64, C.POINTER(_PermDesc), C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
     sig("h2sha_check_batch", [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
     sig("h2sha_gather", [C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
     sig("h2sha_zero_outputs", [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p])
@@ -572,6 +580,97 @@ class Sha256DynamicConfig:
                                                         bg[0].ctypes.data, bg[1].ctypes.data, z.data_ptr(), err.data_ptr(),
                                                         torch.cuda.current_stream(self.device).cuda_stream))
         return z, int(err.item())
+
+    # ---- per-instance challenges: one (theta_i, beta_i, gamma_i) per instance, for batches of independent proofs ----
+    @staticmethod
+    def _challenge_rows(x, n: int, name: str):
+        """[n, 4] u64 host array (Montgomery) of one challenge per instance, or None."""
+        if x is None:
+            return None
+        a = np.ascontiguousarray(x, dtype=np.uint64)
+        if a.shape != (n, 4):
+            raise EngineError(H2SHA_EINVAL, f"{name} must be [n_instances, 4] u64, not {list(a.shape)}")
+        return a
+
+    def _per_instance_errors(self, n: int):
+        import torch
+        return torch.zeros(n, dtype=torch.int32, device=torch.device("cuda", self.device))
+
+    def permute_lookup_per_instance(self, mult, lookup_idx: int, usable_rows: int, thetas=None):
+        """(A', S', errors) like permute_lookup with theta_i of instance i (`thetas` [n, 4] u64 Montgomery; None for a range lookup).
+        errors [n] int numpy: instance i's multiplicities do not cover usable_rows, or theta_i makes two spread-table rows equal
+        (its A', S' rows are then left unwritten).  Never raises for such per-instance failures."""
+        import torch
+        n = mult.shape[0]
+        th = self._challenge_rows(thetas, n, "thetas")
+        dev = torch.device("cuda", self.device)
+        a = torch.empty((n, usable_rows, 4), dtype=torch.int64, device=dev)
+        s = torch.empty((n, usable_rows, 4), dtype=torch.int64, device=dev)
+        err = self._per_instance_errors(n)
+        _check(load_library().h2sha_permute_lookup_per_instance(self._h, n, lookup_idx, mult.data_ptr(), usable_rows, th.ctypes.data if th is not None else None,
+                                                                a.data_ptr(), s.data_ptr(), err.data_ptr(), torch.cuda.current_stream(self.device).cuda_stream))
+        return a, s, err.cpu().numpy()
+
+    def permute_lookup_from_raw_per_instance(self, first_instance: int, n_instances: int, lookup_idx: int, usable_rows: int, thetas=None):
+        """(A', S', errors) like permute_lookup_per_instance, from the raw value lists the last keep_lookup_raw / lookup_mult batch left in
+        the engine; row i of `thetas` belongs to instance first_instance + i."""
+        import torch
+        th = self._challenge_rows(thetas, n_instances, "thetas")
+        dev = torch.device("cuda", self.device)
+        a = torch.empty((n_instances, usable_rows, 4), dtype=torch.int64, device=dev)
+        s = torch.empty((n_instances, usable_rows, 4), dtype=torch.int64, device=dev)
+        err = self._per_instance_errors(n_instances)
+        _check(load_library().h2sha_permute_lookup_from_raw_per_instance(self._h, first_instance, n_instances, lookup_idx, usable_rows,
+                                                                         th.ctypes.data if th is not None else None, a.data_ptr(), s.data_ptr(),
+                                                                         err.data_ptr(), torch.cuda.current_stream(self.device).cuda_stream))
+        return a, s, err.cpu().numpy()
+
+    def lookup_product_per_instance(self, res: "BatchResult", lookup_idx: int, a_p, s_p, usable_rows: int, betas, gammas, thetas=None):
+        """(z, errors) like lookup_product with theta_i, beta_i, gamma_i of instance i ([n, 4] u64 Montgomery each; thetas only for a
+        spread lookup).  errors [n] int numpy: instance i's z[usable_rows] != 1."""
+        import torch
+        n = a_p.shape[0]
+        if tuple(a_p.shape) != (n, usable_rows, 4) or tuple(s_p.shape) != (n, usable_rows, 4):
+            raise EngineError(H2SHA_EINVAL, "A' and S' must be [n_instances, usable_rows, 4]")
+        for buf in (res.lookup, res.spread):
+            if buf is not None and buf.shape[0] < n:
+                raise EngineError(H2SHA_EINVAL, "the witness holds fewer instances than A' and S'")
+        ch = [self._challenge_rows(x, n, name) for x, name in ((thetas, "thetas"), (betas, "betas"), (gammas, "gammas"))]
+        dev = torch.device("cuda", self.device)
+        z = torch.empty((n, usable_rows + 1, 4), dtype=torch.int64, device=dev)
+        err = self._per_instance_errors(n)
+        ptr = lambda t: t.data_ptr() if t is not None else None
+        _check(load_library().h2sha_lookup_product_per_instance(self._h, n, lookup_idx, ptr(res.lookup), ptr(res.spread), a_p.data_ptr(), s_p.data_ptr(),
+                                                                usable_rows, *[x.ctypes.data if x is not None else None for x in ch], z.data_ptr(),
+                                                                err.data_ptr(), torch.cuda.current_stream(self.device).cuda_stream))
+        return z, err.cpu().numpy()
+
+    def permutation_product_per_instance(self, res: "BatchResult", columns, usable_rows: int, betas, gammas, *, columns_per_chunk: int,
+                                         num_fixed: int = 1, bind_output_bytes: bool = False, digests=None, k: int = 0):
+        """(z, errors) like permutation_product with beta_i, gamma_i of instance i ([n, 4] u64 Montgomery each).  errors [n] int numpy:
+        instance i's last z[usable_rows] != 1."""
+        import torch
+        n = res.gate.shape[0]
+        for buf in (res.lookup, res.spread):
+            if buf is not None and buf.shape[0] < n:
+                raise EngineError(H2SHA_EINVAL, "the witness buffers hold different numbers of instances")
+        bg = [self._challenge_rows(x, n, name) for x, name in ((betas, "betas"), (gammas, "gammas"))]
+        d, cols = self._perm_desc(columns, num_fixed, columns_per_chunk, bind_output_bytes, k)
+        dev = torch.device("cuda", self.device)
+        n_chunks = -(-len(cols) // columns_per_chunk) if columns_per_chunk else 0
+        z = torch.empty((n, n_chunks, usable_rows + 1, 4), dtype=torch.int64, device=dev)
+        err = self._per_instance_errors(n)
+        dg = None
+        if digests is not None:
+            dg = digests if isinstance(digests, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(digests, dtype=np.uint8))
+            dg = dg.to(dev).contiguous()
+            if dg.numel() < n * 32 * len(self.max_variable_byte_sizes):
+                raise EngineError(H2SHA_EINVAL, "digests holds fewer messages than the batch")
+        ptr = lambda t: t.data_ptr() if t is not None else None
+        _check(load_library().h2sha_permutation_product_per_instance(self._h, n, C.byref(d), usable_rows, ptr(res.gate), ptr(res.lookup), ptr(res.spread),
+                                                                     ptr(dg), bg[0].ctypes.data, bg[1].ctypes.data, z.data_ptr(), err.data_ptr(),
+                                                                     torch.cuda.current_stream(self.device).cuda_stream))
+        return z, err.cpu().numpy()
 
     def launches_last_batch(self) -> int:
         return int(load_library().h2sha_last_launch_count(self._h))

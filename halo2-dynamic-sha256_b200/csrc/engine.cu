@@ -1145,6 +1145,8 @@ struct h2sha_engine {
   uint32_t* d_range_tab = nullptr;   // Montgomery form of the range table's values
   uint64_t* d_lp_ws = nullptr;   // lookup product (lookup_product.cuh): spread table, tile products and tile constants
   uint64_t lp_ws_bytes = 0;
+  uint64_t* d_chal = nullptr;    // per-instance challenges of the last *_per_instance call: [n][3][4] theta, beta, gamma (Montgomery)
+  uint64_t chal_bytes = 0;
   // device-side batch check (batch_check.cuh)
   uint32_t *d_chk_gate_on = nullptr, *d_chk_pairs = nullptr, *d_chk_out_bytes = nullptr;
   uint64_t *d_chk_fixed = nullptr, *d_chk_bytes = nullptr;
@@ -1442,7 +1444,7 @@ void h2sha_destroy(h2sha_engine_t* e) {
     if (H.copied) cudaEventDestroy(H.copied);
   if (e->pinned_arena) cudaFreeHost(e->pinned_arena);
   for (int i = 0; i < 4; i++) if (e->ev[i]) cudaEventDestroy(e->ev[i]);
-  cudaFree(e->d_lk_ws); cudaFree(e->d_lk_tab); cudaFree(e->d_range_tab); cudaFree(e->d_lp_ws); cudaFree(e->d_lookup_raw); cudaFree(e->d_dense_raw);
+  cudaFree(e->d_lk_ws); cudaFree(e->d_lk_tab); cudaFree(e->d_range_tab); cudaFree(e->d_lp_ws); cudaFree(e->d_chal); cudaFree(e->d_lookup_raw); cudaFree(e->d_dense_raw);
   h2sha_free_perm_state(e->perm); e->perm = nullptr;
   cudaFree(e->d_chk_gate_on); cudaFree(e->d_chk_pairs); cudaFree(e->d_chk_out_bytes); cudaFree(e->d_chk_fixed); cudaFree(e->d_chk_bytes); cudaFree(e->d_chk_viol);
   delete e;

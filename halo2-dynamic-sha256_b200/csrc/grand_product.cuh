@@ -8,6 +8,7 @@
 // prod u / prod v.  ff's `batch_invert` leaves a zero denominator as zero: a row with v_i = 0 contributes the fraction 0 and every
 // later z is 0.  That is (u_i, v_i) := (0, 1) here.
 // The caller's row source `Rows` says what the rows contribute:
+//   void setup(inst)               run by the whole CTA before any row: loads what its instance needs into shared memory
 //   bool any(h, i0, i1)            does some row in [i0, i1) of chunk h contribute a fraction other than 1?
 //   bool terms(inst, h, i, u, v)   the raw u_i, v_i of row i < rows of chunk h; false (u, v unset) when the row contributes 1
 // Rows split into tiles of GP_TILE contiguous rows of one chunk:
@@ -34,7 +35,16 @@ struct GrandProduct {
   uint64_t* consts;             // [n][n_chunks * tiles_per_chunk][4]: C_t
   uint64_t* z;                  // [n][n_chunks][z_stride] Fr
   uint32_t* errors;             // may be null
+  uint32_t err_stride;          // 0: errors is one counter for the batch; 1: errors[inst] (the *_per_instance calls)
 };
+
+// the challenges of the CTA's instance for the row sources of the *_per_instance calls: theta, beta, gamma (Montgomery), loaded
+// once per CTA from the staged [n][3][4] array instead of once per row (the fill kernel has no registers to spare for them)
+__shared__ uint64_t s_chal[3][4];
+__device__ __forceinline__ void load_chal(const uint64_t* chal, uint64_t inst) {
+  if (threadIdx.x < 12) s_chal[threadIdx.x / 4][threadIdx.x % 4] = chal[inst * 12 + threadIdx.x];
+  __syncthreads();
+}
 
 __device__ __forceinline__ void store_fr(uint64_t* p, const uint64_t x[4]) {
   store_cell2(reinterpret_cast<uint32_t*>(p), make_uint4((uint32_t)x[0], (uint32_t)(x[0] >> 32), (uint32_t)x[1], (uint32_t)(x[1] >> 32)),
@@ -69,6 +79,7 @@ __global__ void __launch_bounds__(GP_THREADS) k_product_tiles(const GrandProduct
   __shared__ uint64_t s_w[GP_THREADS / 32][2][4];
   __shared__ uint32_t s_any[GP_THREADS / 32];
   const uint64_t inst = blockIdx.y;
+  R.setup(inst);
   const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const uint32_t h = blockIdx.x / G.tiles_per_chunk, t0 = (blockIdx.x % G.tiles_per_chunk) * (uint32_t)GP_TILE;
   uint64_t pu[4], pv[4], u[4], v[4];
@@ -146,7 +157,7 @@ __global__ void __launch_bounds__(32 * GP_FOLD_WARPS) k_product_fold(const Grand
     mont_mul_dev(u_all, inv, y);   // the closing value: the last z of the instance
     store_fr(G.z + ((inst + 1) * G.n_chunks * G.z_stride - 1) * 4, y);
     fr_one(x);
-    if (((y[0] ^ x[0]) | (y[1] ^ x[1]) | (y[2] ^ x[2]) | (y[3] ^ x[3])) && G.errors) atomicAdd(G.errors, 1u);
+    if (((y[0] ^ x[0]) | (y[1] ^ x[1]) | (y[2] ^ x[2]) | (y[3] ^ x[3])) && G.errors) atomicAdd(G.errors + inst * G.err_stride, 1u);
   }
 }
 
@@ -154,6 +165,7 @@ template <class Rows>
 __global__ void __launch_bounds__(GP_THREADS) k_product_fill(const GrandProduct G, const Rows R) {
   __shared__ uint64_t s_w[GP_THREADS / 32][2][4];   // per warp: inclusive product of u, of v; then the warp's constant
   const uint64_t inst = blockIdx.y;
+  R.setup(inst);
   const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const uint32_t h = blockIdx.x / G.tiles_per_chunk;
   const uint32_t s = (blockIdx.x % G.tiles_per_chunk) * (uint32_t)GP_TILE + threadIdx.x * GP_ROWS;

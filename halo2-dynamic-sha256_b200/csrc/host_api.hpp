@@ -108,6 +108,30 @@ class Sha256DynamicConfig {
     check(h2sha_permutation_product(engine_, n_instances, &desc, usable_rows, gate, lookup, spread, digests_dev, beta_mont, gamma_mont, z_dev,
                                     errors_dev, stream));
   }
+  // ---- per-instance challenges (independent proofs): challenge arrays [n_instances][4] on the host, errors_dev [n_instances] ----
+  void permute_lookup_per_instance(uint64_t n_instances, uint32_t lookup_idx, const uint32_t* mult_dev, uint32_t usable_rows,
+                                   const uint64_t* thetas_mont, void* permuted_input_dev, void* permuted_table_dev, uint32_t* errors_dev, void* stream) {
+    check(h2sha_permute_lookup_per_instance(engine_, n_instances, lookup_idx, mult_dev, usable_rows, thetas_mont, permuted_input_dev,
+                                            permuted_table_dev, errors_dev, stream));
+  }
+  void permute_lookup_from_raw_per_instance(uint64_t first_instance, uint64_t n_instances, uint32_t lookup_idx, uint32_t usable_rows,
+                                            const uint64_t* thetas_mont, void* permuted_input_dev, void* permuted_table_dev, uint32_t* errors_dev,
+                                            void* stream) {
+    check(h2sha_permute_lookup_from_raw_per_instance(engine_, first_instance, n_instances, lookup_idx, usable_rows, thetas_mont, permuted_input_dev,
+                                                     permuted_table_dev, errors_dev, stream));
+  }
+  void lookup_product_per_instance(uint64_t n_instances, uint32_t lookup_idx, const void* lookup, const void* spread, const void* permuted_input_dev,
+                                   const void* permuted_table_dev, uint32_t usable_rows, const uint64_t* thetas_mont, const uint64_t* betas_mont,
+                                   const uint64_t* gammas_mont, void* z_dev, uint32_t* errors_dev, void* stream) {
+    check(h2sha_lookup_product_per_instance(engine_, n_instances, lookup_idx, lookup, spread, permuted_input_dev, permuted_table_dev, usable_rows,
+                                            thetas_mont, betas_mont, gammas_mont, z_dev, errors_dev, stream));
+  }
+  void permutation_product_per_instance(uint64_t n_instances, const h2sha_perm_desc_t& desc, uint32_t usable_rows, const void* gate,
+                                        const void* lookup, const void* spread, const uint8_t* digests_dev, const uint64_t* betas_mont,
+                                        const uint64_t* gammas_mont, void* z_dev, uint32_t* errors_dev, void* stream) {
+    check(h2sha_permutation_product_per_instance(engine_, n_instances, &desc, usable_rows, gate, lookup, spread, digests_dev, betas_mont, gammas_mont,
+                                                 z_dev, errors_dev, stream));
+  }
   // MockProver-style check of every instance of a batch on the device (lib.rs:525-526): violations[5] = gates, copies,
   // range lookups, spread lookups, digest bytes
   void check_batch(uint64_t n_instances, const void* gate, const void* lookup, const void* spread, const uint8_t* digests_dev,

@@ -15,6 +15,8 @@
 // oracle/lookup_prework.py is the CPU restatement the tests compare against.
 #pragma once
 
+#include <cub/device/device_segmented_sort.cuh>
+
 namespace {
 
 struct LookupGeom {
@@ -101,6 +103,9 @@ struct PermuteArgs {
   uint32_t* vrow;              // [n_inst][usable_rows]: sorted position of the value in row r of A', for r >= m[0] (rows below are the run of 0)
   uint32_t* llist;             // [n_inst][n_vals]: the unused table rows > 0 in increasing order (leftover element j >= lf0 is llist[j - lf0])
   uint32_t* errors;            // may be null
+  uint32_t err_stride;         // 0: errors is one counter for the batch; 1: errors[inst] (the *_per_instance calls)
+  uint32_t tab_stride;         // per-instance spread tables: sorted positions per instance in order / vals (0: one table for the batch)
+  const uint32_t* skip;        // per-instance spread tables: [n_inst] nonzero when theta_i makes two table rows collide, or null
   uint64_t* out_input;         // [n_inst][usable_rows] Fr
   uint64_t* out_table;
 };
@@ -115,6 +120,11 @@ template <int VPT>
 __global__ void __launch_bounds__(1024) k_permute_scan(const PermuteArgs A) {
   __shared__ uint32_t s_part[2][3][32];   // double-buffered by round: two barriers per round
   const uint32_t inst = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  if (A.skip && A.skip[inst]) {   // colliding table rows: counted once, the pair is not written
+    if (tid == 0 && A.errors) atomicAdd(A.errors + (uint64_t)inst * A.err_stride, 1u);
+    return;
+  }
+  const uint32_t* order = A.order ? A.order + (uint64_t)inst * A.tab_stride : nullptr;
   const uint32_t* m = A.mult + (uint64_t)inst * A.mult_stride;
   uint32_t* start = A.scan + (uint64_t)inst * 3 * A.n_vals;
   uint32_t* dpre = start + A.n_vals;
@@ -137,7 +147,7 @@ __global__ void __launch_bounds__(1024) k_permute_scan(const PermuteArgs A) {
     } else {
       mk[0] = 0; lf[0] = 0;
       if (k < A.n_vals) {
-        const uint32_t row = A.order ? A.order[k] : k;
+        const uint32_t row = order ? order[k] : k;
         mk[0] = m[row];
         lf[0] = 1u + (row == 0 ? pad : 0u) - (mk[0] ? 1u : 0u);
       }
@@ -188,7 +198,7 @@ __global__ void __launch_bounds__(1024) k_permute_scan(const PermuteArgs A) {
     } else if (k < A.n_vals) {
       start[k] = ex[0]; dpre[k] = ex[1]; lpre[k] = ex[2];
     }
-    if (A.vrow && A.order == nullptr) {
+    if (A.vrow && order == nullptr) {
       // inverse maps for the fill kernel (identity order: sorted position == table row).  Position 0 is implicit in both:
       // its run is rows [0, m[0]) of A' and its leftover copies are elements [0, lf0) of the leftover sequence.
       uint32_t* vr = A.vrow + (uint64_t)inst * A.usable_rows;
@@ -208,10 +218,10 @@ __global__ void __launch_bounds__(1024) k_permute_scan(const PermuteArgs A) {
   if (tid == 0) {
     A.totals[4 * inst] = base[1];
     A.totals[4 * inst + 1] = base[0];
-    const uint32_t m_first = m[A.order ? A.order[0] : 0];
+    const uint32_t m_first = m[order ? order[0] : 0];
     A.totals[4 * inst + 2] = m_first;
-    A.totals[4 * inst + 3] = 1u + ((A.order ? A.order[0] : 0u) == 0u ? pad : 0u) - (m_first ? 1u : 0u);
-    if (base[0] != A.usable_rows && A.errors) atomicAdd(A.errors, 1u);   // multiplicities do not cover the usable rows
+    A.totals[4 * inst + 3] = 1u + ((order ? order[0] : 0u) == 0u ? pad : 0u) - (m_first ? 1u : 0u);
+    if (base[0] != A.usable_rows && A.errors) atomicAdd(A.errors + (uint64_t)inst * A.err_stride, 1u);   // multiplicities do not cover the usable rows
   }
 }
 
@@ -272,9 +282,9 @@ __device__ __forceinline__ uint32_t last_leq(const uint32_t* __restrict__ a, uin
   return lo;
 }
 
-__device__ __forceinline__ void permuted_value(const PermuteArgs& A, uint32_t k, uint32_t x[8]) {
-  if (A.vals) {
-    const uint4 lo = __ldg(reinterpret_cast<const uint4*>(A.vals + (uint64_t)k * 8)), hi = __ldg(reinterpret_cast<const uint4*>(A.vals + (uint64_t)k * 8) + 1);
+__device__ __forceinline__ void permuted_value(const uint32_t* vals, uint32_t k, uint32_t x[8]) {
+  if (vals) {
+    const uint4 lo = __ldg(reinterpret_cast<const uint4*>(vals + (uint64_t)k * 8)), hi = __ldg(reinterpret_cast<const uint4*>(vals + (uint64_t)k * 8) + 1);
     x[0] = lo.x; x[1] = lo.y; x[2] = lo.z; x[3] = lo.w; x[4] = hi.x; x[5] = hi.y; x[6] = hi.z; x[7] = hi.w;
   } else {
     mont_from_u32(k, x);
@@ -288,9 +298,11 @@ __device__ __forceinline__ void permuted_value(const PermuteArgs& A, uint32_t k,
 __global__ void __launch_bounds__(256) k_permute_fill(const PermuteArgs A) {
   __shared__ uint32_t s_start[256], s_lpre[256];
   const uint32_t inst = blockIdx.y;
+  if (A.skip && A.skip[inst]) return;   // colliding table rows: counted by the scan kernel
   const uint32_t* start = A.scan + (uint64_t)inst * 3 * A.n_vals;
   const uint32_t* dpre = start + A.n_vals;
   const uint32_t* lpre = dpre + A.n_vals;
+  const uint32_t* vals = A.vals ? A.vals + (uint64_t)inst * A.tab_stride * 8 : nullptr;
   const uint32_t n_distinct = A.totals[4 * inst];
   if (A.totals[4 * inst + 1] != A.usable_rows) return;   // inconsistent multiplicities: reported by the scan kernel
   const uint32_t n_rep = A.usable_rows - n_distinct;
@@ -306,12 +318,12 @@ __global__ void __launch_bounds__(256) k_permute_fill(const PermuteArgs A) {
       uint32_t k = 0, st = 0, dp = 0;
       if (row >= m0) { k = __ldg(vr + row); st = __ldg(start + k); dp = __ldg(dpre + k); }
       uint32_t x[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // value 0 is 0 in Montgomery form as well
-      if (k) permuted_value(A, k, x);
+      if (k) permuted_value(vals, k, x);
       store_cell2(out_a + (uint64_t)row * 8, make_uint4(x[0], x[1], x[2], x[3]), make_uint4(x[4], x[5], x[6], x[7]));
       if (row != st) {
         const uint32_t j = n_rep - 1u - (row - dp - 1u);
         const uint32_t w = j < lf0 ? 0u : __ldg(ll + (j - lf0));
-        if (w) permuted_value(A, w, x);
+        if (w) permuted_value(vals, w, x);
         else {
 #pragma unroll
           for (int q = 0; q < 8; q++) x[q] = 0;
@@ -328,7 +340,7 @@ __global__ void __launch_bounds__(256) k_permute_fill(const PermuteArgs A) {
     const uint32_t c = last_leq(s_start, 0, n_coarse, row) * stride;
     const uint32_t k = last_leq(start, c, c + stride, row);
     uint32_t x[8];
-    permuted_value(A, k, x);
+    permuted_value(vals, k, x);
     store_cell2(out_a + (uint64_t)row * 8, make_uint4(x[0], x[1], x[2], x[3]), make_uint4(x[4], x[5], x[6], x[7]));
     if (row != __ldg(start + k)) {
       // a repeated row: halo2 pops the repeated rows from the back while walking the leftover table elements upwards.
@@ -337,7 +349,7 @@ __global__ void __launch_bounds__(256) k_permute_fill(const PermuteArgs A) {
       const uint32_t j = n_rep - 1u - rank;
       const uint32_t c2 = last_leq(s_lpre, 0, n_coarse, j) * stride;
       const uint32_t w = last_leq(lpre, c2, c2 + stride, j);
-      permuted_value(A, w, x);
+      permuted_value(vals, w, x);
     }
     store_cell2(out_s + (uint64_t)row * 8, make_uint4(x[0], x[1], x[2], x[3]), make_uint4(x[4], x[5], x[6], x[7]));
   }
@@ -350,6 +362,143 @@ __global__ void k_range_table(uint32_t* tab, uint32_t n) {
   uint32_t x[8];
   mont_from_u32(i, x);
   store_cell2(tab + (uint64_t)i * 8, make_uint4(x[0], x[1], x[2], x[3]), make_uint4(x[4], x[5], x[6], x[7]));
+}
+
+// Spread table per instance (h2sha_permute_lookup_per_instance): the host path below (compressed_spread_table, std::stable_sort by
+// canonical value, collision check) on the device for every (instance, table row).  The rows are sorted by four stable segmented
+// sorts on the 64-bit limbs of the canonical value, least significant limb first (one segment per instance, the row index as the
+// value): equal to std::stable_sort on the whole 256-bit value for any theta.
+
+// dense * theta + spread of spread-table row i (halo2 `compress_expressions`), Montgomery form: compressed_spread_table on the device
+__device__ __forceinline__ void compressed_spread_row(const uint64_t theta[4], uint32_t i, uint64_t r[4]) {
+  uint64_t d[4], s[4], t[4];
+  mont_from_u64(i, d);
+  mont_from_u64(spread32(i), s);
+  mont_mul_dev(theta, d, t);
+  fr_add_dev(t, s, r);
+}
+
+struct SpreadSort {
+  const uint64_t* chal;   // [n][3][4]: theta_i first
+  uint32_t n_vals;
+  uint64_t* canon;        // [n][4][n_vals]: canonical value of each table row, limb-major
+  uint64_t* key;          // [n][n_vals]: the limb the next sort pass orders by
+  uint32_t* idx;          // [n][n_vals]: table row at each position
+  int* seg;               // [n + 1] segment offsets
+  uint32_t* vals;         // [n][n_vals][8]: Montgomery value at each sorted position
+  uint32_t* skip;         // [n]: two sorted neighbours are equal
+};
+
+// grid (tiles, instances)
+__global__ void __launch_bounds__(256) k_spread_rows(const SpreadSort S) {
+  const uint32_t inst = blockIdx.y, i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i == 0) {
+    S.seg[inst] = (int)(inst * S.n_vals);
+    S.skip[inst] = 0;
+    if (inst + 1 == gridDim.y) S.seg[inst + 1] = (int)((inst + 1) * S.n_vals);
+  }
+  if (i >= S.n_vals) return;
+  uint64_t th[4], cm[4], c[4];
+  load_cell(S.chal + (uint64_t)inst * 12, th);
+  compressed_spread_row(th, i, cm);
+  mont_reduce(cm, c);   // canonical value: what `impl Ord for Fr` compares
+#pragma unroll
+  for (int l = 0; l < 4; l++) S.canon[((uint64_t)inst * 4 + l) * S.n_vals + i] = c[l];
+  S.key[(uint64_t)inst * S.n_vals + i] = c[0];
+  S.idx[(uint64_t)inst * S.n_vals + i] = i;
+}
+
+// the next sort key: limb `limb` of the row at each position
+__global__ void __launch_bounds__(256) k_spread_key(const SpreadSort S, const uint32_t* __restrict__ idx, uint64_t* __restrict__ key, uint32_t limb) {
+  const uint32_t inst = blockIdx.y, k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= S.n_vals) return;
+  const uint64_t p = (uint64_t)inst * S.n_vals + k;
+  key[p] = S.canon[((uint64_t)inst * 4 + limb) * S.n_vals + idx[p]];
+}
+
+// values in sorted order, and the flag of an instance in which two neighbouring sorted values are equal (row 0 compresses to 0, so
+// a row that also compresses to 0 is caught too)
+__global__ void __launch_bounds__(256) k_spread_sorted(const SpreadSort S, const uint32_t* __restrict__ order) {
+  const uint32_t inst = blockIdx.y, k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= S.n_vals) return;
+  const uint64_t p = (uint64_t)inst * S.n_vals + k;
+  const uint32_t row = order[p];
+  uint64_t th[4], cm[4];
+  load_cell(S.chal + (uint64_t)inst * 12, th);
+  compressed_spread_row(th, row, cm);
+  store_cell2(S.vals + p * 8, make_uint4((uint32_t)cm[0], (uint32_t)(cm[0] >> 32), (uint32_t)cm[1], (uint32_t)(cm[1] >> 32)),
+              make_uint4((uint32_t)cm[2], (uint32_t)(cm[2] >> 32), (uint32_t)cm[3], (uint32_t)(cm[3] >> 32)));
+  if (k == 0) return;
+  const uint32_t prev = order[p - 1];
+  const uint64_t* c = S.canon + (uint64_t)inst * 4 * S.n_vals;
+  bool eq = true;
+#pragma unroll
+  for (int l = 0; l < 4; l++) eq = eq && c[(uint64_t)l * S.n_vals + row] == c[(uint64_t)l * S.n_vals + prev];
+  if (eq) atomicOr(S.skip + inst, 1u);
+}
+
+// bytes of the SpreadSort arrays of `ni` instances, and their place in `base` (256-byte aligned each)
+uint64_t spread_sort_layout(uint64_t ni, uint32_t n_vals, uint64_t cub_bytes, uint8_t* base, SpreadSort* S, void** cub_tmp, uint64_t** key_alt, uint32_t** idx_alt) {
+  uint64_t off = 0;
+  auto take = [&](uint64_t bytes) { uint8_t* p = base ? base + off : nullptr; off += (bytes + 255) / 256 * 256; return p; };
+  const uint64_t rows = ni * n_vals;
+  S->vals = (uint32_t*)take(rows * 32);
+  S->canon = (uint64_t*)take(rows * 32);
+  S->key = (uint64_t*)take(rows * 8);
+  *key_alt = (uint64_t*)take(rows * 8);
+  S->idx = (uint32_t*)take(rows * 4);
+  *idx_alt = (uint32_t*)take(rows * 4);
+  S->seg = (int*)take((ni + 1) * 4);
+  S->skip = (uint32_t*)take(ni * 4);
+  *cub_tmp = take(cub_bytes);
+  return off;
+}
+
+// builds, sorts and checks the spread tables of `ni` instances; returns the order (sorted position -> table row) in *order
+int build_spread_tables(SpreadSort S, uint64_t ni, void* cub_tmp, uint64_t cub_bytes, uint64_t* key_alt, uint32_t* idx_alt, const uint32_t** order,
+                        cudaStream_t st) {
+  const dim3 grid((S.n_vals + 255) / 256, (unsigned)ni);
+  k_spread_rows<<<grid, 256, 0, st>>>(S);
+  CUDA_TRY(cudaGetLastError());
+  cub::DoubleBuffer<uint64_t> keys(S.key, key_alt);
+  cub::DoubleBuffer<uint32_t> rows(S.idx, idx_alt);
+  for (uint32_t limb = 0; limb < 4; limb++) {
+    if (limb) {
+      k_spread_key<<<grid, 256, 0, st>>>(S, rows.Current(), keys.Current(), limb);
+      CUDA_TRY(cudaGetLastError());
+    }
+    size_t tmp = cub_bytes;
+    CUDA_TRY(cub::DeviceSegmentedSort::StableSortPairs(cub_tmp, tmp, keys, rows, (int)(ni * S.n_vals), (int)ni, S.seg, S.seg + 1, st));
+  }
+  k_spread_sorted<<<grid, 256, 0, st>>>(S, rows.Current());
+  CUDA_TRY(cudaGetLastError());
+  *order = rows.Current();
+  return H2SHA_OK;
+}
+
+// per-instance challenges: every row of a host array [n][4] must be a reduced field element
+int check_challenge_rows(const uint64_t* a, uint64_t n, const char* name) {
+  for (uint64_t i = 0; i < n; i++)
+    if (fr::geq_p(a + 4 * i)) return set_err(H2SHA_EINVAL, std::string(name) + " row " + std::to_string(i) + " is not a reduced field element");
+  return H2SHA_OK;
+}
+
+// host rows [n][4] of theta, beta, gamma (each may be null: zeros) -> the engine's device array [n][3][4].  The copy goes through a
+// pageable vector, so it is staged before the call returns and the caller may reuse its arrays at once.
+int stage_challenges(h2sha_engine* e, uint64_t n, const uint64_t* theta, const uint64_t* beta, const uint64_t* gamma, cudaStream_t st) {
+  std::vector<uint64_t> host(n * 12, 0);
+  const uint64_t* src[3] = {theta, beta, gamma};
+  for (uint64_t i = 0; i < n; i++)
+    for (int c = 0; c < 3; c++)
+      if (src[c]) memcpy(&host[i * 12 + c * 4], src[c] + 4 * i, 32);
+  const uint64_t need = host.size() * 8;
+  if (need > e->chal_bytes) {
+    cudaFree(e->d_chal); e->d_chal = nullptr; e->chal_bytes = 0;
+    CUDA_TRY(cudaMalloc(&e->d_chal, need));
+    e->chal_bytes = need;
+  }
+  CUDA_TRY(cudaMemcpyAsync(e->d_chal, host.data(), need, cudaMemcpyHostToDevice, st));
+  return H2SHA_OK;
 }
 
 LookupGeom lookup_geom(const h2sha_engine* e, uint64_t n_inst, uint32_t usable_rows) {
@@ -460,9 +609,11 @@ int h2sha_lookup_multiplicities(h2sha_engine_t* e, uint64_t n_instances, const v
 }  // extern "C"
 
 namespace {
-// mult_dev == null: the multiplicities come from the engine's raw value lists (instances first_raw .. of the last keep_lookup_raw batch)
+// mult_dev == null: the multiplicities come from the engine's raw value lists (instances first_raw .. of the last keep_lookup_raw batch).
+// per_inst: theta_mont is [n_instances][4] (rows checked by the caller), errors_dev is [n_instances], and a spread lookup sorts one
+// table per instance on the device.
 int permute_lookup_impl(h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup_idx, const uint32_t* mult_dev, uint64_t first_raw, uint32_t usable_rows,
-                        const uint64_t* theta_mont, void* permuted_input_dev, void* permuted_table_dev, uint32_t* errors_dev, void* stream) {
+                        const uint64_t* theta_mont, bool per_inst, void* permuted_input_dev, void* permuted_table_dev, uint32_t* errors_dev, void* stream) {
   if (!e || !permuted_input_dev || !permuted_table_dev) return set_err(H2SHA_EINVAL, "null argument");
   const bool from_raw = mult_dev == nullptr;
   if (e->device < 0) return set_err(H2SHA_ECUDA, "plan-only engine (device = -1): there is no CPU path");
@@ -479,19 +630,43 @@ int permute_lookup_impl(h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup
   const uint32_t n_vals = is_range ? (1u << G.lookup_bits) : (1u << G.limb_bits);
   // workspace: scans + totals of one chunk of instances (the chunks run one after the other on `stream` and share it)
   if (n_vals > (1u << 22)) return set_err(H2SHA_EINVAL, "lookup table too large for the permutation workspace (lookup_bits > 22)");
-  // instances per pass: at most `lkchunk` (default 256) and at most ~1 GB of scans
+  // instances per pass: at most `lkchunk` (default 256) and at most ~1 GB of scans (and per-instance spread tables)
   const uint64_t per_inst_words = 3ull * n_vals + 4 + (is_range ? (uint64_t)usable_rows + n_vals : 0) + (from_raw ? align_up(n_vals, 4) : 0);   // scans, totals, inverse maps (identity order), this lookup's bins
-  const uint64_t by_mem = std::max<uint64_t>(1, (1ull << 30) / (per_inst_words * 4));
+  const bool sort_tabs = per_inst && !is_range;
+  const uint64_t per_inst_bytes = per_inst_words * 4 + (sort_tabs ? 88ull * n_vals + 8 : 0);
+  const uint64_t by_mem = std::max<uint64_t>(1, (1ull << 30) / per_inst_bytes);
   const uint64_t chunk = std::min<uint64_t>(std::min<uint64_t>(n_instances, by_mem), (uint64_t)std::max(1, tune_value("lkchunk", 256)));
-  const uint64_t need = chunk * per_inst_words * 4;
+  // workspace: [per-instance spread tables of a chunk] [bins of a chunk (from_raw)] [scans, totals, inverse maps of a chunk]
+  size_t cub_bytes = 0;
+  uint64_t sort_bytes = 0;
+  if (sort_tabs) {
+    cub::DoubleBuffer<uint64_t> k0(nullptr, nullptr);
+    cub::DoubleBuffer<uint32_t> v0(nullptr, nullptr);
+    CUDA_TRY(cub::DeviceSegmentedSort::StableSortPairs(nullptr, cub_bytes, k0, v0, (int)(chunk * n_vals), (int)chunk, (int*)nullptr, (int*)nullptr, st));
+    SpreadSort S0{};
+    void* t0; uint64_t* ka0; uint32_t* ia0;
+    sort_bytes = spread_sort_layout(chunk, n_vals, cub_bytes, nullptr, &S0, &t0, &ka0, &ia0);
+  }
+  const uint64_t need = sort_bytes + chunk * per_inst_words * 4;
   if (need > e->lk_ws_bytes) {
     cudaFree(e->d_lk_ws); e->d_lk_ws = nullptr; e->lk_ws_bytes = 0;
     CUDA_TRY(cudaMalloc(&e->d_lk_ws, need));
     e->lk_ws_bytes = need;
   }
   PermuteArgs A{};
-  uint32_t* raw_bins = nullptr;   // from_raw: [chunk][n_vals] at the start of the workspace (16-byte aligned rows for the vectorised scan)
-  uint32_t* ws = e->d_lk_ws;
+  SpreadSort S{};
+  void* cub_tmp = nullptr;
+  uint64_t* key_alt = nullptr;
+  uint32_t* idx_alt = nullptr;
+  if (sort_tabs) {
+    spread_sort_layout(chunk, n_vals, cub_bytes, (uint8_t*)e->d_lk_ws, &S, &cub_tmp, &key_alt, &idx_alt);
+    int rc = stage_challenges(e, n_instances, theta_mont, nullptr, nullptr, st);
+    if (rc) return rc;
+    S.n_vals = n_vals;
+    A.vals = S.vals; A.tab_stride = n_vals; A.skip = S.skip;
+  }
+  uint32_t* raw_bins = nullptr;   // from_raw: [chunk][n_vals] (16-byte aligned rows for the vectorised scan)
+  uint32_t* ws = e->d_lk_ws + sort_bytes / 4;
   if (from_raw) {
     raw_bins = ws;
     ws += chunk * (uint64_t)align_up(n_vals, 4);
@@ -504,13 +679,13 @@ int permute_lookup_impl(h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup
   A.n_vals = n_vals; A.usable_rows = usable_rows;
   A.scan = ws; A.totals = ws + chunk * 3ull * n_vals;
   if (is_range && tune_value("lkinv", 1)) { A.vrow = A.totals + chunk * 4; A.llist = A.vrow + chunk * (uint64_t)usable_rows; }
-  A.errors = errors_dev;
+  A.err_stride = per_inst ? 1u : 0u;
   A.out_input = (uint64_t*)permuted_input_dev; A.out_table = (uint64_t*)permuted_table_dev;
   if (is_range) {
     int rc = ensure_range_tab(e, st);
     if (rc) return rc;
     A.vals = tune_value("lktab", 1) ? e->d_range_tab : nullptr;   // lktab=0: convert each value on the fly (mont_from_u32) instead of the 32-byte gather
-  } else {
+  } else if (!sort_tabs) {
     // the compressed table rows sorted by canonical value (`impl Ord for Fr`)
     U256 th_m; memcpy(th_m.l, theta_mont, 32);
     if (fr::geq_p(th_m.l)) return set_err(H2SHA_EINVAL, "theta is not a reduced field element");
@@ -548,6 +723,12 @@ int permute_lookup_impl(h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup
     } else {
       A.mult = mult0 + i0 * A.mult_stride;
     }
+    if (sort_tabs) {
+      S.chal = e->d_chal + i0 * 12;
+      int rc = build_spread_tables(S, ni, cub_tmp, cub_bytes, key_alt, idx_alt, &A.order, st);
+      if (rc) return rc;
+    }
+    A.errors = errors_dev ? errors_dev + (per_inst ? i0 : 0) : nullptr;
     A.out_input = (uint64_t*)permuted_input_dev + i0 * (uint64_t)usable_rows * 4;
     A.out_table = (uint64_t*)permuted_table_dev + i0 * (uint64_t)usable_rows * 4;
     {
@@ -570,7 +751,7 @@ extern "C" {
 int h2sha_permute_lookup(h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup_idx, const uint32_t* mult_dev, uint32_t usable_rows,
                          const uint64_t* theta_mont, void* permuted_input_dev, void* permuted_table_dev, uint32_t* errors_dev, void* stream) {
   if (!mult_dev) return set_err(H2SHA_EINVAL, "null argument");
-  return permute_lookup_impl(e, n_instances, lookup_idx, mult_dev, 0, usable_rows, theta_mont, permuted_input_dev, permuted_table_dev, errors_dev, stream);
+  return permute_lookup_impl(e, n_instances, lookup_idx, mult_dev, 0, usable_rows, theta_mont, false, permuted_input_dev, permuted_table_dev, errors_dev, stream);
 }
 
 int h2sha_permute_lookup_from_raw(h2sha_engine_t* e, uint64_t first_instance, uint64_t n_instances, uint32_t lookup_idx, uint32_t usable_rows,
@@ -578,7 +759,31 @@ int h2sha_permute_lookup_from_raw(h2sha_engine_t* e, uint64_t first_instance, ui
   if (!e) return set_err(H2SHA_EINVAL, "null argument");
   if (first_instance + n_instances > e->raw_n)
     return set_err(H2SHA_EINVAL, "the engine holds no raw value lists for these instances: generate the batch with keep_lookup_raw (or lookup_mult_dev) first");
-  return permute_lookup_impl(e, n_instances, lookup_idx, nullptr, first_instance, usable_rows, theta_mont, permuted_input_dev, permuted_table_dev, errors_dev, stream);
+  return permute_lookup_impl(e, n_instances, lookup_idx, nullptr, first_instance, usable_rows, theta_mont, false, permuted_input_dev, permuted_table_dev, errors_dev, stream);
+}
+
+// the checks of the per-instance calls that need no device: the plan-only engine is refused after them, by permute_lookup_impl
+static int check_permute_per_instance(const h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup_idx, const uint64_t* thetas_mont) {
+  if (!e) return set_err(H2SHA_EINVAL, "null argument");
+  const bool is_range = lookup_idx < e->plan.n_lookup_cols;
+  if (!is_range && lookup_idx < e->plan.n_lookup_cols + e->plan.cfg.spread_cols && !thetas_mont)
+    return set_err(H2SHA_EINVAL, "a spread lookup has two expressions: thetas_mont is needed to compress them");
+  return !is_range && thetas_mont ? check_challenge_rows(thetas_mont, n_instances, "thetas_mont") : H2SHA_OK;
+}
+
+int h2sha_permute_lookup_per_instance(h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup_idx, const uint32_t* mult_dev, uint32_t usable_rows,
+                                      const uint64_t* thetas_mont, void* permuted_input_dev, void* permuted_table_dev, uint32_t* errors_dev, void* stream) {
+  if (!mult_dev) return set_err(H2SHA_EINVAL, "null argument");
+  if (int rc = check_permute_per_instance(e, n_instances, lookup_idx, thetas_mont)) return rc;
+  return permute_lookup_impl(e, n_instances, lookup_idx, mult_dev, 0, usable_rows, thetas_mont, true, permuted_input_dev, permuted_table_dev, errors_dev, stream);
+}
+
+int h2sha_permute_lookup_from_raw_per_instance(h2sha_engine_t* e, uint64_t first_instance, uint64_t n_instances, uint32_t lookup_idx, uint32_t usable_rows,
+                                               const uint64_t* thetas_mont, void* permuted_input_dev, void* permuted_table_dev, uint32_t* errors_dev, void* stream) {
+  if (int rc = check_permute_per_instance(e, n_instances, lookup_idx, thetas_mont)) return rc;
+  if (first_instance + n_instances > e->raw_n)
+    return set_err(H2SHA_EINVAL, "the engine holds no raw value lists for these instances: generate the batch with keep_lookup_raw (or lookup_mult_dev) first");
+  return permute_lookup_impl(e, n_instances, lookup_idx, nullptr, first_instance, usable_rows, thetas_mont, true, permuted_input_dev, permuted_table_dev, errors_dev, stream);
 }
 
 }  // extern "C"

@@ -9,7 +9,9 @@
 //   plan (host, once per desc)  permutation.cc replays the copies; the moved cells, sorted by (chunk, row), with their source
 //                               (buffer and Fr offset in an instance, fixed constant, digest byte), identity delta^j w^r and sigma;
 //                               per chunk a row index ptr[h][0 .. U+1] into that list
-//   k_perm_prep                 per call: a = beta id + gamma, b = beta sigma + gamma per moved cell (shared by all instances)
+//   k_perm_prep                 per call: a = beta id + gamma, b = beta sigma + gamma per moved cell (shared by all instances);
+//                               with per-instance challenges (h2sha_permutation_product_per_instance) a and b are formed in the row
+//                               source instead, from the resident identity and sigma and the CTA's beta_i, gamma_i
 //   grand_product.cuh           with the row source PermRows: u_i = prod (p + a), v_i = prod (p + b) over the moved cells of a row;
 //                               rows run 0 .. U in every chunk (row U has no moved cell), so the fill writes z[0 .. U] of every
 //                               chunk, and the closing value the fold checks against 1 is the last chunk's z[U]
@@ -24,7 +26,8 @@ namespace {
 enum : uint64_t { PS_GATE = 0, PS_LOOKUP = 1, PS_SPREAD = 2, PS_FIXED = 3, PS_BYTE = 4, PS_ZERO = 5 };   // source kind (bits 60..63)
 constexpr uint64_t PS_OFF_MASK = (1ull << 60) - 1;
 
-// the moved cells of a batch as a row source of grand_product.cuh
+// the moved cells of a batch as a row source of grand_product.cuh; PI: beta and gamma per instance, from s_chal
+template <bool PI>
 struct PermRows {
   const uint64_t* gate;         // batch buffers at instance 0 of the launch
   const uint64_t* lookup;
@@ -35,10 +38,14 @@ struct PermRows {
   const uint64_t* fixed;        // [n_fixed][4] Montgomery
   const uint64_t* bytes;        // [256][4] Montgomery of 0 .. 255
   const uint64_t* src;          // [n_moved] (kind << 60) | offset
-  const uint64_t* ab;           // [n_moved][2][4]: beta id + gamma, beta sigma + gamma
+  const uint64_t* ab;           // [n_moved][2][4]: beta id + gamma, beta sigma + gamma; PI: id, sigma
   const uint32_t* ptr;          // [n_chunks][U + 2]: first moved cell of each row
   uint32_t usable_rows;
+  const uint64_t* chal;         // PI: [n][3][4] at instance 0 of the launch
 
+  __device__ __forceinline__ void setup(uint64_t inst) const {
+    if constexpr (PI) load_chal(chal, inst);
+  }
   __device__ __forceinline__ bool any(uint32_t h, uint32_t i0, uint32_t i1) const;
   __device__ bool terms(uint64_t inst, uint32_t h, uint32_t i, uint64_t u[4], uint64_t v[4]) const;
 };
@@ -59,7 +66,8 @@ __global__ void k_perm_prep(const uint64_t* __restrict__ idsig, uint64_t* __rest
   }
 }
 
-__device__ __forceinline__ void perm_value(const PermRows& A, uint64_t inst, uint64_t s, uint64_t p[4]) {
+template <class Rows>
+__device__ __forceinline__ void perm_value(const Rows& A, uint64_t inst, uint64_t s, uint64_t p[4]) {
   const uint64_t off = s & PS_OFF_MASK;
   switch (s >> 60) {
     case PS_GATE: load_cell(A.gate + (inst * A.gate_inst + off) * 4, p); break;
@@ -72,20 +80,34 @@ __device__ __forceinline__ void perm_value(const PermRows& A, uint64_t inst, uin
 }
 
 // a moved cell in rows [i0, i1) of chunk h (ptr ends at index U + 1)
-__device__ __forceinline__ bool PermRows::any(uint32_t h, uint32_t i0, uint32_t i1) const {
+template <bool PI>
+__device__ __forceinline__ bool PermRows<PI>::any(uint32_t h, uint32_t i0, uint32_t i1) const {
   const uint32_t* pr = ptr + (uint64_t)h * (usable_rows + 2);
   return pr[min(i0, usable_rows + 1)] != pr[min(i1, usable_rows + 1)];
 }
 
 // u, v of a row from its moved cells [k0, k1); false for a row without any
-__device__ bool PermRows::terms(uint64_t inst, uint32_t h, uint32_t i, uint64_t u[4], uint64_t v[4]) const {
+template <bool PI>
+__device__ bool PermRows<PI>::terms(uint64_t inst, uint32_t h, uint32_t i, uint64_t u[4], uint64_t v[4]) const {
   const uint32_t* pr = ptr + (uint64_t)h * (usable_rows + 2);
   const uint32_t k0 = pr[i], k1 = pr[i + 1];
   if (k0 == k1) return false;
   uint64_t p[4], t[4];
   for (uint32_t k = k0; k < k1; k++) {
     perm_value(*this, inst, src[k], p);
-    if (k == k0) {
+    if constexpr (PI) {   // p + beta x + gamma for x = id, sigma: two more products per moved cell than the shared path
+      uint64_t x[4], a[4];
+#pragma unroll
+      for (int q = 0; q < 2; q++) {
+        load_cell(ab + (uint64_t)k * 8 + 4 * q, x);
+        mont_mul_dev(s_chal[1], x, t);
+        fr_add_dev(t, s_chal[2], a);
+        fr_add_dev(p, a, x);
+        uint64_t* acc = q ? v : u;
+        if (k == k0) fr_copy(x, acc);
+        else fr_mul_into(acc, x);
+      }
+    } else if (k == k0) {
       fr_add_dev(p, ab + (uint64_t)k * 8, u);
       fr_add_dev(p, ab + (uint64_t)k * 8 + 4, v);
     } else {
@@ -217,15 +239,20 @@ int h2sha_get_permutation(h2sha_engine_t* e, const h2sha_perm_desc_t* desc, uint
   return H2SHA_OK;
 }
 
-int h2sha_permutation_product(h2sha_engine_t* e, uint64_t n_instances, const h2sha_perm_desc_t* desc, uint32_t usable_rows,
-                              const void* gate, const void* lookup, const void* spread, const uint8_t* digests_dev,
-                              const uint64_t* beta_mont, const uint64_t* gamma_mont, void* z_dev, uint32_t* errors_dev, void* stream) {
+}  // extern "C"
+
+namespace {
+
+// per_inst: beta_mont and gamma_mont are [n_instances][4] with rows checked by the caller, errors_dev is [n_instances]
+int permutation_product_impl(h2sha_engine_t* e, uint64_t n_instances, const h2sha_perm_desc_t* desc, uint32_t usable_rows,
+                             const void* gate, const void* lookup, const void* spread, const uint8_t* digests_dev,
+                             const uint64_t* beta_mont, const uint64_t* gamma_mont, bool per_inst, void* z_dev, uint32_t* errors_dev, void* stream) {
   if (!e || !desc || !beta_mont || !gamma_mont || !z_dev) return set_err(H2SHA_EINVAL, "null argument");
   const Plan& P = e->plan;
   PermColumns C;
   std::string err;
   if (!perm_columns(P, *desc, usable_rows, &C, &err)) return set_err(H2SHA_EINVAL, err);
-  if (fr::geq_p(beta_mont) || fr::geq_p(gamma_mont)) return set_err(H2SHA_EINVAL, "beta and gamma must be reduced field elements");
+  if (!per_inst && (fr::geq_p(beta_mont) || fr::geq_p(gamma_mont))) return set_err(H2SHA_EINVAL, "beta and gamma must be reduced field elements");
   if (e->device < 0) return set_err(H2SHA_ECUDA, "plan-only engine (device = -1): there is no CPU path");
   bool reads[3] = {false, false, false};
   for (uint32_t k : C.kind) {
@@ -245,19 +272,15 @@ int h2sha_permutation_product(h2sha_engine_t* e, uint64_t n_instances, const h2s
   if (rc) return rc;
   h2sha_perm_state* S = e->perm;
   cudaStream_t st = (cudaStream_t)stream;
-  PermRows A{};
-  A.usable_rows = usable_rows;
-  A.gate_inst = e->dplan.gate_inst_cells; A.lookup_inst = e->dplan.lookup_inst_cells; A.spread_inst = e->dplan.spread_inst_cells;
-  A.digest_bytes = 32u * (uint32_t)P.digests.size();
-  A.fixed = S->d_fixed; A.bytes = S->d_bytes; A.src = S->d_src; A.ab = S->d_ab; A.ptr = S->d_ptr;
   GrandProduct Z{};
   Z.rows = usable_rows + 1; Z.n_chunks = C.n_chunks; Z.z_stride = usable_rows + 1;
   Z.tiles_per_chunk = (uint32_t)((usable_rows + 1ull + GP_TILE - 1) / GP_TILE);
   const uint32_t n_tiles = Z.n_chunks * Z.tiles_per_chunk;
-  // per call: a, b of every moved cell
-  PermChallenges ch;
-  memcpy(ch.beta, beta_mont, 32); memcpy(ch.gamma, gamma_mont, 32);
-  if (S->n_moved) {
+  if (per_inst) {
+    if ((rc = stage_challenges(e, n_instances, nullptr, beta_mont, gamma_mont, st))) return rc;
+  } else if (S->n_moved) {   // per call: a, b of every moved cell
+    PermChallenges ch;
+    memcpy(ch.beta, beta_mont, 32); memcpy(ch.gamma, gamma_mont, 32);
     k_perm_prep<<<(S->n_moved + 255) / 256, 256, 0, st>>>(S->d_idsig, S->d_ab, S->n_moved, ch);
     CUDA_TRY(cudaGetLastError());
   }
@@ -271,17 +294,54 @@ int h2sha_permutation_product(h2sha_engine_t* e, uint64_t n_instances, const h2s
   }
   Z.tiles = S->d_ws;
   Z.consts = S->d_ws + chunk * n_tiles * 8;
-  Z.errors = errors_dev;
-  for (uint64_t i0 = 0; i0 < n_instances; i0 += chunk) {
-    const unsigned ni = (unsigned)std::min<uint64_t>(chunk, n_instances - i0);
-    A.gate = gate ? (const uint64_t*)gate + i0 * A.gate_inst * 4 : nullptr;
-    A.lookup = lookup ? (const uint64_t*)lookup + i0 * A.lookup_inst * 4 : nullptr;
-    A.spread = spread ? (const uint64_t*)spread + i0 * A.spread_inst * 4 : nullptr;
-    A.digests = digests_dev ? digests_dev + i0 * A.digest_bytes : nullptr;
-    Z.z = (uint64_t*)z_dev + i0 * Z.n_chunks * (usable_rows + 1ull) * 4;
-    if ((rc = launch_product(Z, A, ni, st))) return rc;
+  Z.err_stride = per_inst ? 1u : 0u;
+  auto run = [&](auto& A) {
+    A.usable_rows = usable_rows;
+    A.gate_inst = e->dplan.gate_inst_cells; A.lookup_inst = e->dplan.lookup_inst_cells; A.spread_inst = e->dplan.spread_inst_cells;
+    A.digest_bytes = 32u * (uint32_t)P.digests.size();
+    A.fixed = S->d_fixed; A.bytes = S->d_bytes; A.src = S->d_src; A.ptr = S->d_ptr;
+    A.ab = per_inst ? S->d_idsig : S->d_ab;
+    for (uint64_t i0 = 0; i0 < n_instances; i0 += chunk) {
+      const unsigned ni = (unsigned)std::min<uint64_t>(chunk, n_instances - i0);
+      A.gate = gate ? (const uint64_t*)gate + i0 * A.gate_inst * 4 : nullptr;
+      A.lookup = lookup ? (const uint64_t*)lookup + i0 * A.lookup_inst * 4 : nullptr;
+      A.spread = spread ? (const uint64_t*)spread + i0 * A.spread_inst * 4 : nullptr;
+      A.digests = digests_dev ? digests_dev + i0 * A.digest_bytes : nullptr;
+      if (per_inst) A.chal = e->d_chal + i0 * 12;
+      Z.z = (uint64_t*)z_dev + i0 * Z.n_chunks * (usable_rows + 1ull) * 4;
+      Z.errors = errors_dev ? errors_dev + (per_inst ? i0 : 0) : nullptr;
+      if (int r = launch_product(Z, A, ni, st)) return r;
+    }
+    return (int)H2SHA_OK;
+  };
+  if (per_inst) {
+    PermRows<true> A{};
+    return run(A);
   }
-  return H2SHA_OK;
+  PermRows<false> A{};
+  return run(A);
+}
+
+}  // namespace
+
+extern "C" {
+
+int h2sha_permutation_product(h2sha_engine_t* e, uint64_t n_instances, const h2sha_perm_desc_t* desc, uint32_t usable_rows,
+                              const void* gate, const void* lookup, const void* spread, const uint8_t* digests_dev,
+                              const uint64_t* beta_mont, const uint64_t* gamma_mont, void* z_dev, uint32_t* errors_dev, void* stream) {
+  return permutation_product_impl(e, n_instances, desc, usable_rows, gate, lookup, spread, digests_dev, beta_mont, gamma_mont, false, z_dev,
+                                  errors_dev, stream);
+}
+
+int h2sha_permutation_product_per_instance(h2sha_engine_t* e, uint64_t n_instances, const h2sha_perm_desc_t* desc, uint32_t usable_rows,
+                                           const void* gate, const void* lookup, const void* spread, const uint8_t* digests_dev,
+                                           const uint64_t* betas_mont, const uint64_t* gammas_mont, void* z_dev, uint32_t* errors_dev, void* stream) {
+  if (!e || !betas_mont || !gammas_mont) return set_err(H2SHA_EINVAL, "null argument");
+  int rc;
+  if ((rc = check_challenge_rows(betas_mont, n_instances, "betas_mont")) || (rc = check_challenge_rows(gammas_mont, n_instances, "gammas_mont"))) return rc;
+  return permutation_product_impl(e, n_instances, desc, usable_rows, gate, lookup, spread, digests_dev, betas_mont, gammas_mont, true, z_dev,
+                                  errors_dev, stream);
 }
 
 }  // extern "C"
+

@@ -303,6 +303,34 @@ int h2sha_permutation_product(h2sha_engine_t* e, uint64_t n_instances, const h2s
                               const void* gate, const void* lookup, const void* spread, const uint8_t* digests_dev,
                               const uint64_t* beta_mont, const uint64_t* gamma_mont, void* z_dev, uint32_t* errors_dev, void* stream);
 
+/* ---- Per-instance challenges ---------------------------------------------------------------------------------------------
+ * The four calls above take one theta / beta / gamma for the whole batch: right when the batch holds the circuits of ONE
+ * create_proof over many circuits.  A batch of independent proofs (one per message or request) has one transcript, and so one
+ * (theta_i, beta_i, gamma_i), per instance; these four calls take them, at batch speed:
+ *   thetas_mont / betas_mont / gammas_mont   host [n_instances][4] u64 Montgomery; row i belongs to instance i of the call (for
+ *                          from_raw: instance first_instance + i, like the output rows).  Every row must be reduced (< p), or the
+ *                          call returns H2SHA_EINVAL naming the row.  thetas_mont may be NULL for a range lookup.  The rows are
+ *                          staged before the call returns (the caller may reuse the arrays at once); the call stays asynchronous.
+ *   errors_dev             device [n_instances] u32, or NULL: entry i is incremented (never zeroed) when instance i fails for a
+ *                          reason that increments the shared calls' single counter, and, for the permuted pair of a spread lookup,
+ *                          when theta_i makes two compressed table rows equal (the shared call refuses such a theta with
+ *                          H2SHA_EINVAL; here only that instance is counted and its A', S' rows are left unwritten).
+ * Every other argument is that of the matching shared call.  For every instance the outputs are bit-identical to the shared call
+ * on that instance alone with row i's challenges; with all rows equal they are bit-identical to the shared call on the batch, and
+ * the per-instance errors sum to its counter.  A slice of a batch is passed by offsetting every pointer, the challenge arrays too.
+ * The spread table of each instance is compressed, sorted by canonical value and checked on the device. */
+int h2sha_permute_lookup_per_instance(h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup_idx, const uint32_t* mult_dev, uint32_t usable_rows,
+                                      const uint64_t* thetas_mont, void* permuted_input_dev, void* permuted_table_dev, uint32_t* errors_dev, void* stream);
+int h2sha_permute_lookup_from_raw_per_instance(h2sha_engine_t* e, uint64_t first_instance, uint64_t n_instances, uint32_t lookup_idx, uint32_t usable_rows,
+                                               const uint64_t* thetas_mont, void* permuted_input_dev, void* permuted_table_dev, uint32_t* errors_dev, void* stream);
+int h2sha_lookup_product_per_instance(h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup_idx, const void* lookup, const void* spread,
+                                      const void* permuted_input_dev, const void* permuted_table_dev, uint32_t usable_rows,
+                                      const uint64_t* thetas_mont, const uint64_t* betas_mont, const uint64_t* gammas_mont,
+                                      void* z_dev, uint32_t* errors_dev, void* stream);
+int h2sha_permutation_product_per_instance(h2sha_engine_t* e, uint64_t n_instances, const h2sha_perm_desc_t* desc, uint32_t usable_rows,
+                                           const void* gate, const void* lookup, const void* spread, const uint8_t* digests_dev,
+                                           const uint64_t* betas_mont, const uint64_t* gammas_mont, void* z_dev, uint32_t* errors_dev, void* stream);
+
 /* MockProver-style check of a whole batch where it lies, in HBM -- what the reference's tests accept a witness by
  * (`MockProver::run(..).verify() == Ok(())`, lib.rs:525-526), for every instance instead of one:
  *   violations[0] gates           q * (a + b*c - d) = 0 on every enabled gate row (halo2-base FlexGate, Vertical)

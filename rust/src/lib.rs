@@ -382,6 +382,48 @@ pub mod batch {
         check(unsafe { h2sha_permutation_product(engine, n as u64, desc, usable_rows, gate as *const _, lookup as *const _, spread as *const _,
                                                  digests_dev as *const u8, beta_mont.as_ptr(), gamma_mont.as_ptr(), z_dev as *mut _, errors_dev as *mut u32, stream) })
     }
+    /// Per-instance challenges, for a batch of independent proofs: row i of `thetas_mont` ([n][4] Montgomery limbs) belongs to
+    /// instance i; `thetas_mont` may be empty for a range lookup.  errors_dev: device [n] u32 (or 0), entry i counts instance i's failures.
+    pub fn permute_lookup_per_instance(engine: *mut h2sha_engine_t, n: usize, lookup_idx: u32, mult_dev: u64, usable_rows: u32, thetas_mont: &[[u64; 4]],
+                                       permuted_input_dev: u64, permuted_table_dev: u64, errors_dev: u64, stream: *mut std::ffi::c_void) -> Result<(), Error> {
+        if !thetas_mont.is_empty() && thetas_mont.len() != n { return Err(Error::Synthesis); }
+        let th = if thetas_mont.is_empty() { std::ptr::null() } else { thetas_mont.as_ptr() as *const u64 };
+        check(unsafe { h2sha_permute_lookup_per_instance(engine, n as u64, lookup_idx, mult_dev as *const u32, usable_rows, th, permuted_input_dev as *mut _,
+                                                         permuted_table_dev as *mut _, errors_dev as *mut u32, stream) })
+    }
+    /// `permute_lookup_per_instance` from the raw value lists of the last keep_lookup_raw batch: row i of `thetas_mont` belongs to
+    /// instance first_instance + i.
+    pub fn permute_lookup_from_raw_per_instance(engine: *mut h2sha_engine_t, first_instance: usize, n: usize, lookup_idx: u32, usable_rows: u32,
+                                                thetas_mont: &[[u64; 4]], permuted_input_dev: u64, permuted_table_dev: u64, errors_dev: u64,
+                                                stream: *mut std::ffi::c_void) -> Result<(), Error> {
+        if !thetas_mont.is_empty() && thetas_mont.len() != n { return Err(Error::Synthesis); }
+        let th = if thetas_mont.is_empty() { std::ptr::null() } else { thetas_mont.as_ptr() as *const u64 };
+        check(unsafe { h2sha_permute_lookup_from_raw_per_instance(engine, first_instance as u64, n as u64, lookup_idx, usable_rows, th,
+                                                                  permuted_input_dev as *mut _, permuted_table_dev as *mut _, errors_dev as *mut u32, stream) })
+    }
+    /// halo2 `commit_product` of one lookup with per-instance (theta_i, beta_i, gamma_i); `thetas_mont` may be empty for a range lookup.
+    pub fn lookup_product_per_instance(engine: *mut h2sha_engine_t, n: usize, lookup_idx: u32, lookup: u64, spread: u64, permuted_input_dev: u64,
+                                       permuted_table_dev: u64, usable_rows: u32, thetas_mont: &[[u64; 4]], betas_mont: &[[u64; 4]],
+                                       gammas_mont: &[[u64; 4]], z_dev: u64, errors_dev: u64, stream: *mut std::ffi::c_void) -> Result<(), Error> {
+        if (!thetas_mont.is_empty() && thetas_mont.len() != n) || betas_mont.len() != n || gammas_mont.len() != n {
+            return Err(Error::Synthesis); // one challenge row per instance
+        }
+        let th = if thetas_mont.is_empty() { std::ptr::null() } else { thetas_mont.as_ptr() as *const u64 };
+        check(unsafe { h2sha_lookup_product_per_instance(engine, n as u64, lookup_idx, lookup as *const _, spread as *const _, permuted_input_dev as *const _,
+                                                         permuted_table_dev as *const _, usable_rows, th, betas_mont.as_ptr() as *const u64,
+                                                         gammas_mont.as_ptr() as *const u64, z_dev as *mut _, errors_dev as *mut u32, stream) })
+    }
+    /// `permutation_product` with per-instance (beta_i, gamma_i).
+    pub fn permutation_product_per_instance(engine: *mut h2sha_engine_t, n: usize, desc: &h2sha_perm_desc_t, usable_rows: u32, gate: u64, lookup: u64,
+                                            spread: u64, digests_dev: u64, betas_mont: &[[u64; 4]], gammas_mont: &[[u64; 4]], z_dev: u64, errors_dev: u64,
+                                            stream: *mut std::ffi::c_void) -> Result<(), Error> {
+        if betas_mont.len() != n || gammas_mont.len() != n {
+            return Err(Error::Synthesis); // one challenge row per instance
+        }
+        check(unsafe { h2sha_permutation_product_per_instance(engine, n as u64, desc, usable_rows, gate as *const _, lookup as *const _, spread as *const _,
+                                                              digests_dev as *const u8, betas_mont.as_ptr() as *const u64, gammas_mont.as_ptr() as *const u64,
+                                                              z_dev as *mut _, errors_dev as *mut u32, stream) })
+    }
     /// `MockProver::run(..).verify()` (lib.rs:525-526) for every instance of a batch, on the device.
     pub fn check_batch(engine: *mut h2sha_engine_t, n: usize, gate: u64, lookup: u64, spread: u64, digests_dev: u64, stream: *mut std::ffi::c_void) -> Result<[u64; 5], Error> {
         let mut v = [0u64; 5];
