@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libh2sha_b200.so")
 SOURCES = ["engine.cu", "planner.cc", "permutation.cc"]
-HEADERS = ["h2sha_defs.h", "planner.h", "fr_host.h", "fr_dev.cuh", "lookup_prework.cuh", "batch_check.cuh", "grand_product.cuh", "lookup_product.cuh", "permutation.h", "permutation_product.cuh", "export.cuh", os.path.join("..", "..", "include", "h2sha_b200.h")]
+HEADERS = ["h2sha_defs.h", "planner.h", "fr_host.h", "fr_dev.cuh", "lookup_geom.h", "lookup_prework.cuh", "batch_check.cuh", "grand_product.cuh", "lookup_product.cuh", "permutation.h", "permutation_product.cuh", "export.cuh", os.path.join("..", "..", "include", "h2sha_b200.h")]
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-shared", "-Xcompiler", "-fPIC", "-cudart", "shared", "-ldl"]
 MARKER = b"H2SHA_BUILD_ID="
 

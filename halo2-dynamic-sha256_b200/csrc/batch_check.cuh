@@ -116,16 +116,17 @@ int ensure_check_tables(h2sha_engine* e) {
   std::vector<uint32_t> pairs;
   auto tag = [&](uint32_t kind, uint32_t idx) { return kind == CP_GATE ? gate_pos(idx) : ((3u << 30) | idx); };
   for (const CopyPair& cp : S->copies) { pairs.push_back(tag(cp.a_kind, cp.a_idx)); pairs.push_back(tag(cp.b_kind, cp.b_idx)); }
-  for (uint32_t k = 0; k < S->lookup_cells.size(); k++) {   // range.finalize: push order, wrapping at max_rows
-    const uint32_t col = k / P.cfg.max_rows, row = k - col * P.cfg.max_rows;
-    pairs.push_back((1u << 30) | (col * P.lookup_col_rows + row));
+  const LookupGeom G = lookup_geom(P);
+  for (uint32_t k = 0; k < S->lookup_cells.size(); k++) {   // range.finalize
+    const LookupCell c = G.range_cell(k);
+    pairs.push_back((1u << 30) | (c.col * P.lookup_col_rows + c.row));
     pairs.push_back(gate_pos(S->lookup_cells[k]));
   }
-  for (uint32_t n = 0; n < S->limb_gate_dense.size(); n++) {   // limb n -> column n % cols, row n / cols (spread.rs:202,228-231)
-    const uint32_t col = n % P.cfg.spread_cols, row = n / P.cfg.spread_cols;
-    pairs.push_back((2u << 30) | (col * P.spread_rows + row));
+  for (uint32_t n = 0; n < S->limb_gate_dense.size(); n++) {   // the dense and the spread cell of limb n
+    const LookupCell c = G.spread_cell(n);
+    pairs.push_back((2u << 30) | (c.col * P.spread_rows + c.row));
     pairs.push_back(gate_pos(S->limb_gate_dense[n]));
-    pairs.push_back((2u << 30) | ((P.cfg.spread_cols + col) * P.spread_rows + row));
+    pairs.push_back((2u << 30) | ((G.spread_cols + c.col) * P.spread_rows + c.row));
     pairs.push_back(gate_pos(S->limb_gate_spread[n]));
   }
   std::vector<uint64_t> fixed(S->fixed_consts.size() * 4 + 4, 0);
@@ -174,7 +175,7 @@ int h2sha_check_batch(h2sha_engine_t* e, uint64_t n_instances, const void* gate,
   CUDA_TRY(cudaMemsetAsync(e->d_chk_viol, 0, 5 * 8, st));
   // lookups: the multiplicity kernels without bins (cells outside their table are counted)
   uint32_t* bad32 = reinterpret_cast<uint32_t*>(e->d_chk_viol + 2);   // [2] range (low word), [3] spread (low word)
-  const LookupGeom G = lookup_geom(e, n_instances, 0);
+  const LookupGeom G = lookup_geom(P);
   for (uint64_t i0 = 0; i0 < n_instances; i0 += 65535) {
     const unsigned ni = (unsigned)std::min<uint64_t>(65535, n_instances - i0);
     A.gate = (const uint64_t*)gate + i0 * A.gate_inst_cells * 4;

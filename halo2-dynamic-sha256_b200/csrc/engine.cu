@@ -29,6 +29,7 @@
 
 #include "../../include/h2sha_b200.h"
 #include "h2sha_defs.h"
+#include "lookup_geom.h"
 #include "permutation.h"
 #include "planner.h"
 
@@ -926,43 +927,43 @@ struct MultArgs {
   const uint8_t* dense_raw;
   uint32_t* mult;
   uint32_t* bad;
-  uint64_t mult_words;
-  uint32_t n_lookup, n_limb, max_rows, n_lookup_cols, spread_cols, lookup_bits, limb_bits, usable_rows;
+  LookupGeom G;
 };
 enum { MULT_SMALL_BINS = 4096 };   // looked-up values below this (bytes, zeros: the hot bins) are binned in shared memory
 __global__ void __launch_bounds__(512) k_mult_from_raw(const MultArgs A) {
   extern __shared__ uint32_t s_bins[];   // [MULT_SMALL_BINS] range bins of lookup column 0 | [spread_cols << limb_bits] spread bins
+  const LookupGeom& G = A.G;
   const uint64_t inst = blockIdx.x;
-  uint32_t* bins = A.mult + inst * A.mult_words;
-  const uint32_t n_small = min((uint32_t)MULT_SMALL_BINS, 1u << A.lookup_bits), n_sp = A.spread_cols << A.limb_bits;
+  const uint64_t mult_words = G.mult_words();
+  uint32_t* bins = A.mult + inst * mult_words;
+  const uint32_t n_small = min((uint32_t)MULT_SMALL_BINS, 1u << G.lookup_bits), n_sp = G.spread_cols << G.limb_bits;
   uint32_t* s_sp = s_bins + MULT_SMALL_BINS;
   for (uint32_t i = threadIdx.x; i < MULT_SMALL_BINS + n_sp; i += blockDim.x) s_bins[i] = 0;
   __syncthreads();
   // pass A: the hot bins in shared memory (same-address atomics on the zeros and small bytes would serialise in L2)
   uint32_t n_bad = 0;
-  const uint32_t* lr = A.lookup_raw + inst * A.n_lookup;
-  const uint32_t n0 = min(A.n_lookup, A.max_rows);   // cells of lookup column 0 (range.finalize wraps at max_rows)
+  const uint32_t* lr = A.lookup_raw + inst * G.n_lookup;
+  const uint32_t n0 = G.range_used(0);   // cells of lookup column 0
   for (uint32_t k = threadIdx.x; k < n0; k += blockDim.x) {
     const uint32_t v = lr[k];
     if (v < n_small) atomicAdd(&s_bins[v], 1u);
   }
-  const uint8_t* dr = A.dense_raw + inst * A.n_limb;
-  for (uint32_t n = threadIdx.x; n < A.n_limb; n += blockDim.x) atomicAdd(&s_sp[((n % A.spread_cols) << A.limb_bits) + dr[n]], 1u);
-  if (threadIdx.x < A.n_lookup_cols + A.spread_cols) {   // never-assigned rows of every lookup input column hold 0 = table row 0
+  const uint8_t* dr = A.dense_raw + inst * G.n_limb;
+  for (uint32_t n = threadIdx.x; n < G.n_limb; n += blockDim.x) atomicAdd(&s_sp[(G.spread_cell(n).col << G.limb_bits) + dr[n]], 1u);
+  if (threadIdx.x < G.n_lookup_cols + G.spread_cols) {   // never-assigned rows of every lookup input column hold 0 = table row 0
     const uint32_t c = threadIdx.x;
-    if (c == 0) { if (A.usable_rows > n0) atomicAdd(&s_bins[0], A.usable_rows - n0); }
-    else if (c >= A.n_lookup_cols) {
-      const uint32_t cc = c - A.n_lookup_cols;
-      const uint32_t used = A.n_limb > cc ? (A.n_limb - cc + A.spread_cols - 1) / A.spread_cols : 0u;
-      if (A.usable_rows > used) atomicAdd(&s_sp[cc << A.limb_bits], A.usable_rows - used);
+    if (c == 0) { if (G.usable_rows > n0) atomicAdd(&s_bins[0], G.usable_rows - n0); }
+    else if (c >= G.n_lookup_cols) {
+      const uint32_t cc = c - G.n_lookup_cols, used = G.spread_used(cc);
+      if (G.usable_rows > used) atomicAdd(&s_sp[cc << G.limb_bits], G.usable_rows - used);
     }
   }
   __syncthreads();
   // pass B: every bin of the instance written once, coalesced: the shared-memory counts where they exist, zero elsewhere
   {
     uint4* b4 = reinterpret_cast<uint4*>(bins);   // mult_words is a multiple of 4 and the buffer 16-byte aligned: checked on the host
-    const uint64_t sp0 = (uint64_t)A.n_lookup_cols << A.lookup_bits;
-    for (uint64_t i = threadIdx.x; i < A.mult_words / 4; i += blockDim.x) {
+    const uint64_t sp0 = G.range_words();
+    for (uint64_t i = threadIdx.x; i < mult_words / 4; i += blockDim.x) {
       uint4 v = make_uint4(0, 0, 0, 0);
       const uint64_t w = i * 4;
       if (w < n_small) v = *reinterpret_cast<const uint4*>(s_bins + w);
@@ -972,16 +973,15 @@ __global__ void __launch_bounds__(512) k_mult_from_raw(const MultArgs A) {
   }
   __syncthreads();
   // pass C: the (spread-out) large values and the further lookup columns, with global atomics on bins that are now L2-resident
-  for (uint32_t k = threadIdx.x; k < A.n_lookup; k += blockDim.x) {
-    const uint32_t v = lr[k], col = k / A.max_rows;
-    if ((v >> A.lookup_bits) != 0) { n_bad++; continue; }
+  for (uint32_t k = threadIdx.x; k < G.n_lookup; k += blockDim.x) {
+    const uint32_t v = lr[k], col = G.range_cell(k).col;
+    if ((v >> G.lookup_bits) != 0) { n_bad++; continue; }
     if (col == 0 && v < n_small) continue;
-    atomicAdd(&bins[((uint64_t)col << A.lookup_bits) + v], 1u);
+    atomicAdd(&bins[((uint64_t)col << G.lookup_bits) + v], 1u);
   }
-  if (threadIdx.x >= 1 && threadIdx.x < A.n_lookup_cols) {
-    const uint32_t c = threadIdx.x, first = c * A.max_rows;
-    const uint32_t used = A.n_lookup > first ? min(A.max_rows, A.n_lookup - first) : 0u;
-    if (A.usable_rows > used) atomicAdd(&bins[(uint64_t)c << A.lookup_bits], A.usable_rows - used);
+  if (threadIdx.x >= 1 && threadIdx.x < G.n_lookup_cols) {
+    const uint32_t c = threadIdx.x, used = G.range_used(c);
+    if (G.usable_rows > used) atomicAdd(&bins[(uint64_t)c << G.lookup_bits], G.usable_rows - used);
   }
   if (n_bad && A.bad) atomicAdd(A.bad, n_bad);
 }
@@ -1203,8 +1203,6 @@ int ensure_slot(h2sha_engine* e, HostSlot* H, uint64_t bytes) {
   return H2SHA_OK;
 }
 
-uint32_t lookup_rows_needed(const Plan& P);   // lookup_prework.cuh
-
 struct EngineGuard {   // error paths of h2sha_create: releases whatever has been allocated so far
   h2sha_engine* e;
   ~EngineGuard() { if (e) h2sha_destroy(e); }
@@ -1373,8 +1371,8 @@ int h2sha_create(const h2sha_config_t* cfg, h2sha_engine_t** out) {
   D.n_lookup_cols = P.n_lookup_cols; D.lookup_col_rows = P.lookup_col_rows; D.spread_rows = P.spread_rows;
   D.blocks_per_inst = bp; D.dtrace_words_per_inst = dw;
   D.gate_inst_cells = (uint64_t)P.n_gate_cols * P.gate_col_rows;
-  D.lookup_inst_cells = (uint64_t)P.n_lookup_cols * P.lookup_col_rows;
-  D.spread_inst_cells = (uint64_t)2 * pc.spread_cols * P.spread_rows;
+  D.lookup_inst_cells = lookup_geom(P).lookup_inst_cells;
+  D.spread_inst_cells = lookup_geom(P).spread_inst_cells;
   CUDA_TRY(cudaMalloc(&e->d_blob, blob.size()));
   CUDA_TRY(cudaMemcpy(e->d_blob, blob.data(), blob.size(), cudaMemcpyHostToDevice));
   D.blob = e->d_blob;
@@ -1545,7 +1543,7 @@ int h2sha_digest_batch(h2sha_engine_t* e, const h2sha_batch_t* b) {
     if (P.cfg.limb_bits > 8) return set_err(H2SHA_EINVAL, "the fused multiplicity count keeps the spread-table bins in shared memory: num_bits_lookup <= 8");
   }
   if (b->lookup_mult_dev) {
-    if (b->mult_usable_rows < lookup_rows_needed(P)) return set_err(H2SHA_EINVAL, "mult_usable_rows is smaller than an assigned column or a lookup table");
+    if (b->mult_usable_rows < lookup_geom(P).min_usable_rows()) return set_err(H2SHA_EINVAL, "mult_usable_rows is smaller than an assigned column or a lookup table");
     if (P.cfg.lookup_bits < 2 || P.cfg.limb_bits < 2 || ((uintptr_t)b->lookup_mult_dev & 15u)) return set_err(H2SHA_EINVAL, "lookup_mult_dev must be 16-byte aligned (tables of >= 4 rows)");
   }
   CUDA_TRY(cudaSetDevice(e->device));
@@ -1674,9 +1672,7 @@ int h2sha_digest_batch(h2sha_engine_t* e, const h2sha_batch_t* b) {
     if (b->lookup_mult_dev) {
       MultArgs ma{};
       ma.lookup_raw = e->d_lookup_raw; ma.dense_raw = e->d_dense_raw; ma.mult = b->lookup_mult_dev; ma.bad = b->mult_not_in_table_dev;
-      ma.mult_words = ((uint64_t)P.n_lookup_cols << P.cfg.lookup_bits) + ((uint64_t)P.cfg.spread_cols << P.cfg.limb_bits);
-      ma.n_lookup = P.n_lookup; ma.n_limb = P.n_limb; ma.max_rows = P.cfg.max_rows; ma.n_lookup_cols = P.n_lookup_cols; ma.spread_cols = P.cfg.spread_cols;
-      ma.lookup_bits = P.cfg.lookup_bits; ma.limb_bits = P.cfg.limb_bits; ma.usable_rows = b->mult_usable_rows;
+      ma.G = lookup_geom(P, b->mult_usable_rows);
       const size_t mult_smem = ((size_t)MULT_SMALL_BINS + ((size_t)P.cfg.spread_cols << P.cfg.limb_bits)) * 4;
       if (mult_smem > 48 * 1024) return set_err(H2SHA_EINVAL, "spread tables too large for the multiplicity kernel's shared memory");
       k_mult_from_raw<<<(unsigned)b->n_instances, 512, mult_smem, st>>>(ma);
@@ -1698,6 +1694,7 @@ int h2sha_export_instance(h2sha_engine_t* e, uint64_t instance, const void* gate
   if (!e || !host_columns) return set_err(H2SHA_EINVAL, "null argument");
   if (e->device < 0) return set_err(H2SHA_ECUDA, "plan-only engine");
   const Plan& P = e->plan;
+  const LookupGeom G = lookup_geom(P);
   const uint32_t col_rows[3] = {P.gate_col_rows, P.lookup_col_rows, P.spread_rows};
   const uint32_t n_cols[3] = {P.n_gate_cols, P.n_lookup_cols, 2 * P.cfg.spread_cols};
   const void* bufs[3] = {gate, lookup, spread};
@@ -1705,7 +1702,7 @@ int h2sha_export_instance(h2sha_engine_t* e, uint64_t instance, const void* gate
   for (int b = 0; b < 3; b++)
     if (col_rows[b] > rows_per_column && bufs[b]) {
       // only the assigned prefix of a column has to fit: the stride may exceed rows_per_column through alignment padding
-      uint32_t used = (b == 0) ? 0 : (b == 1 ? std::min(P.n_lookup, P.cfg.max_rows) : (P.n_limb + P.cfg.spread_cols - 1) / P.cfg.spread_cols);
+      uint32_t used = (b == 0) ? 0 : (b == 1 ? G.max_range_used() : G.max_spread_used());
       if (b == 0)
         for (size_t c = 0; c < P.breaks.size(); c++) used = std::max(used, ((c + 1 < P.breaks.size()) ? P.breaks[c + 1] : P.n_gate) - P.breaks[c]);
       if (used > rows_per_column) return set_err(H2SHA_EINVAL, "rows_per_column is smaller than the assigned rows of a column");

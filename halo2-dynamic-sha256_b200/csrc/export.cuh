@@ -57,8 +57,9 @@ HostGeom host_geom(const Plan& P, uint32_t rows_per_column) {
 void used_rows(const Plan& P, uint32_t used[3]) {
   used[0] = 0;
   for (size_t c = 0; c < P.breaks.size(); c++) used[0] = std::max(used[0], ((c + 1 < P.breaks.size()) ? P.breaks[c + 1] : P.n_gate) - P.breaks[c]);
-  used[1] = std::min(P.n_lookup, P.cfg.max_rows);
-  used[2] = (P.n_limb + P.cfg.spread_cols - 1) / P.cfg.spread_cols;
+  const LookupGeom G = lookup_geom(P);
+  used[1] = G.max_range_used();
+  used[2] = G.max_spread_used();
 }
 
 }  // namespace
@@ -128,6 +129,7 @@ int h2sha_expand_compact(h2sha_engine_t* e, const void* dict_host, uint64_t n_in
   if (rc) return rc;
   const Plan& P = e->plan;
   const Plan& C = e->compact->plan;
+  const LookupGeom L = lookup_geom(P);
   uint32_t used[3];
   used_rows(P, used);
   if (std::max(used[0], std::max(used[1], used[2])) > rows_per_column) return set_err(H2SHA_EINVAL, "rows_per_column is smaller than the assigned rows of a column");
@@ -168,21 +170,21 @@ int h2sha_expand_compact(h2sha_engine_t* e, const void* dict_host, uint64_t n_in
       } else if (seg == G.n_gate_cols) {
         for (uint32_t c = 0; c < G.n_lookup_cols; c++) {
           uint64_t* col = out + (uint64_t)(G.n_gate_cols + c) * G.rows * 4;
-          const uint32_t lo = std::min(P.n_lookup, c * P.cfg.max_rows), hi = std::min(P.n_lookup, (c + 1) * P.cfg.max_rows);
+          const uint32_t lo = L.range_first(c), hi = lo + L.range_used(c);
           for (uint32_t k = lo; k < hi; k++) put(col + (uint64_t)(k - lo) * 4, dict, C.map_lookup[k]);
           if (zero_fill) memset(col + (uint64_t)(hi - lo) * 4, 0, (size_t)(G.rows - (hi - lo)) * 32);
         }
       } else {
-        const uint32_t nc = P.cfg.spread_cols;
+        const uint32_t nc = L.spread_cols;
         uint64_t* base = out + (uint64_t)(G.n_gate_cols + G.n_lookup_cols) * G.rows * 4;
         for (uint32_t n = 0; n < P.n_limb; n++) {
-          const uint32_t c = n % nc, row = n / nc;
-          put(base + ((uint64_t)c * G.rows + row) * 4, dict, C.map_dense[n]);
-          put(base + ((uint64_t)(nc + c) * G.rows + row) * 4, dict, C.map_spread[n]);
+          const LookupCell c = L.spread_cell(n);
+          put(base + ((uint64_t)c.col * G.rows + c.row) * 4, dict, C.map_dense[n]);
+          put(base + ((uint64_t)(nc + c.col) * G.rows + c.row) * 4, dict, C.map_spread[n]);
         }
         if (zero_fill)
           for (uint32_t c = 0; c < 2 * nc; c++) {
-            const uint32_t cc = c % nc, rows_used = P.n_limb > cc ? (P.n_limb - cc + nc - 1) / nc : 0;
+            const uint32_t rows_used = L.spread_used(c % nc);
             memset(base + ((uint64_t)c * G.rows + rows_used) * 4, 0, (size_t)(G.rows - rows_used) * 32);
           }
       }

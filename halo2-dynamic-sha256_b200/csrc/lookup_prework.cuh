@@ -12,21 +12,15 @@
 //   k_permute_scan                 per (instance, lookup): exclusive scans over the table rows in sorted order,
 //   k_permute_fill                 one thread per row: two-level search in the scans, 2 x 256-bit stores.
 // HBM-bound like the rest of the path: the fill writes 64 B per usable row and reads only the (L2-resident) scans.
-// oracle/lookup_prework.py is the CPU restatement the tests compare against.
+// oracle/lookup_prework.py is the CPU restatement the tests compare against.  Where the input cells sit, the layout of the
+// multiplicity buffer and the meaning of lookup_idx: LookupGeom and select_lookup (lookup_geom.h).
 #pragma once
 
 #include <cub/device/device_segmented_sort.cuh>
 
-namespace {
+#include "lookup_geom.h"
 
-struct LookupGeom {
-  uint64_t n_inst;
-  uint64_t lookup_inst_cells, spread_inst_cells;   // Fr per instance in the lookup / spread buffers
-  uint32_t n_lookup, max_rows, n_lookup_cols, lookup_col_rows, lookup_bits;
-  uint32_t n_limb, spread_cols, spread_rows, limb_bits;
-  uint32_t usable_rows;
-  uint64_t mult_words;   // u32 words per instance in the multiplicity buffer
-};
+namespace {
 
 // range lookup: one thread per assigned cell of the lookup advice column(s).  grid = (tiles, instances).  mult == null: only count
 // the cells that are not in the table (batch_check.cuh).
@@ -34,26 +28,24 @@ __global__ void __launch_bounds__(256) k_range_mult(const LookupGeom G, const ui
                                                    uint32_t* __restrict__ bad) {
   const uint64_t inst = blockIdx.y;
   const uint64_t* base = lookup + inst * G.lookup_inst_cells * 4;
-  uint32_t* m_inst = mult + inst * G.mult_words;
+  uint32_t* m_inst = mult + inst * G.mult_words();
   const uint32_t n_vals = 1u << G.lookup_bits;
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < G.n_lookup; i += gridDim.x * blockDim.x) {
-    const uint32_t col = i / G.max_rows, row = i - col * G.max_rows;   // range.finalize wraps at max_rows
+    const LookupCell c = G.range_cell(i);
     uint64_t x[4], v[4];
-    load_cell(base + ((uint64_t)col * G.lookup_col_rows + row) * 4, x);
+    load_cell(base + ((uint64_t)c.col * G.lookup_col_rows + c.row) * 4, x);
     mont_reduce(x, v);
-    if ((v[1] | v[2] | v[3]) == 0 && v[0] < n_vals) { if (mult) atomicAdd(&m_inst[(uint64_t)col * n_vals + (uint32_t)v[0]], 1u); }
+    if ((v[1] | v[2] | v[3]) == 0 && v[0] < n_vals) { if (mult) atomicAdd(&m_inst[(uint64_t)c.col * n_vals + (uint32_t)v[0]], 1u); }
     else if (bad) atomicAdd(bad, 1u);
   }
   // never-assigned rows of a column hold 0
   if (mult && blockIdx.x == 0 && threadIdx.x < G.n_lookup_cols) {
-    const uint32_t col = threadIdx.x;
-    const uint32_t first = col * G.max_rows;
-    const uint32_t used = (G.n_lookup > first) ? min(G.max_rows, G.n_lookup - first) : 0u;
+    const uint32_t col = threadIdx.x, used = G.range_used(col);
     if (G.usable_rows > used) atomicAdd(&m_inst[(uint64_t)col * n_vals], G.usable_rows - used);
   }
 }
 
-// spread lookups: limb n sits in column pair n % cols, row n / cols (spread.rs:202,228-231).  Block-local histograms in
+// spread lookups, one histogram per column pair.  Block-local histograms in
 // shared memory, flushed with one global atomic per non-empty bin.  grid = (tiles, instances); dynamic smem = cols * 2^bits * 4.
 __global__ void __launch_bounds__(256) k_spread_mult(const LookupGeom G, const uint64_t* __restrict__ spread, uint32_t* __restrict__ mult,
                                                     uint32_t* __restrict__ bad) {
@@ -65,19 +57,19 @@ __global__ void __launch_bounds__(256) k_spread_mult(const LookupGeom G, const u
   }
   const uint64_t inst = blockIdx.y;
   const uint64_t* base = spread + inst * G.spread_inst_cells * 4;
-  uint32_t* m_inst = mult + inst * G.mult_words + (uint64_t)G.n_lookup_cols * (1u << G.lookup_bits);
+  uint32_t* m_inst = mult + inst * G.mult_words() + G.range_words();
   uint32_t n_bad = 0;
   for (uint32_t n = blockIdx.x * blockDim.x + threadIdx.x; n < G.n_limb; n += gridDim.x * blockDim.x) {
-    const uint32_t row = n / G.spread_cols, col = n - row * G.spread_cols;
+    const LookupCell c = G.spread_cell(n);
     uint64_t x[4], d[4], s[4];
-    load_cell(base + ((uint64_t)col * G.spread_rows + row) * 4, x);
+    load_cell(base + ((uint64_t)c.col * G.spread_rows + c.row) * 4, x);
     mont_reduce(x, d);
-    load_cell(base + ((uint64_t)(G.spread_cols + col) * G.spread_rows + row) * 4, x);
+    load_cell(base + ((uint64_t)(G.spread_cols + c.col) * G.spread_rows + c.row) * 4, x);
     mont_reduce(x, s);
     bool ok = (d[1] | d[2] | d[3]) == 0 && d[0] < n_vals && (s[1] | s[2] | s[3]) == 0;
     if (ok) ok = spread32(d[0]) == s[0];   // the pair has to be a table row, not just the dense half
     if (!ok) n_bad++;
-    else if (mult) atomicAdd(&s_hist[col * n_vals + (uint32_t)d[0]], 1u);
+    else if (mult) atomicAdd(&s_hist[c.col * n_vals + (uint32_t)d[0]], 1u);
   }
   if (n_bad && bad) atomicAdd(bad, n_bad);
   __syncthreads();
@@ -85,8 +77,7 @@ __global__ void __launch_bounds__(256) k_spread_mult(const LookupGeom G, const u
   for (uint32_t i = threadIdx.x; i < n_bins; i += blockDim.x)
     if (s_hist[i]) atomicAdd(&m_inst[i], s_hist[i]);
   if (blockIdx.x == 0 && threadIdx.x < G.spread_cols) {
-    const uint32_t col = threadIdx.x;
-    const uint32_t used = (G.n_limb > col) ? (G.n_limb - col + G.spread_cols - 1) / G.spread_cols : 0u;
+    const uint32_t col = threadIdx.x, used = G.spread_used(col);
     if (G.usable_rows > used) atomicAdd(&m_inst[col * n_vals], G.usable_rows - used);
   }
 }
@@ -234,32 +225,33 @@ struct MultOneArgs {
   uint32_t* out;                // [gridDim.x][n_vals]
   uint32_t* bad;                // may be null
   uint64_t first;
-  uint32_t n_lookup, n_limb, max_rows, spread_cols, n_vals, usable_rows, is_range, col;
+  uint32_t n_vals, is_range, col;
+  LookupGeom G;
 };
-enum { MULT_ONE_SMALL = 4096 };
 __global__ void __launch_bounds__(512) k_mult_one(const MultOneArgs A) {
-  __shared__ uint32_t s_small[MULT_ONE_SMALL];
+  __shared__ uint32_t s_small[MULT_SMALL_BINS];
+  const LookupGeom& G = A.G;
   const uint64_t inst = A.first + blockIdx.x;
   uint32_t* bins = A.out + (uint64_t)blockIdx.x * A.n_vals;
-  const uint32_t n_small = min((uint32_t)MULT_ONE_SMALL, A.n_vals);
+  const uint32_t n_small = min((uint32_t)MULT_SMALL_BINS, A.n_vals);
   for (uint32_t i = threadIdx.x; i < n_small; i += blockDim.x) s_small[i] = 0;
   __syncthreads();
   uint32_t n_bad = 0, used = 0;
-  const uint32_t* lr = A.lookup_raw + inst * A.n_lookup;
-  const uint8_t* dr = A.dense_raw + inst * A.n_limb;
+  const uint32_t* lr = A.lookup_raw + inst * G.n_lookup;
+  const uint8_t* dr = A.dense_raw + inst * G.n_limb;
   uint32_t k0 = 0, k1 = 0;
   if (A.is_range) {
-    k0 = min(A.n_lookup, A.col * A.max_rows); k1 = min(A.n_lookup, (A.col + 1) * A.max_rows);   // range.finalize wraps at max_rows
-    used = k1 - k0;
+    used = G.range_used(A.col);
+    k0 = G.range_first(A.col); k1 = k0 + used;
     for (uint32_t k = k0 + threadIdx.x; k < k1; k += blockDim.x) {
       const uint32_t v = lr[k];
       if (v < n_small) atomicAdd(&s_small[v], 1u);
     }
   } else {
-    used = A.n_limb > A.col ? (A.n_limb - A.col + A.spread_cols - 1) / A.spread_cols : 0u;
-    for (uint32_t n = A.col + threadIdx.x * A.spread_cols; n < A.n_limb; n += blockDim.x * A.spread_cols) atomicAdd(&s_small[dr[n]], 1u);   // dense limbs are < 2^8 <= n_small
+    used = G.spread_used(A.col);
+    for (uint32_t n = A.col + threadIdx.x * G.spread_cols; n < G.n_limb; n += blockDim.x * G.spread_cols) atomicAdd(&s_small[dr[n]], 1u);   // dense limbs are < 2^8 <= n_small
   }
-  if (threadIdx.x == 0 && A.usable_rows > used) atomicAdd(&s_small[0], A.usable_rows - used);   // never-assigned rows hold 0 = table row 0
+  if (threadIdx.x == 0 && G.usable_rows > used) atomicAdd(&s_small[0], G.usable_rows - used);   // never-assigned rows hold 0 = table row 0
   __syncthreads();
   for (uint32_t i = threadIdx.x; i < A.n_vals; i += blockDim.x) bins[i] = i < n_small ? s_small[i] : 0u;
   __syncthreads();
@@ -501,26 +493,6 @@ int stage_challenges(h2sha_engine* e, uint64_t n, const uint64_t* theta, const u
   return H2SHA_OK;
 }
 
-LookupGeom lookup_geom(const h2sha_engine* e, uint64_t n_inst, uint32_t usable_rows) {
-  const Plan& P = e->plan;
-  LookupGeom G{};
-  G.n_inst = n_inst;
-  G.lookup_inst_cells = e->dplan.lookup_inst_cells; G.spread_inst_cells = e->dplan.spread_inst_cells;
-  G.n_lookup = P.n_lookup; G.max_rows = P.cfg.max_rows; G.n_lookup_cols = P.n_lookup_cols; G.lookup_col_rows = P.lookup_col_rows;
-  G.lookup_bits = P.cfg.lookup_bits;
-  G.n_limb = P.n_limb; G.spread_cols = P.cfg.spread_cols; G.spread_rows = P.spread_rows; G.limb_bits = P.cfg.limb_bits;
-  G.usable_rows = usable_rows;
-  G.mult_words = (uint64_t)P.n_lookup_cols * (1u << P.cfg.lookup_bits) + (uint64_t)P.cfg.spread_cols * (1u << P.cfg.limb_bits);
-  return G;
-}
-
-// rows of the largest advice column the two lookups read
-uint32_t lookup_rows_needed(const Plan& P) {
-  const uint32_t lk = std::min(P.n_lookup, P.cfg.max_rows);
-  const uint32_t sp = (P.n_limb + P.cfg.spread_cols - 1) / P.cfg.spread_cols;
-  return std::max(std::max(lk, sp), std::max(1u << P.cfg.lookup_bits, 1u << P.cfg.limb_bits));
-}
-
 bool u256_less(const U256& a, const U256& b) {
   for (int i = 3; i >= 0; i--)
     if (a.l[i] != b.l[i]) return a.l[i] < b.l[i];
@@ -557,13 +529,13 @@ extern "C" {
 
 int h2sha_get_lookup_info(const h2sha_engine_t* e, h2sha_lookup_info_t* out) {
   if (!e || !out) return set_err(H2SHA_EINVAL, "null argument");
-  const Plan& P = e->plan;
-  out->n_range_lookups = P.n_lookup_cols;
-  out->n_spread_lookups = P.cfg.spread_cols;
-  out->range_table_rows = 1u << P.cfg.lookup_bits;
-  out->spread_table_rows = 1u << P.cfg.limb_bits;
-  out->min_usable_rows = lookup_rows_needed(P);
-  out->mult_words_per_instance = (uint64_t)P.n_lookup_cols * (1u << P.cfg.lookup_bits) + (uint64_t)P.cfg.spread_cols * (1u << P.cfg.limb_bits);
+  const LookupGeom G = lookup_geom(e->plan);
+  out->n_range_lookups = G.n_lookup_cols;
+  out->n_spread_lookups = G.spread_cols;
+  out->range_table_rows = 1u << G.lookup_bits;
+  out->spread_table_rows = 1u << G.limb_bits;
+  out->min_usable_rows = G.min_usable_rows();
+  out->mult_words_per_instance = G.mult_words();
   return H2SHA_OK;
 }
 
@@ -572,24 +544,24 @@ int h2sha_lookup_multiplicities(h2sha_engine_t* e, uint64_t n_instances, const v
   if (!e || !mult_dev) return set_err(H2SHA_EINVAL, "null argument");
   if (e->device < 0) return set_err(H2SHA_ECUDA, "plan-only engine (device = -1): there is no CPU path");
   if (!lookup && !spread) return set_err(H2SHA_EINVAL, "neither the lookup nor the spread buffer was given");
-  if (usable_rows < lookup_rows_needed(e->plan)) return set_err(H2SHA_EINVAL, "usable_rows is smaller than an assigned column or a lookup table");
+  const LookupGeom G = lookup_geom(e->plan, usable_rows);
+  if (usable_rows < G.min_usable_rows()) return set_err(H2SHA_EINVAL, "usable_rows is smaller than an assigned column or a lookup table");
   if (n_instances == 0) return H2SHA_OK;
   CUDA_TRY(cudaSetDevice(e->device));
   cudaStream_t st = (cudaStream_t)stream;
-  const LookupGeom G = lookup_geom(e, n_instances, usable_rows);
-  const uint64_t range_words = (uint64_t)G.n_lookup_cols << G.lookup_bits;
+  const uint64_t mult_words = G.mult_words(), range_words = G.range_words();
   // only the halves whose buffer was given are (re)computed
   if (lookup && spread) {
-    CUDA_TRY(cudaMemsetAsync(mult_dev, 0, n_instances * G.mult_words * 4, st));
+    CUDA_TRY(cudaMemsetAsync(mult_dev, 0, n_instances * mult_words * 4, st));
   } else {
-    const uint64_t off = lookup ? 0 : range_words, cnt = lookup ? range_words : G.mult_words - range_words;
-    CUDA_TRY(cudaMemset2DAsync(mult_dev + off, G.mult_words * 4, 0, cnt * 4, n_instances, st));
+    const uint64_t off = lookup ? 0 : range_words, cnt = lookup ? range_words : mult_words - range_words;
+    CUDA_TRY(cudaMemset2DAsync(mult_dev + off, mult_words * 4, 0, cnt * 4, n_instances, st));
   }
   if (not_in_table_dev) CUDA_TRY(cudaMemsetAsync(not_in_table_dev, 0, 4, st));
   // grid.y = instance: at most 65535 per launch
   for (uint64_t i0 = 0; i0 < n_instances; i0 += 65535) {
     const unsigned ni = (unsigned)std::min<uint64_t>(65535, n_instances - i0);
-    uint32_t* m0 = mult_dev + i0 * G.mult_words;
+    uint32_t* m0 = mult_dev + i0 * mult_words;
     if (lookup) {
       const unsigned tiles = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((G.n_lookup + 255) / 256, 64));
       k_range_mult<<<dim3(tiles, ni), 256, 0, st>>>(G, (const uint64_t*)lookup + i0 * G.lookup_inst_cells * 4, m0, not_in_table_dev);
@@ -617,17 +589,16 @@ int permute_lookup_impl(h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup
   if (!e || !permuted_input_dev || !permuted_table_dev) return set_err(H2SHA_EINVAL, "null argument");
   const bool from_raw = mult_dev == nullptr;
   if (e->device < 0) return set_err(H2SHA_ECUDA, "plan-only engine (device = -1): there is no CPU path");
-  const Plan& P = e->plan;
-  const uint32_t n_range = P.n_lookup_cols, n_spread = P.cfg.spread_cols;
-  if (lookup_idx >= n_range + n_spread) return set_err(H2SHA_EINVAL, "bad lookup index");
-  const bool is_range = lookup_idx < n_range;
+  const LookupGeom G = lookup_geom(e->plan, usable_rows);
+  const LookupSel L = select_lookup(G, lookup_idx);
+  if (!L.valid) return set_err(H2SHA_EINVAL, "bad lookup index");
+  const bool is_range = L.is_range;
   if (!is_range && !theta_mont) return set_err(H2SHA_EINVAL, "a spread lookup has two expressions: theta is needed to compress them");
-  if (usable_rows < lookup_rows_needed(P)) return set_err(H2SHA_EINVAL, "usable_rows is smaller than an assigned column or a lookup table");
+  if (usable_rows < G.min_usable_rows()) return set_err(H2SHA_EINVAL, "usable_rows is smaller than an assigned column or a lookup table");
   if (n_instances == 0) return H2SHA_OK;
   CUDA_TRY(cudaSetDevice(e->device));
   cudaStream_t st = (cudaStream_t)stream;
-  const LookupGeom G = lookup_geom(e, n_instances, usable_rows);
-  const uint32_t n_vals = is_range ? (1u << G.lookup_bits) : (1u << G.limb_bits);
+  const uint32_t n_vals = L.n_vals;
   // workspace: scans + totals of one chunk of instances (the chunks run one after the other on `stream` and share it)
   if (n_vals > (1u << 22)) return set_err(H2SHA_EINVAL, "lookup table too large for the permutation workspace (lookup_bits > 22)");
   // instances per pass: at most `lkchunk` (default 256) and at most ~1 GB of scans (and per-instance spread tables)
@@ -673,8 +644,8 @@ int permute_lookup_impl(h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup
     A.mult_stride = align_up(n_vals, 4);
     A.mult = raw_bins;
   } else {
-    A.mult_stride = G.mult_words;
-    A.mult = mult_dev + (is_range ? (uint64_t)lookup_idx * n_vals : ((uint64_t)n_range << G.lookup_bits) + (uint64_t)(lookup_idx - n_range) * n_vals);
+    A.mult_stride = G.mult_words();
+    A.mult = mult_dev + L.mult_off;
   }
   A.n_vals = n_vals; A.usable_rows = usable_rows;
   A.scan = ws; A.totals = ws + chunk * 3ull * n_vals;
@@ -715,8 +686,7 @@ int permute_lookup_impl(h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup
     if (from_raw) {
       MultOneArgs M{};
       M.lookup_raw = e->d_lookup_raw; M.dense_raw = e->d_dense_raw; M.out = raw_bins; M.bad = nullptr; M.first = first_raw + i0;
-      M.n_lookup = P.n_lookup; M.n_limb = P.n_limb; M.max_rows = P.cfg.max_rows; M.spread_cols = P.cfg.spread_cols; M.n_vals = n_vals;
-      M.usable_rows = usable_rows; M.is_range = is_range ? 1u : 0u; M.col = is_range ? lookup_idx : lookup_idx - n_range;
+      M.n_vals = n_vals; M.is_range = is_range ? 1u : 0u; M.col = L.col; M.G = G;
       if (A.mult_stride != n_vals) return set_err(H2SHA_EINVAL, "lookup tables of fewer than 4 rows are not supported by the raw-list path");
       k_mult_one<<<(unsigned)ni, 512, 0, st>>>(M);
       CUDA_TRY(cudaGetLastError());
@@ -765,10 +735,9 @@ int h2sha_permute_lookup_from_raw(h2sha_engine_t* e, uint64_t first_instance, ui
 // the checks of the per-instance calls that need no device: the plan-only engine is refused after them, by permute_lookup_impl
 static int check_permute_per_instance(const h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup_idx, const uint64_t* thetas_mont) {
   if (!e) return set_err(H2SHA_EINVAL, "null argument");
-  const bool is_range = lookup_idx < e->plan.n_lookup_cols;
-  if (!is_range && lookup_idx < e->plan.n_lookup_cols + e->plan.cfg.spread_cols && !thetas_mont)
-    return set_err(H2SHA_EINVAL, "a spread lookup has two expressions: thetas_mont is needed to compress them");
-  return !is_range && thetas_mont ? check_challenge_rows(thetas_mont, n_instances, "thetas_mont") : H2SHA_OK;
+  const LookupSel L = select_lookup(lookup_geom(e->plan), lookup_idx);
+  if (L.valid && !L.is_range && !thetas_mont) return set_err(H2SHA_EINVAL, "a spread lookup has two expressions: thetas_mont is needed to compress them");
+  return !L.is_range && thetas_mont ? check_challenge_rows(thetas_mont, n_instances, "thetas_mont") : H2SHA_OK;
 }
 
 int h2sha_permute_lookup_per_instance(h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup_idx, const uint32_t* mult_dev, uint32_t usable_rows,

@@ -1,6 +1,7 @@
 // lookup_product.cuh -- the lookup argument's grand-product column z on the device (SURVEY.md §8f #4), the step after
 // the permutation: PSE halo2_proofs plonk/lookup/prover.rs `Permuted::commit_product`, for one lookup of every instance.
-// Included at the end of engine.cu, after lookup_prework.cuh (LookupGeom, ensure_range_tab) and grand_product.cuh.
+// Included at the end of engine.cu, after lookup_prework.cuh (ensure_range_tab) and grand_product.cuh.  Which column a lookup
+// reads and how many of its rows are assigned: select_lookup (lookup_geom.h).
 //
 //   u_i = (A[i] + beta)(S[i] + gamma),  v_i = (A'[i] + beta)(S'[i] + gamma),  i < U = usable_rows
 //   z[0] = 1,  z[j+1] = z[j] * u_j / v_j                                      (U + 1 values)
@@ -76,24 +77,24 @@ int lookup_product_impl(h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup
                         const uint64_t* beta_mont, const uint64_t* gamma_mont, bool per_inst, void* z_dev, uint32_t* errors_dev, void* stream) {
   if (!e || !permuted_input_dev || !permuted_table_dev || !beta_mont || !gamma_mont || !z_dev) return set_err(H2SHA_EINVAL, "null argument");
   if (e->device < 0) return set_err(H2SHA_ECUDA, "plan-only engine (device = -1): there is no CPU path");
-  const Plan& P = e->plan;
-  const uint32_t n_range = P.n_lookup_cols, n_spread = P.cfg.spread_cols;
-  if (lookup_idx >= n_range + n_spread) return set_err(H2SHA_EINVAL, "bad lookup index");
-  const bool is_range = lookup_idx < n_range;
-  if (is_range ? !lookup : !spread) return set_err(H2SHA_EINVAL, "null argument: the witness buffer this lookup reads");
+  const LookupGeom G = lookup_geom(e->plan, usable_rows);
+  const LookupSel L = select_lookup(G, lookup_idx);
+  if (!L.valid) return set_err(H2SHA_EINVAL, "bad lookup index");
+  const bool is_range = L.is_range;
+  const void* cells = L.buffer(lookup, spread);
+  if (!cells) return set_err(H2SHA_EINVAL, "null argument: the witness buffer this lookup reads");
   if (!is_range && !theta_mont) return set_err(H2SHA_EINVAL, "a spread lookup has two expressions: theta is needed to compress them");
-  if (usable_rows < lookup_rows_needed(P)) return set_err(H2SHA_EINVAL, "usable_rows is smaller than an assigned column or a lookup table");
+  if (usable_rows < G.min_usable_rows()) return set_err(H2SHA_EINVAL, "usable_rows is smaller than an assigned column or a lookup table");
   if (!per_inst && (fr::geq_p(beta_mont) || fr::geq_p(gamma_mont) || (theta_mont && !is_range && fr::geq_p(theta_mont))))
     return set_err(H2SHA_EINVAL, "beta, gamma and theta must be reduced field elements");
-  const void* bufs[] = {is_range ? lookup : spread, permuted_input_dev, permuted_table_dev, z_dev};
+  const void* bufs[] = {cells, permuted_input_dev, permuted_table_dev, z_dev};
   for (const void* b : bufs)
     if ((uintptr_t)b & 31u) return set_err(H2SHA_EINVAL, "Fr buffers must be 32-byte aligned");
   if (n_instances == 0) return H2SHA_OK;
   CUDA_TRY(cudaSetDevice(e->device));
   int rc;
   cudaStream_t st = (cudaStream_t)stream;
-  const LookupGeom G = lookup_geom(e, n_instances, usable_rows);
-  const uint32_t n_vals = is_range ? (1u << G.lookup_bits) : (1u << G.limb_bits);
+  const uint32_t n_vals = L.n_vals;
   GrandProduct Z{};
   Z.rows = usable_rows; Z.n_chunks = 1; Z.z_stride = usable_rows + 1;
   Z.tiles_per_chunk = (uint32_t)((usable_rows + (uint64_t)GP_TILE - 1) / GP_TILE);
@@ -122,19 +123,9 @@ int lookup_product_impl(h2sha_engine_t* e, uint64_t n_instances, uint32_t lookup
   if (per_inst && (rc = stage_challenges(e, n_instances, is_range ? nullptr : theta_mont, beta_mont, gamma_mont, st))) return rc;
   auto run = [&](auto& A) {
     A.n_vals = n_vals; A.usable_rows = usable_rows; A.tab = tab;
-    if (is_range) {
-      const uint32_t first = lookup_idx * G.max_rows;
-      A.cells = (const uint64_t*)lookup; A.inst_cells = G.lookup_inst_cells;
-      A.col_off = (uint64_t)lookup_idx * G.lookup_col_rows;
-      A.used = G.n_lookup > first ? std::min(G.max_rows, G.n_lookup - first) : 0u;   // range.finalize wraps at max_rows
-    } else {
-      const uint32_t col = lookup_idx - n_range;
-      A.cells = (const uint64_t*)spread; A.inst_cells = G.spread_inst_cells;
-      A.col_off = (uint64_t)col * G.spread_rows; A.spread_off = (uint64_t)G.spread_cols * G.spread_rows;
-      A.used = G.n_limb > col ? (G.n_limb - col + G.spread_cols - 1) / G.spread_cols : 0u;   // limb n -> column n % cols, row n / cols
-      A.is_spread = 1;
-    }
-    const uint64_t* cells0 = A.cells;
+    A.inst_cells = L.inst_cells; A.col_off = L.col_off; A.spread_off = L.spread_off; A.used = L.used;
+    A.is_spread = is_range ? 0u : 1u;
+    const uint64_t* cells0 = (const uint64_t*)cells;
     for (uint64_t i0 = 0; i0 < n_instances; i0 += chunk) {
       const unsigned ni = (unsigned)std::min<uint64_t>(chunk, n_instances - i0);
       A.cells = cells0 + i0 * A.inst_cells * 4;
@@ -173,7 +164,8 @@ int h2sha_lookup_product_per_instance(h2sha_engine_t* e, uint64_t n_instances, u
                                       const uint64_t* thetas_mont, const uint64_t* betas_mont, const uint64_t* gammas_mont,
                                       void* z_dev, uint32_t* errors_dev, void* stream) {
   if (!e || !betas_mont || !gammas_mont) return set_err(H2SHA_EINVAL, "null argument");
-  const bool is_spread = lookup_idx >= e->plan.n_lookup_cols && lookup_idx < e->plan.n_lookup_cols + e->plan.cfg.spread_cols;
+  const LookupSel L = select_lookup(lookup_geom(e->plan), lookup_idx);
+  const bool is_spread = L.valid && !L.is_range;
   if (is_spread && !thetas_mont) return set_err(H2SHA_EINVAL, "a spread lookup has two expressions: thetas_mont is needed to compress them");
   int rc;
   if ((rc = check_challenge_rows(betas_mont, n_instances, "betas_mont")) || (rc = check_challenge_rows(gammas_mont, n_instances, "gammas_mont")) ||

@@ -7,13 +7,15 @@
 //   per digest() call d:  (2) the shape copies whose newer cell lies in d's gate range, shape order:
 //                             constrain_equal(gate(a), gate(b) | fixed(k))
 //                         (3) per spread limb n of d: constrain_equal(dense cell, gate(limb_dense_src[n])), then the spread cell
-//   range.finalize:       constrain_equal(lookup cell k, gate(lookup_src[k])), push order (wrapping at max_rows)
+//   range.finalize:       constrain_equal(lookup cell k, gate(lookup_src[k])), push order (LookupGeom::range_cell)
 //   bind_output_bytes:    constrain_instance(output_bytes[i], instance, i), i < 32 * n_digests
 // A change to that order in chip_api.hpp has to be made here too (tests/test_permutation_product.py replays the recorded calls of
 // the C++ facade against h2sha_get_permutation).
 #include "permutation.h"
 
 #include <algorithm>
+
+#include "lookup_geom.h"
 
 namespace h2sha {
 
@@ -37,7 +39,8 @@ bool perm_columns(const Plan& P, const h2sha_perm_desc_t& d, uint32_t U, PermCol
     while ((1ull << C.k) < (uint64_t)U + 2) C.k++;
     if (C.k > 28) return fail("usable_rows needs a domain larger than 2^28");
   }
-  const uint32_t nc = P.cfg.spread_cols;
+  const LookupGeom G = lookup_geom(P);
+  const uint32_t nc = G.spread_cols;
   const uint32_t limit[7] = {P.n_gate_cols, P.n_lookup_cols, nc, nc, C.num_fixed, 0, 1};
   for (int k = 0; k < 7; k++) C.pos[k].assign(limit[k], -1);
   for (uint32_t c = 0; c < C.n_cols; c++) {
@@ -52,9 +55,9 @@ bool perm_columns(const Plan& P, const h2sha_perm_desc_t& d, uint32_t U, PermCol
   // every column the chip copies from or to (the replay checks each cell again)
   for (uint32_t c = 0; c < P.n_gate_cols; c++)
     if (C.pos[H2SHA_COL_GATE][c] < 0) return fail("gate advice column " + std::to_string(c) + " holds copied cells but is not listed");
-  for (uint32_t c = 0; c < P.n_lookup_cols && (uint64_t)c * P.cfg.max_rows < P.n_lookup; c++)
+  for (uint32_t c = 0; c < P.n_lookup_cols && G.range_used(c) > 0; c++)
     if (C.pos[H2SHA_COL_LOOKUP][c] < 0) return fail("lookup advice column " + std::to_string(c) + " holds copied cells but is not listed");
-  for (uint32_t c = 0; c < nc && c < P.n_limb; c++)
+  for (uint32_t c = 0; c < nc && G.spread_used(c) > 0; c++)
     if (C.pos[H2SHA_COL_DENSE][c] < 0 || C.pos[H2SHA_COL_SPREAD][c] < 0)
       return fail("spread column pair " + std::to_string(c) + " holds copied cells but is not listed");
   for (uint32_t c = 0; c < C.num_fixed && c < P.fixed_consts.size(); c++)
@@ -93,7 +96,8 @@ bool replay_permutation(const Plan& P, const PermColumns& C, std::vector<uint32_
     do { aux[i] = left; i = mapping[i]; } while (i != right);
     std::swap(mapping[l], mapping[r]);
   };
-  const uint32_t D = (uint32_t)P.digests.size(), nc = P.cfg.spread_cols;
+  const LookupGeom G = lookup_geom(P);
+  const uint32_t D = (uint32_t)P.digests.size();
   for (uint32_t d = 0; d < D && ok; d++) {
     const bool last = d + 1 == D;
     const uint32_t g0 = P.digests[d].gate_base, g1 = last ? P.n_gate : P.digests[d + 1].gate_base;
@@ -103,13 +107,16 @@ bool replay_permutation(const Plan& P, const PermColumns& C, std::vector<uint32_
       const uint32_t a = gate(cp.a_idx), b = cp.b_kind == CP_GATE ? gate(cp.b_idx) : fixed(cp.b_idx);
       copy(a, b);
     }
-    for (uint32_t l = n0; l < n1; l++) {    // (3) limb l -> column pair l % nc, row l / nc
-      copy(cell(H2SHA_COL_DENSE, l % nc, l / nc), gate(P.limb_gate_dense[l]));
-      copy(cell(H2SHA_COL_SPREAD, l % nc, l / nc), gate(P.limb_gate_spread[l]));
+    for (uint32_t l = n0; l < n1; l++) {    // (3)
+      const LookupCell c = G.spread_cell(l);
+      copy(cell(H2SHA_COL_DENSE, c.col, c.row), gate(P.limb_gate_dense[l]));
+      copy(cell(H2SHA_COL_SPREAD, c.col, c.row), gate(P.limb_gate_spread[l]));
     }
   }
-  for (uint32_t k = 0; k < P.n_lookup && ok; k++)   // range.finalize
-    copy(cell(H2SHA_COL_LOOKUP, k / P.cfg.max_rows, k % P.cfg.max_rows), gate(P.lookup_cells[k]));
+  for (uint32_t k = 0; k < P.n_lookup && ok; k++) {   // range.finalize
+    const LookupCell c = G.range_cell(k);
+    copy(cell(H2SHA_COL_LOOKUP, c.col, c.row), gate(P.lookup_cells[k]));
+  }
   if (C.bind)
     for (uint32_t d = 0; d < D && ok; d++)
       for (uint32_t i = 0; i < 32; i++) copy(gate(P.handles[d].output_bytes_idx[i]), cell(H2SHA_COL_INSTANCE, 0, 32 * d + i));

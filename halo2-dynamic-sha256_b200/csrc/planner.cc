@@ -5,6 +5,8 @@
 // patterns are those of halo2-base v0.2.x (SURVEY.md 8a Table B).
 #include "planner.h"
 
+#include "lookup_geom.h"
+
 #include <algorithm>
 #include <array>
 #include <map>
@@ -1575,9 +1577,10 @@ class Builder {
       rows = std::max(rows, e - P.breaks[c]);
     }
     P.gate_col_rows = up8(rows);
-    P.n_lookup_cols = std::max(1u, (n_lk_ + cfg_.max_rows - 1) / cfg_.max_rows);
-    P.lookup_col_rows = up8(std::min(n_lk_, cfg_.max_rows));
-    P.spread_rows = up8((n_limb_ + cfg_.spread_cols - 1) / cfg_.spread_cols);
+    const LookupGeom G = lookup_geom(P);
+    P.n_lookup_cols = G.range_cols_needed();
+    P.lookup_col_rows = up8(G.max_range_used());
+    P.spread_rows = up8(G.max_spread_used());
     compute_zero_ranges(P_);
   }
 };
@@ -1587,8 +1590,8 @@ class Builder {
 
 void compute_zero_ranges(Plan* plan) {
   Plan& P = *plan;
-  const Config& cfg_ = P.cfg;
-  const uint32_t n_gate_ = P.n_gate, n_lk_ = P.n_lookup, n_limb_ = P.n_limb;
+  const uint32_t n_gate_ = P.n_gate;
+  const LookupGeom G = lookup_geom(P);
   P.zero_ranges.clear();
   // cells of the column-major buffers nobody assigns (column tails, stride padding)
     for (size_t c = 0; c < P.breaks.size(); c++) {
@@ -1597,12 +1600,11 @@ void compute_zero_ranges(Plan* plan) {
       if (used < P.gate_col_rows) P.zero_ranges.push_back(ZeroRange{BUF_GATE, (uint32_t)c * P.gate_col_rows + used, P.gate_col_rows - used});
     }
     for (uint32_t c = 0; c < P.n_lookup_cols; c++) {
-      uint32_t used = std::min(cfg_.max_rows, n_lk_ - std::min(n_lk_, c * cfg_.max_rows));
+      uint32_t used = G.range_used(c);
       if (used < P.lookup_col_rows) P.zero_ranges.push_back(ZeroRange{BUF_LOOKUP, c * P.lookup_col_rows + used, P.lookup_col_rows - used});
     }
-    for (uint32_t c = 0; c < 2 * cfg_.spread_cols; c++) {
-      uint32_t cc = c % cfg_.spread_cols;
-      uint32_t used = (n_limb_ + cfg_.spread_cols - 1 - cc) / cfg_.spread_cols;  // limbs n with n % cols == cc
+    for (uint32_t c = 0; c < 2 * G.spread_cols; c++) {
+      uint32_t used = G.spread_used(c % G.spread_cols);
       if (used < P.spread_rows) P.zero_ranges.push_back(ZeroRange{BUF_SPREAD, c * P.spread_rows + used, P.spread_rows - used});
     }
 }
