@@ -29,7 +29,7 @@ H2SHA_OK, H2SHA_EINVAL, H2SHA_EPANIC, H2SHA_ECUDA, H2SHA_ENOMEM = 0, -1, -2, -3,
 # symbols include/h2sha_b200.h declares (checked by tests/test_abi.py)
 EXPORTED_SYMBOLS = [
     "h2sha_create", "h2sha_destroy", "h2sha_last_error", "h2sha_build_id", "h2sha_get_layout", "h2sha_get_breaks", "h2sha_get_handles", "h2sha_get_digest_ranges", "h2sha_get_shape", "h2sha_get_lookup_tables",
-    "h2sha_digest_batch", "h2sha_export_instance", "h2sha_export_batch", "h2sha_get_compact_info", "h2sha_get_compact_map", "h2sha_expand_compact", "h2sha_get_lookup_info", "h2sha_lookup_multiplicities", "h2sha_permute_lookup", "h2sha_permute_lookup_from_raw", "h2sha_lookup_product", "h2sha_get_permutation", "h2sha_permutation_product", "h2sha_permute_lookup_per_instance", "h2sha_permute_lookup_from_raw_per_instance", "h2sha_lookup_product_per_instance", "h2sha_permutation_product_per_instance", "h2sha_check_batch", "h2sha_gather", "h2sha_zero_outputs", "h2sha_debug_mont_from_u64", "h2sha_debug_mont_from_u32", "h2sha_debug_store_probe", "h2sha_debug_int_probe", "h2sha_last_launch_count", "h2sha_last_kernel_ms", "H2SHA_CK_M",
+    "h2sha_digest_batch", "h2sha_export_instance", "h2sha_export_batch", "h2sha_get_compact_info", "h2sha_get_compact_map", "h2sha_expand_compact", "h2sha_get_lookup_info", "h2sha_lookup_multiplicities", "h2sha_permute_lookup", "h2sha_permute_lookup_from_raw", "h2sha_lookup_product", "h2sha_get_permutation", "h2sha_permutation_product", "h2sha_permute_lookup_per_instance", "h2sha_permute_lookup_from_raw_per_instance", "h2sha_lookup_product_per_instance", "h2sha_permutation_product_per_instance", "h2sha_check_batch", "h2sha_check_batch_per_instance", "h2sha_check_site", "h2sha_gather", "h2sha_zero_outputs", "h2sha_debug_mont_from_u64", "h2sha_debug_mont_from_u32", "h2sha_debug_store_probe", "h2sha_debug_int_probe", "h2sha_last_launch_count", "h2sha_last_kernel_ms", "H2SHA_CK_M",
 ]
 
 
@@ -79,6 +79,15 @@ class _PermDesc(C.Structure):
 
 class _CompactInfo(C.Structure):
     _fields_ = [("dict_cells_per_instance", C.c_uint64), ("dict_bytes_per_instance", C.c_uint64), ("cells_per_instance", C.c_uint64), ("n_consts", C.c_uint32)]
+
+
+class _CheckSite(C.Structure):
+    _fields_ = [("n_cells", C.c_uint32), ("kind", C.c_uint32 * 4), ("index", C.c_uint32 * 4), ("row", C.c_uint32 * 4)]
+
+
+# the classes of the constraint check, in the order of its counters (h2sha_check_batch)
+CHECK_CLASSES = ("gates", "copies", "range_lookups", "spread_lookups", "digest_bytes")
+CHECK_NONE = 0xFFFFFFFF   # first failing item of a class without a failure
 
 
 class _LookupInfo(C.Structure):
@@ -143,6 +152,8 @@ def load_library():
     sig("h2sha_permutation_product_per_instance", [C.c_void_p, C.c_uint64, C.POINTER(_PermDesc), C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p,
                                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
     sig("h2sha_check_batch", [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
+    sig("h2sha_check_batch_per_instance", [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
+    sig("h2sha_check_site", [C.c_void_p, C.c_uint32, C.c_uint32, C.POINTER(_CheckSite)])
     sig("h2sha_gather", [C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p])
     sig("h2sha_zero_outputs", [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p])
     sig("h2sha_debug_mont_from_u64", [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p])
@@ -459,7 +470,26 @@ class Sha256DynamicConfig:
         _check(load_library().h2sha_check_batch(self._h, res.gate.shape[0], res.gate.data_ptr(), res.lookup.data_ptr(), res.spread.data_ptr(),
                                                 C.c_void_p(digests_dev_ptr or None), v.ctypes.data_as(C.c_void_p),
                                                 torch.cuda.current_stream(self.device).cuda_stream))
-        return dict(zip(("gates", "copies", "range_lookups", "spread_lookups", "digest_bytes"), (int(x) for x in v)))
+        return dict(zip(CHECK_CLASSES, (int(x) for x in v)))
+
+    def check_batch_per_instance(self, res: "BatchResult", digests_dev_ptr: int = 0) -> Tuple[np.ndarray, np.ndarray]:
+        """The same check with a verdict per instance: (counts, first), numpy u32 [n_instances, 5] in the order of CHECK_CLASSES.
+        first[i, c] is the smallest failing item number of class c in instance i (CHECK_NONE when none fails); check_site names its cells."""
+        import torch
+        n = res.gate.shape[0]
+        out = torch.empty((2, n, 5), dtype=torch.int32, device=torch.device("cuda", self.device))
+        _check(load_library().h2sha_check_batch_per_instance(self._h, n, res.gate.data_ptr(), res.lookup.data_ptr(), res.spread.data_ptr(),
+                                                             C.c_void_p(digests_dev_ptr or None), out[0].data_ptr(), out[1].data_ptr(),
+                                                             torch.cuda.current_stream(self.device).cuda_stream))
+        o = out.cpu().numpy().view(np.uint32)
+        return o[0], o[1]
+
+    def check_site(self, cls: int, item: int) -> dict:
+        """The cells check item `item` of class `cls` reads: {"kind", "index", "row"} lists (kinds COL_*; rows from the region's row 0)."""
+        s = _CheckSite()
+        _check(load_library().h2sha_check_site(self._h, cls, item, C.byref(s)))
+        n = s.n_cells
+        return dict(kind=list(s.kind[:n]), index=list(s.index[:n]), row=list(s.row[:n]))
 
     # ---- lookup-argument pre-work (halo2 lookup prover `permute_expression_pair`; spread.rs:53-62, lib.rs:409-418,469) ----
     def lookup_info(self) -> dict:

@@ -1106,6 +1106,7 @@ enum { H2SHA_N_SETS = 2, H2SHA_N_SLOTS = 8 };
 
 struct h2sha_compact_state;   // export.cuh
 struct h2sha_perm_state;      // permutation_product.cuh
+struct h2sha_check_items;     // batch_check.cuh
 
 struct h2sha_engine {
   Plan plan;
@@ -1152,6 +1153,9 @@ struct h2sha_engine {
   uint64_t *d_chk_fixed = nullptr, *d_chk_bytes = nullptr;
   unsigned long long* d_chk_viol = nullptr;
   uint32_t n_chk_gate_on = 0, n_chk_pairs = 0;
+  uint32_t* d_chk_counts = nullptr;   // per-instance counts of one chunk (h2sha_check_batch)
+  uint64_t chk_counts_cap = 0;       // instances d_chk_counts holds
+  h2sha_check_items* chk_items = nullptr;   // every check item's cells (host), built on first use
   // compact hand-off (export.cuh): the cell -> dictionary-entry map, planned on first use
   h2sha_compact_state* compact = nullptr;
   // permutation product (permutation_product.cuh): the moved cells of the last column list, planned on first use
@@ -1423,10 +1427,12 @@ int h2sha_create(const h2sha_config_t* cfg, h2sha_engine_t** out) {
 
 void h2sha_free_compact_state(h2sha_compact_state* s);   // defined after export.cuh (complete type)
 void h2sha_free_perm_state(h2sha_perm_state* s);         // permutation_product.cuh
+void h2sha_free_check_items(h2sha_check_items* c);      // batch_check.cuh
 
 void h2sha_destroy(h2sha_engine_t* e) {
   if (!e) return;
   h2sha_free_compact_state(e->compact); e->compact = nullptr;
+  h2sha_free_check_items(e->chk_items); e->chk_items = nullptr;
   if (e->device < 0) { delete e; return; }
   cudaSetDevice(e->device);
   if (e->copy_stream) { cudaStreamSynchronize(e->copy_stream); cudaStreamDestroy(e->copy_stream); }
@@ -1444,7 +1450,7 @@ void h2sha_destroy(h2sha_engine_t* e) {
   for (int i = 0; i < 4; i++) if (e->ev[i]) cudaEventDestroy(e->ev[i]);
   cudaFree(e->d_lk_ws); cudaFree(e->d_lk_tab); cudaFree(e->d_range_tab); cudaFree(e->d_lp_ws); cudaFree(e->d_chal); cudaFree(e->d_lookup_raw); cudaFree(e->d_dense_raw);
   h2sha_free_perm_state(e->perm); e->perm = nullptr;
-  cudaFree(e->d_chk_gate_on); cudaFree(e->d_chk_pairs); cudaFree(e->d_chk_out_bytes); cudaFree(e->d_chk_fixed); cudaFree(e->d_chk_bytes); cudaFree(e->d_chk_viol);
+  cudaFree(e->d_chk_gate_on); cudaFree(e->d_chk_pairs); cudaFree(e->d_chk_out_bytes); cudaFree(e->d_chk_fixed); cudaFree(e->d_chk_bytes); cudaFree(e->d_chk_viol); cudaFree(e->d_chk_counts);
   delete e;
 }
 

@@ -138,6 +138,17 @@ class Sha256DynamicConfig {
                    uint64_t violations[5], void* stream) {
     check(h2sha_check_batch(engine_, n_instances, gate, lookup, spread, digests_dev, violations, stream));
   }
+  // the same check per instance, asynchronous: counts_dev / first_dev [n_instances][5] u32 (first_dev may be null); see the header
+  void check_batch_per_instance(uint64_t n_instances, const void* gate, const void* lookup, const void* spread, const uint8_t* digests_dev,
+                                uint32_t* counts_dev, uint32_t* first_dev, void* stream) {
+    check(h2sha_check_batch_per_instance(engine_, n_instances, gate, lookup, spread, digests_dev, counts_dev, first_dev, stream));
+  }
+  // the cells a check item reads (host only)
+  h2sha_check_site_t check_site(uint32_t check_class, uint32_t item) {
+    h2sha_check_site_t s{};
+    check(h2sha_check_site(engine_, check_class, item, &s));
+    return s;
+  }
   h2sha_engine_t* raw() const { return engine_; }
 
  private:

@@ -22,8 +22,29 @@
 
 namespace {
 
-// range lookup: one thread per assigned cell of the lookup advice column(s).  grid = (tiles, instances).  mult == null: only count
-// the cells that are not in the table (batch_check.cuh).
+// Table membership of the chip's two lookups, from Montgomery cells: REDC, then the range table 0 .. n_vals - 1, or a row
+// (dense, spread32(dense)) of the spread table with dense < n_vals.  *row = the table row a member hits.  The multiplicity kernels
+// and the constraint check (batch_check.cuh) share them.
+__device__ __forceinline__ bool range_table_row(const uint64_t* cell, uint32_t n_vals, uint32_t* row) {
+  uint64_t x[4], v[4];
+  load_cell(cell, x);
+  mont_reduce(x, v);
+  *row = (uint32_t)v[0];
+  return (v[1] | v[2] | v[3]) == 0 && v[0] < n_vals;
+}
+__device__ __forceinline__ bool spread_table_row(const uint64_t* dense_cell, const uint64_t* spread_cell, uint32_t n_vals, uint32_t* row) {
+  uint64_t x[4], d[4], s[4];
+  load_cell(dense_cell, x);
+  mont_reduce(x, d);
+  load_cell(spread_cell, x);
+  mont_reduce(x, s);
+  *row = (uint32_t)d[0];
+  bool ok = (d[1] | d[2] | d[3]) == 0 && d[0] < n_vals && (s[1] | s[2] | s[3]) == 0;
+  if (ok) ok = spread32(d[0]) == s[0];   // the pair has to be a table row, not just the dense half
+  return ok;
+}
+
+// range lookup: one thread per assigned cell of the lookup advice column(s).  grid = (tiles, instances).
 __global__ void __launch_bounds__(256) k_range_mult(const LookupGeom G, const uint64_t* __restrict__ lookup, uint32_t* __restrict__ mult,
                                                    uint32_t* __restrict__ bad) {
   const uint64_t inst = blockIdx.y;
@@ -32,14 +53,12 @@ __global__ void __launch_bounds__(256) k_range_mult(const LookupGeom G, const ui
   const uint32_t n_vals = 1u << G.lookup_bits;
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < G.n_lookup; i += gridDim.x * blockDim.x) {
     const LookupCell c = G.range_cell(i);
-    uint64_t x[4], v[4];
-    load_cell(base + ((uint64_t)c.col * G.lookup_col_rows + c.row) * 4, x);
-    mont_reduce(x, v);
-    if ((v[1] | v[2] | v[3]) == 0 && v[0] < n_vals) { if (mult) atomicAdd(&m_inst[(uint64_t)c.col * n_vals + (uint32_t)v[0]], 1u); }
+    uint32_t v;
+    if (range_table_row(base + ((uint64_t)c.col * G.lookup_col_rows + c.row) * 4, n_vals, &v)) atomicAdd(&m_inst[(uint64_t)c.col * n_vals + v], 1u);
     else if (bad) atomicAdd(bad, 1u);
   }
   // never-assigned rows of a column hold 0
-  if (mult && blockIdx.x == 0 && threadIdx.x < G.n_lookup_cols) {
+  if (blockIdx.x == 0 && threadIdx.x < G.n_lookup_cols) {
     const uint32_t col = threadIdx.x, used = G.range_used(col);
     if (G.usable_rows > used) atomicAdd(&m_inst[(uint64_t)col * n_vals], G.usable_rows - used);
   }
@@ -49,31 +68,24 @@ __global__ void __launch_bounds__(256) k_range_mult(const LookupGeom G, const ui
 // shared memory, flushed with one global atomic per non-empty bin.  grid = (tiles, instances); dynamic smem = cols * 2^bits * 4.
 __global__ void __launch_bounds__(256) k_spread_mult(const LookupGeom G, const uint64_t* __restrict__ spread, uint32_t* __restrict__ mult,
                                                     uint32_t* __restrict__ bad) {
-  extern __shared__ uint32_t s_hist[];   // [spread_cols << limb_bits]; not allocated in check-only mode (mult == null), which therefore also serves 16-bit limbs
+  extern __shared__ uint32_t s_hist[];   // [spread_cols << limb_bits]
   const uint32_t n_vals = 1u << G.limb_bits, n_bins = G.spread_cols * n_vals;
-  if (mult) {
-    for (uint32_t i = threadIdx.x; i < n_bins; i += blockDim.x) s_hist[i] = 0;
-    __syncthreads();
-  }
+  for (uint32_t i = threadIdx.x; i < n_bins; i += blockDim.x) s_hist[i] = 0;
+  __syncthreads();
   const uint64_t inst = blockIdx.y;
   const uint64_t* base = spread + inst * G.spread_inst_cells * 4;
   uint32_t* m_inst = mult + inst * G.mult_words() + G.range_words();
   uint32_t n_bad = 0;
   for (uint32_t n = blockIdx.x * blockDim.x + threadIdx.x; n < G.n_limb; n += gridDim.x * blockDim.x) {
     const LookupCell c = G.spread_cell(n);
-    uint64_t x[4], d[4], s[4];
-    load_cell(base + ((uint64_t)c.col * G.spread_rows + c.row) * 4, x);
-    mont_reduce(x, d);
-    load_cell(base + ((uint64_t)(G.spread_cols + c.col) * G.spread_rows + c.row) * 4, x);
-    mont_reduce(x, s);
-    bool ok = (d[1] | d[2] | d[3]) == 0 && d[0] < n_vals && (s[1] | s[2] | s[3]) == 0;
-    if (ok) ok = spread32(d[0]) == s[0];   // the pair has to be a table row, not just the dense half
-    if (!ok) n_bad++;
-    else if (mult) atomicAdd(&s_hist[c.col * n_vals + (uint32_t)d[0]], 1u);
+    uint32_t d;
+    if (spread_table_row(base + ((uint64_t)c.col * G.spread_rows + c.row) * 4, base + ((uint64_t)(G.spread_cols + c.col) * G.spread_rows + c.row) * 4,
+                         n_vals, &d))
+      atomicAdd(&s_hist[c.col * n_vals + d], 1u);
+    else n_bad++;
   }
   if (n_bad && bad) atomicAdd(bad, n_bad);
   __syncthreads();
-  if (!mult) return;   // check-only mode (batch_check.cuh): cells outside the table have been counted
   for (uint32_t i = threadIdx.x; i < n_bins; i += blockDim.x)
     if (s_hist[i]) atomicAdd(&m_inst[i], s_hist[i]);
   if (blockIdx.x == 0 && threadIdx.x < G.spread_cols) {

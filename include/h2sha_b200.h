@@ -344,6 +344,35 @@ int h2sha_permutation_product_per_instance(h2sha_engine_t* e, uint64_t n_instanc
 int h2sha_check_batch(h2sha_engine_t* e, uint64_t n_instances, const void* gate, const void* lookup, const void* spread, const uint8_t* digests_dev,
                       uint64_t* violations_host, void* stream);
 
+/* The same check with a verdict per instance, for batches of independent proofs and for finding a wrong cell:
+ *   counts_dev  device [n_instances][5] u32: instance i's violations per class, classes and order of h2sha_check_batch
+ *   first_dev   device [n_instances][5] u32, or NULL: the smallest failing item number (below) per class, 0xFFFFFFFF when none fails
+ * Both arrays are overwritten, never accumulated into.  Asynchronous on `stream`; the static shape is built on first use.
+ * Summed over the instances, counts_dev equals h2sha_check_batch's counters.  A slice of a batch is passed by offsetting every pointer.
+ *
+ * Item numbers, per instance (the cells of an item are what h2sha_check_site returns):
+ *   class 0 gates          item i = the i-th enabled selector in gate-stream order; 4 cells: gate-stream indices s .. s+3
+ *   class 1 copies         first the n_copies copies of h2sha_get_shape, in its order; then one item per lookup cell k (the lookup
+ *                          cell against lookup_src[k], range.finalize); then two items per spread limb n (the dense cell against
+ *                          limb_dense_src[n], then the spread cell against limb_spread_src[n]); 2 cells each.  A fixed constant k is
+ *                          the cell (H2SHA_COL_FIXED, 0, k): row k of the single fixed column the check assumes
+ *   class 2 range lookups  item k = lookup cell k in cells_to_lookup order; 1 cell (its column is the lookup_idx of the range lookup)
+ *   class 3 spread lookups item n = spread limb n; 2 cells, the dense and the spread cell of column pair n % num_advice_columns
+ *                          (lookup_idx n_range_lookups + n % num_advice_columns)
+ *   class 4 digest bytes   item d * 32 + j = output byte j of digest() call d; 1 cell, the output-byte gate cell */
+int h2sha_check_batch_per_instance(h2sha_engine_t* e, uint64_t n_instances, const void* gate, const void* lookup, const void* spread,
+                                   const uint8_t* digests_dev, uint32_t* counts_dev, uint32_t* first_dev, void* stream);
+
+/* The cells check item `item` of class `check_class` reads, as halo2's MockProver names a failure's place (VerifyFailure): cell c is
+ * column (kind[c], index[c]) -- kinds H2SHA_COL_* -- at row[c]; the region starts at row 0.  Host only: works on a plan-only engine
+ * and builds the shape on first use when the engine was made without build_shape.  H2SHA_EINVAL for a class >= 5 or an item
+ * beyond the class. */
+typedef struct {
+  uint32_t n_cells;
+  uint32_t kind[4], index[4], row[4];
+} h2sha_check_site_t;
+int h2sha_check_site(h2sha_engine_t* e, uint32_t check_class, uint32_t item, h2sha_check_site_t* out);
+
 /* The only collective of the path: all-gather of digests [n_instances_per_rank * n_digests][32] and per-instance checksums
  * [n_instances_per_rank][4] over the caller's communicator (`ncclComm_t`, one per GPU/rank; inside an ncclGroup when one
  * thread drives several GPUs).  Receive buffers hold n_ranks x the send size, rank-major.  Either pair may be NULL.

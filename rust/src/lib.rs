@@ -430,4 +430,17 @@ pub mod batch {
         check(unsafe { h2sha_check_batch(engine, n as u64, gate as *const _, lookup as *const _, spread as *const _, digests_dev as *const u8, v.as_mut_ptr(), stream) })?;
         Ok(v)
     }
+    /// The same check per instance, asynchronous on `stream`: counts / first failing item per instance and class into the device
+    /// arrays [n][5] u32 at `counts_dev` / `first_dev` (`first_dev` may be 0).  Item numbering: `h2sha_check_batch_per_instance`.
+    pub fn check_batch_per_instance(engine: *mut h2sha_engine_t, n: usize, gate: u64, lookup: u64, spread: u64, digests_dev: u64, counts_dev: u64,
+                                    first_dev: u64, stream: *mut std::ffi::c_void) -> Result<(), Error> {
+        check(unsafe { h2sha_check_batch_per_instance(engine, n as u64, gate as *const _, lookup as *const _, spread as *const _, digests_dev as *const u8,
+                                                      counts_dev as *mut u32, first_dev as *mut u32, stream) })
+    }
+    /// The cells (`VerifyFailure`'s column and row) check item `item` of class `check_class` reads; host only.
+    pub fn check_site(engine: *mut h2sha_engine_t, check_class: u32, item: u32) -> Result<h2sha_check_site_t, Error> {
+        let mut s: h2sha_check_site_t = unsafe { std::mem::zeroed() };
+        check(unsafe { h2sha_check_site(engine, check_class, item, &mut s) })?;
+        Ok(s)
+    }
 }
